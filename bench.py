@@ -1,10 +1,16 @@
 #!/usr/bin/env python
-"""bench.py - headline benchmark of the B200 backend (contract in the task statement).
+"""bench.py - headline benchmark of the B200 backend.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload shuffle|msm|both]
+                    [--dump-outputs DIR]
 
 BASELINE.json metric: "shuffle proofs/sec prove+verify (52-card); MSM points/sec at 2^20".
-One "step" = one pass of the hot path over one batch of synthetic input.
+One "step" = one pass of the hot path over one batch of synthetic input.  Every leg's rate is timed over K steps (the
+roofline's kernel timings and the pipe probes keep their own repetition counts).
+
+--dump-outputs DIR: after the timed steps, the outputs of the last step of each leg (proofs, accept bytes, MSM results)
+are written as DIR/<name>.npy, bytes as float32.  The inputs are seeded, so two builds run with the same arguments
+can be compared output for output.
 
 workload `shuffle` (headline; BASELINE configs[1], and configs[3] when --gpus > 1):
     one step = prove + verify a batch of `--batch` independent 52-card shuffle proofs
@@ -436,6 +442,36 @@ def _pin(arr):
     return t
 
 
+# ---------------------------------------------------------------------------------- --dump-outputs
+DUMP_ROWS = 1024            # proofs kept per leg: 1024 x 7008 B x 4 = 29 MB for the 52-card `reference-fixed` proofs
+DUMP_LIMIT = 64 << 20       # bytes of all dumped arrays together
+
+
+def dump_rows(n):
+    """A fixed, seeded sample of min(n, DUMP_ROWS) row indices in ascending order: the same rows in every run."""
+    if n <= DUMP_ROWS:
+        return np.arange(n)
+    return np.sort(np.random.RandomState(0).choice(n, DUMP_ROWS, replace=False))
+
+
+def bytes_f32(buf, rows=1):
+    """Bytes (or a uint8 array) as a (rows, len / rows) float32 array; every byte value is exact in float32."""
+    return np.frombuffer(bytes(buf), dtype=np.uint8).reshape(rows, -1).astype(np.float32)
+
+
+def write_dump(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy, float32 or float64 only, DUMP_LIMIT bytes in all."""
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise ValueError(f"outputs to dump take {total} bytes, more than {DUMP_LIMIT}")
+    for name, a in arrays.items():
+        if a.dtype not in (np.float32, np.float64):
+            raise TypeError(f"{name}: {a.dtype}, expected float32 or float64")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def shuffle_setup_mode(be, k, mode, window_bits):
     """Generators as RistrettoPoint::random (lib.rs:164-167,179-180) from a seeded byte stream (the first 2 n + 2 are
     the stream of the `reference-fixed` runs; `fixed` needs next_pow2(n) per vector), the library-built k-card shuffle
@@ -567,6 +603,14 @@ def bench_shuffle(E, mode, steps, warmup, want_cpu):
         ln["be"].synchronize()
         ln["ok"] = ln["ok"] and bytes(ln["accept"].numpy().tobytes()) == b"\x01" * B
     ms_e2e = timed_block(run_lanes(lane_e2e), steps, lane_warm, [ln["stream"] for ln in lanes])
+    if E["dump"] is not None:
+        # the proofs and accept bytes the last timed step copied to the host
+        last = next(ln for ln in lanes if ln["last"] == lane_warm + steps - 1)
+        rows = dump_rows(B)
+        name = "fixed" if mode == "fixed" else "shuffle"
+        E["dump"][f"{name}_proofs"] = bytes_f32(last["proofs"].numpy(), B)[rows]
+        E["dump"][f"{name}_proof_rows"] = rows.astype(np.float32)
+        E["dump"][f"{name}_accept"] = bytes_f32(last["accept"].numpy())[0]
     all_ok = state["ok"] and all(ln["ok"] for ln in lanes)
     # the same input set gives the same proof bytes on a lane as in the serial run
     same_bytes = None
@@ -683,11 +727,15 @@ def bench_large_deck(E, k=4096, window_bits=8):
     for _ in range(3):
         batch.prove()
         batch.verify(None)
+    steps = E["args"].steps
     l0 = be.launch_count
-    tp = _event_ms(stream, batch.prove, 5)
-    lp = (be.launch_count - l0) // 5
-    tv = _event_ms(stream, lambda: batch.verify(None), 5)
+    tp = _event_ms(stream, batch.prove, steps)
+    lp = (be.launch_count - l0) // steps
+    tv = _event_ms(stream, lambda: batch.verify(None), steps)
     ok = batch.download_accept() == b"\x01"
+    if E["dump"] is not None:
+        E["dump"]["large_deck_proof"] = bytes_f32(batch.download_proofs())[0]
+        E["dump"]["large_deck_accept"] = bytes_f32(batch.download_accept())[0]
     Wn = (256 + window_bits - 1) // window_bits
     alg = shuffle_imad_per_proof(n, Q, m, "fixed", Wn, 16)
     out = {"workload": f"large-deck shuffle, k = {k} committed card values, single proof, `fixed` mode (BASELINE configs[2])",
@@ -754,9 +802,9 @@ def bench_batch_verify(E, total=4096, corrupt_every=97):
             res[key] = d_all[key]
         return step
 
-    steps, warm = max(5, args.steps), max(3, args.warmup)
-    ms_good = E["timed"](run(d_good, "good"), steps, warm)
-    ms_bad = E["timed"](run(d_bad, "bad"), steps, warm)
+    steps = args.steps
+    ms_good = E["timed"](run(d_good, "good"), steps, args.warmup)
+    ms_bad = E["timed"](run(d_bad, "bad"), steps, args.warmup)
     acc_all = bytes(res["bad"].cpu().numpy().tobytes())
     mine = acc_all[per * rank: per * rank + cnt]
     ok = mine == bytes(expect)
@@ -768,6 +816,8 @@ def bench_batch_verify(E, total=4096, corrupt_every=97):
     out = None
     if rank == 0:
         rebuilt = b"".join(acc_all[per * r: per * r + par.shard_bounds(total, world, r)[1]] for r in range(world))
+        if E["dump"] is not None:
+            E["dump"]["batch_verify_accept"] = bytes_f32(rebuilt)[0]
         out = {"metric": "batch verification proofs/sec (52-card, `fixed` mode)", "unit": "proofs/s", "scaling": "strong",
                "workload": f"{total} independent 52-card proofs in total, sharded over {world} GPU(s) ({cnt} on rank 0), "
                            f"{n_bad_total} of them ({100.0 * n_bad_total / total:.1f} %) corrupted in different fields; verify only; "
@@ -806,7 +856,7 @@ def bench_small_msm(E):
         want = cref.msm(scb, cref.decompress(enc))
         for _ in range(3):
             got = be.msm_host(scb, enc)
-        R = 20
+        R = E["args"].steps
         t0 = time.time()
         for _ in range(R):
             got = be.msm_host(scb, enc)
@@ -838,11 +888,14 @@ def bench_small_msm(E):
         for _ in range(2):
             outs = be.msm_batch(scs.tobytes(), pts, npts, cnt)
         t0 = time.time()
-        for _ in range(5):
+        for _ in range(R):
             outs = be.msm_batch(scs.tobytes(), pts, npts, cnt)
-        t_b = (time.time() - t0) / 5
+        t_b = (time.time() - t0) / R
         row["batch_4096_shared_points_us_per_msm"] = t_b / cnt * 1e6
         row["batch_first_matches_cpu"] = outs[:32] == cref.msm(scs[:npts].tobytes(), cp)
+        if E["dump"] is not None:
+            E["dump"][f"trait_call_msm_{npts}"] = bytes_f32(got + got_res + got_tab, 3)
+            E["dump"][f"trait_call_msm_batch_{npts}"] = bytes_f32(outs, cnt)
         rows.append(row)
         pts.free()
     return {"note": "wall clock around the public call (host buffers in and out, one synchronisation per call): host_call = "
@@ -1013,7 +1066,8 @@ def run_ours(args):
     sampler = ClockSampler(local)
 
     E = dict(be=be, dev=dev, stream=stream, world=world, rank=rank, local=local, timed=timed, timed_block=timed_block,
-             imad_peak=imad_peak, imad_probes=imad_probes, peak_src=peak_src, peaks=peaks, peaks_src=peaks_src, args=args, dist=dist)
+             imad_peak=imad_peak, imad_probes=imad_probes, peak_src=peak_src, peaks=peaks, peaks_src=peaks_src, args=args, dist=dist,
+             dump={} if args.dump_outputs else None)
     # ------------------------------------------------------------------ shuffle proofs (headline)
     if args.workload in ("shuffle", "both"):
         if rank == 0:
@@ -1024,7 +1078,7 @@ def run_ours(args):
             line["clocks"] = clocks
         if not args.no_fixed:
             # the north_star's own protocol: l, r replaced by the inner-product argument (SURVEY 8 row a16)
-            fx = bench_shuffle(E, "fixed", max(3, args.steps // 2), args.warmup, want_cpu=(world == 1 and not args.no_cpu))
+            fx = bench_shuffle(E, "fixed", args.steps, args.warmup, want_cpu=(world == 1 and not args.no_cpu))
             if rank == 0:
                 line["fixed"] = fx
         if not args.no_extra:
@@ -1076,7 +1130,7 @@ def run_ours(args):
                 be.msm_submit_dev(d_sets[(first + i) % n_sets].data_ptr(), table, 0, n, d_outs[i & 1].data_ptr())
             be.msm_wait()
 
-        msm_steps = max(args.steps, 10)
+        msm_steps = args.steps
         l0 = be.launch_count
         samp2 = ClockSampler(local)
         if rank == 0 and args.workload == "msm":
@@ -1084,15 +1138,16 @@ def run_ours(args):
         ms_single = timed(msm_resident, msm_steps, args.warmup)
         launches = (be.launch_count - l0) * msm_steps // (msm_steps + args.warmup)
         ms_res = timed_block(msm_submitted, msm_steps, args.warmup)
-        # the submitted results are the single-call results
+        # the submitted results of the last two timed steps are the single-call results
+        last_two = range(max(0, msm_steps - 2), msm_steps)
         want = []
-        for i in range(2):
-            msm_once(d_sets[(args.warmup + msm_steps - 2 + i) % n_sets])
+        for i in last_two:
+            msm_once(d_sets[(args.warmup + i) % n_sets])
             want.append(bytes(d_out[:32].cpu().numpy().tobytes()))
         if world == 1:
-            got = [bytes(d_outs[(msm_steps - 2 + i) & 1][:32].cpu().numpy().tobytes()) for i in range(2)]
+            got = [bytes(d_outs[i & 1][:32].cpu().numpy().tobytes()) for i in last_two]
         else:
-            got = [bytes(smsm.d_outs[(msm_steps - 2 + i) % 3][:32].cpu().numpy().tobytes()) for i in range(2)]
+            got = [bytes(smsm.d_outs[i % 3][:32].cpu().numpy().tobytes()) for i in last_two]
         assert got == want, "submitted MSM results differ from the single-call results"
         sharded_check = None
         if world > 1:
@@ -1107,7 +1162,7 @@ def run_ours(args):
             dist.all_gather_into_tensor(d_allp, d_part)
             torch.cuda.synchronize()
             be.points_sum_compress_dev(d_allp.data_ptr(), world, d_chk.data_ptr())
-            sharded_check = bytes(d_chk.cpu().numpy().tobytes()) == want[1]
+            sharded_check = bytes(d_chk.cpu().numpy().tobytes()) == want[-1]
             assert sharded_check, "sharded MSM (library NCCL) differs from partials gathered by torch.distributed"
         clocks2 = samp2.stop() if (rank == 0 and args.workload == "msm") else None
         ms_e2e_serial = timed(msm_e2e, msm_steps, args.warmup)
@@ -1172,6 +1227,8 @@ def run_ours(args):
             h_out.copy_(smsm.d_outs[(cnt - 1) % 3][:32], non_blocking=True)
 
         ms_e2e = timed_block(msm_pipelined, msm_steps, args.warmup, [copy_stream])
+        if E["dump"] is not None:
+            E["dump"]["msm_result"] = bytes_f32(h_out.numpy())[0]    # the last step's result, on the host
         be.set_profiling(True)
         acc_ms = []
         for i in range(5):
@@ -1240,6 +1297,8 @@ def run_ours(args):
                              "dtype": "u32 (8x32-bit limbs, IMAD.WIDE.U32)", "data": "synthetic"})
 
     if rank == 0:
+        if E["dump"] is not None:
+            write_dump(args.dump_outputs, E["dump"])
         _emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -1267,7 +1326,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline legs")
     ap.add_argument("--no-fixed", action="store_true", help="skip the `fixed` (inner-product) mode leg of the shuffle workload")
     ap.add_argument("--no-extra", action="store_true", help="skip batch_verify / large_deck / trait_call_msm")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of each leg's last step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     # The contract is ONE JSON line on stdout.  Libraries write to file descriptor 1 behind Python's back (NCCL prints

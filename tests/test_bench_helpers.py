@@ -29,3 +29,26 @@ def test_whole_step_operation_counts():
     assert ref["imad"] == 8243528 and fix["imad"] == 23952856
     # the roofline bound quoted for the `fixed` mode: 9.31 T IMAD/s / 23.95 M per proof = 389 K proofs/s
     assert 385e3 < 148 * 32 * 1.965e9 / fix["imad"] < 392e3
+
+
+def test_dump_outputs_helpers(tmp_path):
+    """--dump-outputs: the same sample of rows in every run, every byte value exact, float arrays only, 64 MB in all."""
+    import numpy as np
+    import pytest
+    import bench
+    rows = bench.dump_rows(4096)
+    assert len(rows) == bench.DUMP_ROWS and np.all(np.diff(rows) > 0) and rows[-1] < 4096
+    assert np.array_equal(rows, bench.dump_rows(4096))
+    assert np.array_equal(bench.dump_rows(100), np.arange(100))
+    buf = bytes(range(256)) * 2
+    a = bench.bytes_f32(buf, 4)
+    assert a.dtype == np.float32 and a.shape == (4, 128)
+    assert bytes(a.astype(np.uint8).tobytes()) == buf
+    bench.write_dump(str(tmp_path / "out"), {"x": a, "y": np.zeros(3)})
+    assert np.array_equal(np.load(tmp_path / "out" / "x.npy"), a)
+    assert np.load(tmp_path / "out" / "y.npy").dtype == np.float64
+    with pytest.raises(TypeError):
+        bench.write_dump(str(tmp_path / "bad"), {"z": np.zeros(3, dtype=np.uint8)})
+    with pytest.raises(ValueError):
+        bench.write_dump(str(tmp_path / "big"), {"z": np.zeros(bench.DUMP_LIMIT // 8 + 1)})
+    assert not (tmp_path / "bad").exists() and not (tmp_path / "big").exists()
