@@ -305,25 +305,106 @@ struct fb_consts {
 #define FB_GROUP 4  // windows handled per work item
 #endif
 
-__global__ void __launch_bounds__(FB_THREADS) k_fb_msm(const uint32_t *__restrict__ blk, acp_layout lay, fb_shape sh,
-                                                       const uint32_t *__restrict__ table, int c, int Wn, fb_consts kc,
-                                                       uint32_t *__restrict__ out_ext /* [p][outs] x 32 */) {
-    __shared__ __align__(16) uint32_t red[FB_THREADS][32];
-    const uint32_t p = blockIdx.x, o = blockIdx.y;
-    const uint32_t half = 1u << (c - 1), mask = (1u << c) - 1u;
-    const uint32_t groups = (Wn + FB_GROUP - 1) / FB_GROUP;
-    uint32_t total_terms = 0;
-    for (uint32_t s = 0; s < sh.nseg; s++) total_terms += sh.cnt[s];
-    const uint32_t items = total_terms * groups;
-    ge_ext acc;
+// ---- pieces shared by the table kernels ----
+static __host__ __device__ __forceinline__ uint32_t fb_terms(const fb_shape &sh) {
+    uint32_t n = 0;
+    for (uint32_t s = 0; s < sh.nseg; s++) n += sh.cnt[s];
+    return n;
+}
+// term t -> (segment, index k inside the segment)
+__device__ __forceinline__ void fb_locate_term(const fb_shape &sh, uint32_t t, uint32_t &seg, uint32_t &k) {
+    seg = 0;
+    k = t;
+    while (seg + 1 < sh.nseg && k >= sh.cnt[seg]) { k -= sh.cnt[seg]; seg++; }
+}
+// whether term k of segment seg enters output o: L (o = 0) takes the upper half of each period where sel is 1, the lower
+// half where sel is 2, and R the other half; every term enters when sel_period or sel is 0
+__device__ __forceinline__ bool fb_term_selected(const fb_shape &sh, uint32_t seg, uint32_t k, uint32_t o) {
+    if (!sh.sel_period || !sh.sel[seg]) return true;
+    const bool upper = (k & (sh.sel_period - 1)) >= (sh.sel_period >> 1);
+    return (upper == (o == 0)) == (sh.sel[seg] == 1);
+}
+__device__ __forceinline__ const uint32_t *fb_scalar(const uint32_t *blk, const acp_layout &lay, const fb_shape &sh, uint32_t p,
+                                                     uint32_t o, uint32_t seg, uint32_t k) {
+    return ACP_PTR(blk, lay, p, sh.sc_off[seg] + o * sh.sc_ostride[seg] + k);
+}
+// s[0..8) = the low 256 bits of s' = *sp + K; returns the carry out of them (s'[8] of the 9-limb form)
+__device__ __forceinline__ uint32_t fb_recode(const uint32_t *sp, const uint32_t *K, uint32_t *s) {
+    const uint4 lo = *reinterpret_cast<const uint4 *>(sp), hi = *reinterpret_cast<const uint4 *>(sp + 4);
+    s[0] = lo.x; s[1] = lo.y; s[2] = lo.z; s[3] = lo.w; s[4] = hi.x; s[5] = hi.y; s[6] = hi.z; s[7] = hi.w;
+    unsigned long long carry = 0;
+#pragma unroll
+    for (int i = 0; i < 8; i++) {
+        carry += (unsigned long long)s[i] + K[i];
+        s[i] = (uint32_t)carry;
+        carry >>= 32;
+    }
+    return (uint32_t)carry;
+}
+// signed digit of window w from the 9 limbs of s'
+__device__ __forceinline__ int fb_digit(const uint32_t *s, int c, int Wn, uint32_t w) {
+    const int bit = c * (int)w, limb = bit >> 5, shf = bit & 31;
+    unsigned long long v = s[limb];
+    if (limb + 1 < 9) v |= (unsigned long long)s[limb + 1] << 32;
+    const uint32_t u = (uint32_t)(v >> shf) & ((1u << c) - 1u);
+    return w + 1 == (uint32_t)Wn ? (int)u : (int)u - (int)(1u << (c - 1));
+}
+// mag * 2^(c w) * P_gen (layout of k_fb_build)
+__device__ __forceinline__ const uint32_t *fb_entry(const uint32_t *table, uint32_t gen, int Wn, uint32_t half, uint32_t w,
+                                                    uint32_t mag) {
+    return table + FB_ENTRY_U32 * (((size_t)gen * Wn + w) * half + (mag - 1));
+}
+// acc = the sum of the stream advance(ptr, neg) yields: (table entry, sign) pairs until it returns false.  The stream is
+// software pipelined: the next entry's 96-byte gather (random access into a multi-GB table) is issued before the current
+// mixed add.
+template <class Advance>
+__device__ __forceinline__ void fb_accumulate(ge_ext &acc, Advance &advance) {
     ge_identity(acc);
-    // Work items (term, group of FB_GROUP windows) are strided over the block; within this thread's items the
-    // non-zero digits form one stream of (table entry, sign) pairs.  The stream is software pipelined: the
-    // next entry's 96-byte gather (random access into a multi-GB table) is issued before the current mixed add.
-    const uint32_t stride = FB_THREADS * gridDim.z;
-    uint32_t it = blockIdx.z * FB_THREADS + threadIdx.x;
+    const uint32_t *ptr = nullptr, *ptr_n = nullptr;
+    bool neg = false, neg_n = false;
+    bool ok = advance(ptr, neg);
+    ge_niels q, qn;
+    if (ok) ge_niels_load(q, ptr);
+#pragma unroll 1
+    while (ok) {
+        bool ok_n = advance(ptr_n, neg_n);
+        qn = q;
+        if (ok_n) ge_niels_load(qn, ptr_n);
+        ge_madd(acc, acc, q, neg);
+        q = qn;
+        neg = neg_n;
+        ok = ok_n;
+    }
+}
+// lane 0: the sum of the warp's 32 points, in five shuffle steps.  NOINLINE: the adds as calls (fewer registers).
+template <bool NOINLINE>
+__device__ __forceinline__ void ge_warp_sum(ge_ext &acc) {
+#pragma unroll 1
+    for (int d = 16; d >= 1; d >>= 1) {
+        ge_ext o2;
+#pragma unroll
+        for (int i = 0; i < 8; i++) {
+            o2.X.v[i] = __shfl_down_sync(0xffffffffu, acc.X.v[i], d);
+            o2.Y.v[i] = __shfl_down_sync(0xffffffffu, acc.Y.v[i], d);
+            o2.Z.v[i] = __shfl_down_sync(0xffffffffu, acc.Z.v[i], d);
+            o2.T.v[i] = __shfl_down_sync(0xffffffffu, acc.T.v[i], d);
+        }
+        if (NOINLINE) ge_add_noinline(acc, acc, o2);
+        else ge_add(acc, acc, o2);
+    }
+}
+// k_fb_msm and k_fb_msm_warp: this thread's work items (term, group of FB_GROUP windows) of output o - it, it + stride,
+// ... - as one stream of non-zero digits into fb_accumulate.  scalar(seg, k, term): where the term's scalar is read.
+// s: the 9 words of the current term's s' - indexed by the window, so in local memory; the kernel owns the array, which
+// keeps its stack frame and register allocation as they were measured.
+template <class Scalar>
+__device__ __forceinline__ void fb_accumulate_items(ge_ext &acc, uint32_t (&s)[9], const fb_shape &sh, const uint32_t *table, int c, int Wn,
+                                                    const fb_consts &kc, uint32_t o, uint32_t total_terms, uint32_t it,
+                                                    uint32_t stride, Scalar scalar) {
+    const uint32_t half = 1u << (c - 1);
+    const uint32_t groups = (Wn + FB_GROUP - 1) / FB_GROUP;
+    const uint32_t items = total_terms * groups;
     uint32_t w = 0, w_end = 0, gen = 0;
-    uint32_t s[9];
     bool first = true;
     auto advance = [&](const uint32_t *&ptr, bool &neg) -> bool {
         for (;;) {
@@ -331,58 +412,39 @@ __global__ void __launch_bounds__(FB_THREADS) k_fb_msm(const uint32_t *__restric
                 if (!first) it += stride;
                 first = false;
                 if (it >= items) return false;
-                uint32_t term = it / groups, grp = it - term * groups;
-                uint32_t seg = 0, k = term;
-                while (seg + 1 < sh.nseg && k >= sh.cnt[seg]) { k -= sh.cnt[seg]; seg++; }
+                const uint32_t term = it / groups, grp = it - term * groups;
+                uint32_t seg, k;
+                fb_locate_term(sh, term, seg, k);
                 w = grp * FB_GROUP;
                 w_end = min((uint32_t)Wn, (grp + 1) * FB_GROUP);
-                if (sh.sel_period && sh.sel[seg]) {
-                    const bool upper = (k & (sh.sel_period - 1)) >= (sh.sel_period >> 1);
-                    if ((upper == (o == 0)) != (sh.sel[seg] == 1)) { w = w_end; continue; }
-                }
-                const uint32_t *sp = ACP_PTR(blk, lay, p, sh.sc_off[seg] + o * sh.sc_ostride[seg] + k);
+                if (!fb_term_selected(sh, seg, k, o)) { w = w_end; continue; }
                 gen = sh.gen[seg] + k;
-                uint4 lo = *reinterpret_cast<const uint4 *>(sp), hi = *reinterpret_cast<const uint4 *>(sp + 4);
-                s[0] = lo.x; s[1] = lo.y; s[2] = lo.z; s[3] = lo.w; s[4] = hi.x; s[5] = hi.y; s[6] = hi.z; s[7] = hi.w;
-                unsigned long long carry = 0;   // s' = s + K
-#pragma unroll
-                for (int i = 0; i < 8; i++) {
-                    carry += (unsigned long long)s[i] + kc.K[i];
-                    s[i] = (uint32_t)carry;
-                    carry >>= 32;
-                }
-                s[8] = (uint32_t)carry;
+                s[8] = fb_recode(scalar(seg, k, term), kc.K, s);
             }
             const uint32_t ww = w++;
-            int bit = c * (int)ww, limb = bit >> 5, shf = bit & 31;
-            unsigned long long v = s[limb];
-            if (limb + 1 < 9) v |= (unsigned long long)s[limb + 1] << 32;
-            uint32_t u = (uint32_t)(v >> shf) & mask;
-            int d = (ww + 1 == (uint32_t)Wn) ? (int)u : (int)u - (int)half;
+            const int d = fb_digit(s, c, Wn, ww);
             if (d == 0) continue;
-            uint32_t mag = d < 0 ? (uint32_t)(-d) : (uint32_t)d;
-            ptr = table + FB_ENTRY_U32 * (((size_t)gen * Wn + ww) * half + (mag - 1));
+            const uint32_t mag = d < 0 ? (uint32_t)(-d) : (uint32_t)d;
+            BPP_ASSERT(mag >= 1 && mag <= half && ww < (uint32_t)Wn && it < items);
+            ptr = fb_entry(table, gen, Wn, half, ww, mag);
             neg = d < 0;
             return true;
         }
     };
-    {
-        const uint32_t *ptr = nullptr, *ptr_n = nullptr;
-        bool neg = false, neg_n = false;
-        bool ok = advance(ptr, neg);
-        ge_niels q, qn;
-        if (ok) ge_niels_load(q, ptr);
-#pragma unroll 1
-        while (ok) {
-            bool ok_n = advance(ptr_n, neg_n);
-            qn = q;
-            if (ok_n) ge_niels_load(qn, ptr_n);
-            ge_madd(acc, acc, q, neg);
-            q = qn;
-            neg = neg_n;
-            ok = ok_n;
-        }
-    }
+    fb_accumulate(acc, advance);
+}
+
+// ---- the table kernels ----
+__global__ void __launch_bounds__(FB_THREADS) k_fb_msm(const uint32_t *__restrict__ blk, acp_layout lay, fb_shape sh,
+                                                       const uint32_t *__restrict__ table, int c, int Wn, fb_consts kc,
+                                                       uint32_t *__restrict__ out_ext /* [p][outs] x 32 */) {
+    __shared__ __align__(16) uint32_t red[FB_THREADS][32];
+    const uint32_t p = blockIdx.x, o = blockIdx.y;
+    uint32_t s[9];
+    ge_ext acc;
+    // work items strided over the block and its gridDim.z splits
+    fb_accumulate_items(acc, s, sh, table, c, Wn, kc, o, fb_terms(sh), blockIdx.z * FB_THREADS + threadIdx.x, FB_THREADS * gridDim.z,
+                        [&](uint32_t seg, uint32_t k, uint32_t) { return fb_scalar(blk, lay, sh, p, o, seg, k); });
     // block tree reduction
     ge_store(&red[threadIdx.x][0], acc);
     __syncthreads();
@@ -422,105 +484,26 @@ __global__ void __launch_bounds__(FB_THREADS, FB_WARP_MINBLOCKS) k_fb_msm_warp(c
     const uint32_t wid = blockIdx.x * (FB_THREADS / 32) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (wid >= B * outs) return;   // whole warps leave together
     const uint32_t p = wid / outs, o = wid - p * outs;
-    const uint32_t half = 1u << (c - 1), mask = (1u << c) - 1u;
-    const uint32_t groups = (Wn + FB_GROUP - 1) / FB_GROUP;
-    uint32_t total_terms = 0;
-    for (uint32_t s = 0; s < sh.nseg; s++) total_terms += sh.cnt[s];
-    const uint32_t items = total_terms * groups;
+    const uint32_t total_terms = fb_terms(sh);
     uint32_t *stage = fb_stage + 8 * (size_t)(threadIdx.x >> 5) * total_terms;
     if (STAGE) {
         for (uint32_t t = lane; t < total_terms; t += 32) {
-            uint32_t seg = 0, k = t;
-            while (seg + 1 < sh.nseg && k >= sh.cnt[seg]) { k -= sh.cnt[seg]; seg++; }
-            const uint32_t *sp = ACP_PTR(blk, lay, p, sh.sc_off[seg] + o * sh.sc_ostride[seg] + k);
+            uint32_t seg, k;
+            fb_locate_term(sh, t, seg, k);
+            const uint32_t *sp = fb_scalar(blk, lay, sh, p, o, seg, k);
             const uint4 lo = *reinterpret_cast<const uint4 *>(sp), hi = *reinterpret_cast<const uint4 *>(sp + 4);
             *reinterpret_cast<uint4 *>(stage + 8 * (size_t)t) = lo;
             *reinterpret_cast<uint4 *>(stage + 8 * (size_t)t + 4) = hi;
         }
         __syncwarp();
     }
-    ge_ext acc;
-    ge_identity(acc);
-    // Work items (term, group of FB_GROUP windows) are strided over the block; within this thread's items the
-    // non-zero digits form one stream of (table entry, sign) pairs.  The stream is software pipelined: the
-    // next entry's 96-byte gather (random access into a multi-GB table) is issued before the current mixed add.
-    const uint32_t stride = 32;
-    uint32_t it = lane;
-    uint32_t w = 0, w_end = 0, gen = 0;
     uint32_t s[9];
-    bool first = true;
-    auto advance = [&](const uint32_t *&ptr, bool &neg) -> bool {
-        for (;;) {
-            if (w >= w_end) {
-                if (!first) it += stride;
-                first = false;
-                if (it >= items) return false;
-                uint32_t term = it / groups, grp = it - term * groups;
-                uint32_t seg = 0, k = term;
-                while (seg + 1 < sh.nseg && k >= sh.cnt[seg]) { k -= sh.cnt[seg]; seg++; }
-                w = grp * FB_GROUP;
-                w_end = min((uint32_t)Wn, (grp + 1) * FB_GROUP);
-                if (sh.sel_period && sh.sel[seg]) {
-                    const bool upper = (k & (sh.sel_period - 1)) >= (sh.sel_period >> 1);
-                    if ((upper == (o == 0)) != (sh.sel[seg] == 1)) { w = w_end; continue; }
-                }
-                const uint32_t *sp = STAGE ? stage + 8 * (size_t)term : ACP_PTR(blk, lay, p, sh.sc_off[seg] + o * sh.sc_ostride[seg] + k);
-                gen = sh.gen[seg] + k;
-                uint4 lo = *reinterpret_cast<const uint4 *>(sp), hi = *reinterpret_cast<const uint4 *>(sp + 4);
-                s[0] = lo.x; s[1] = lo.y; s[2] = lo.z; s[3] = lo.w; s[4] = hi.x; s[5] = hi.y; s[6] = hi.z; s[7] = hi.w;
-                unsigned long long carry = 0;   // s' = s + K
-#pragma unroll
-                for (int i = 0; i < 8; i++) {
-                    carry += (unsigned long long)s[i] + kc.K[i];
-                    s[i] = (uint32_t)carry;
-                    carry >>= 32;
-                }
-                s[8] = (uint32_t)carry;
-            }
-            const uint32_t ww = w++;
-            int bit = c * (int)ww, limb = bit >> 5, shf = bit & 31;
-            unsigned long long v = s[limb];
-            if (limb + 1 < 9) v |= (unsigned long long)s[limb + 1] << 32;
-            uint32_t u = (uint32_t)(v >> shf) & mask;
-            int d = (ww + 1 == (uint32_t)Wn) ? (int)u : (int)u - (int)half;
-            if (d == 0) continue;
-            uint32_t mag = d < 0 ? (uint32_t)(-d) : (uint32_t)d;
-            BPP_ASSERT(mag >= 1 && mag <= half && ww < (uint32_t)Wn && it < items);
-            ptr = table + FB_ENTRY_U32 * (((size_t)gen * Wn + ww) * half + (mag - 1));
-            neg = d < 0;
-            return true;
-        }
-    };
-    {
-        const uint32_t *ptr = nullptr, *ptr_n = nullptr;
-        bool neg = false, neg_n = false;
-        bool ok = advance(ptr, neg);
-        ge_niels q, qn;
-        if (ok) ge_niels_load(q, ptr);
-#pragma unroll 1
-        while (ok) {
-            bool ok_n = advance(ptr_n, neg_n);
-            qn = q;
-            if (ok_n) ge_niels_load(qn, ptr_n);
-            ge_madd(acc, acc, q, neg);
-            q = qn;
-            neg = neg_n;
-            ok = ok_n;
-        }
-    }
-    // warp reduction: five shuffle steps
-#pragma unroll 1
-    for (int d = 16; d >= 1; d >>= 1) {
-        ge_ext o2;
-#pragma unroll
-        for (int i = 0; i < 8; i++) {
-            o2.X.v[i] = __shfl_down_sync(0xffffffffu, acc.X.v[i], d);
-            o2.Y.v[i] = __shfl_down_sync(0xffffffffu, acc.Y.v[i], d);
-            o2.Z.v[i] = __shfl_down_sync(0xffffffffu, acc.Z.v[i], d);
-            o2.T.v[i] = __shfl_down_sync(0xffffffffu, acc.T.v[i], d);
-        }
-        ge_add(acc, acc, o2);
-    }
+    ge_ext acc;
+    // work items strided over the warp
+    fb_accumulate_items(acc, s, sh, table, c, Wn, kc, o, total_terms, lane, 32, [&](uint32_t seg, uint32_t k, uint32_t term) {
+        return STAGE ? stage + 8 * (size_t)term : fb_scalar(blk, lay, sh, p, o, seg, k);
+    });
+    ge_warp_sum<false>(acc);
     if (lane == 0) ge_store(out_ext + 32 * ((size_t)p * sh.outs + o), acc);
 }
 // Digit-staged form of k_fb_msm_warp for the window widths whose window count is a power of two (c = 16: 16 windows,
@@ -548,8 +531,7 @@ __global__ void __launch_bounds__(FB_THREADS, FB_WARP_MINBLOCKS) k_fb_msm_warp_d
     const uint32_t wid = blockIdx.x * (FB_THREADS / 32) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (wid >= B * outs) return;   // whole warps leave together
     const uint32_t p = wid / outs, o = wid - p * outs;
-    uint32_t total_terms = 0;
-    for (uint32_t s = 0; s < sh.nseg; s++) total_terms += sh.cnt[s];
+    const uint32_t total_terms = fb_terms(sh);
     // per warp: total_terms x 8 words of s', then the generator indices (region rounded up to 16 bytes)
     uint32_t *stage = fb_stage + (size_t)(threadIdx.x >> 5) * ((9 * total_terms + 3) & ~3u);
     uint32_t *sgen = stage + 8 * (size_t)total_terms;
@@ -559,26 +541,16 @@ __global__ void __launch_bounds__(FB_THREADS, FB_WARP_MINBLOCKS) k_fb_msm_warp_d
         bool act = t < total_terms;
         uint32_t seg = 0, k = t;
         if (act) {
-            while (seg + 1 < sh.nseg && k >= sh.cnt[seg]) { k -= sh.cnt[seg]; seg++; }
-            if (sh.sel_period && sh.sel[seg]) {
-                const bool upper = (k & (sh.sel_period - 1)) >= (sh.sel_period >> 1);
-                act = (upper == (o == 0)) == (sh.sel[seg] == 1);
-            }
+            fb_locate_term(sh, t, seg, k);
+            act = fb_term_selected(sh, seg, k, o);
         }
         const uint32_t bal = __ballot_sync(0xffffffffu, act);
         if (act) {
             const uint32_t idx = n_act + __popc(bal & ((1u << lane) - 1u));
-            const uint32_t *sp = ACP_PTR(blk, lay, p, sh.sc_off[seg] + o * sh.sc_ostride[seg] + k);
-            const uint4 lo = *reinterpret_cast<const uint4 *>(sp), hi = *reinterpret_cast<const uint4 *>(sp + 4);
-            uint32_t s[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
-            unsigned long long carry = 0;   // s' = s + K < 2^256 (s < 2^255, K < 2^(C (WN - 1)))
-#pragma unroll
-            for (int i = 0; i < 8; i++) {
-                carry += (unsigned long long)s[i] + kc.K[i];
-                s[i] = (uint32_t)carry;
-                carry >>= 32;
-            }
-            BPP_ASSERT(carry == 0 && idx < total_terms);
+            uint32_t s[8];
+            const uint32_t carry = fb_recode(fb_scalar(blk, lay, sh, p, o, seg, k), kc.K, s);
+            BPP_ASSERT(carry == 0 && idx < total_terms);   // s' < 2^256 (s < 2^255, K < 2^(C (WN - 1)))
+            (void)carry;
             *reinterpret_cast<uint4 *>(stage + 8 * (size_t)idx) = make_uint4(s[0], s[1], s[2], s[3]);
             *reinterpret_cast<uint4 *>(stage + 8 * (size_t)idx + 4) = make_uint4(s[4], s[5], s[6], s[7]);
             sgen[idx] = sh.gen[seg] + k;
@@ -590,8 +562,6 @@ __global__ void __launch_bounds__(FB_THREADS, FB_WARP_MINBLOCKS) k_fb_msm_warp_d
     const uint32_t ww = lane & (WN - 1);
     const bool top = ww == WN - 1;                      // the top window's digit is unsigned
     const uint32_t lane_entry = ww << (C - 1);          // entry = (gen * WN + ww) * HALF + mag - 1
-    ge_ext acc;
-    ge_identity(acc);
     uint32_t it = lane;
     auto advance = [&](const uint32_t *&ptr, bool &neg) -> bool {
         for (;;) {
@@ -611,51 +581,25 @@ __global__ void __launch_bounds__(FB_THREADS, FB_WARP_MINBLOCKS) k_fb_msm_warp_d
             return true;
         }
     };
-    {   // software pipelined: the gather of the next entry is issued before the current mixed add
-        const uint32_t *ptr = nullptr, *ptr_n = nullptr;
-        bool neg = false, neg_n = false;
-        bool ok = advance(ptr, neg);
-        ge_niels q, qn;
-        if (ok) ge_niels_load(q, ptr);
-#pragma unroll 1
-        while (ok) {
-            bool ok_n = advance(ptr_n, neg_n);
-            qn = q;
-            if (ok_n) ge_niels_load(qn, ptr_n);
-            ge_madd(acc, acc, q, neg);
-            q = qn;
-            neg = neg_n;
-            ok = ok_n;
-        }
-    }
-#pragma unroll 1
-    for (int d = 16; d >= 1; d >>= 1) {   // warp reduction: five shuffle steps
-        ge_ext o2;
-#pragma unroll
-        for (int i = 0; i < 8; i++) {
-            o2.X.v[i] = __shfl_down_sync(0xffffffffu, acc.X.v[i], d);
-            o2.Y.v[i] = __shfl_down_sync(0xffffffffu, acc.Y.v[i], d);
-            o2.Z.v[i] = __shfl_down_sync(0xffffffffu, acc.Z.v[i], d);
-            o2.T.v[i] = __shfl_down_sync(0xffffffffu, acc.T.v[i], d);
-        }
-        ge_add(acc, acc, o2);
-    }
+    ge_ext acc;
+    fb_accumulate(acc, advance);
+    ge_warp_sum<false>(acc);
     if (lane == 0) ge_store(out_ext + 32 * ((size_t)p * sh.outs + o), acc);
 }
-// host side: the warp-per-output launch (digit-staged form when the table's window width has one and the stage fits)
+// host side: the warp-per-output launch.  The digit-staged form where the window width has one, its stage fits and the
+// entry indices fit 32 bits; else the scalar-staged form where its stage fits; else the unstaged form.
 static inline void fb_warp_launch(const uint32_t *d_sc, const acp_layout &lay, const fb_shape &sh, const uint32_t *table, int c, int Wn,
-                                  const fb_consts &kc, uint32_t B, uint32_t outs, uint32_t terms, uint32_t *d_ext, bool stage_ok,
-                                  bool digits_ok, cudaStream_t st) {
-    const uint32_t n_out = B * outs;
+                                  const fb_consts &kc, uint32_t B, uint32_t outs, uint32_t *d_ext, cudaStream_t st) {
+    const uint32_t n_out = B * outs, terms = fb_terms(sh);
     const unsigned grid = (n_out + FB_THREADS / 32 - 1) / (FB_THREADS / 32);
     const size_t stage_d = (size_t)(FB_THREADS / 32) * ((9 * terms + 3) & ~3u) * 4, stage_b = (size_t)(FB_THREADS / 32) * terms * 32;
-    uint64_t gen_end = 0;   // entry indices are 32-bit in the digit-staged form
+    uint64_t gen_end = 0;
     for (uint32_t k = 0; k < sh.nseg; k++) gen_end = gen_end > (uint64_t)sh.gen[k] + sh.cnt[k] ? gen_end : (uint64_t)sh.gen[k] + sh.cnt[k];
     const bool fits32 = ((gen_end * Wn) << (c - 1)) < (1ull << 32);
-    if (digits_ok && stage_ok && fits32 && stage_d <= FB_STAGE_MAX_BYTES && (c == 16 || c == 8)) {
+    if (fits32 && stage_d <= FB_STAGE_MAX_BYTES && (c == 16 || c == 8)) {
         if (c == 16) k_fb_msm_warp_d<16><<<grid, FB_THREADS, stage_d, st>>>(d_sc, lay, sh, table, kc, B, outs, d_ext);
         else k_fb_msm_warp_d<8><<<grid, FB_THREADS, stage_d, st>>>(d_sc, lay, sh, table, kc, B, outs, d_ext);
-    } else if (stage_ok && stage_b <= FB_STAGE_MAX_BYTES) {
+    } else if (stage_b <= FB_STAGE_MAX_BYTES) {
         k_fb_msm_warp<true><<<grid, FB_THREADS, stage_b, st>>>(d_sc, lay, sh, table, c, Wn, kc, B, outs, d_ext);
     } else {
         k_fb_msm_warp<false><<<grid, FB_THREADS, 0, st>>>(d_sc, lay, sh, table, c, Wn, kc, B, outs, d_ext);
@@ -670,35 +614,23 @@ __global__ void __launch_bounds__(128) k_fb_msm_small(const uint32_t *__restrict
     const uint32_t id = blockIdx.x * blockDim.x + threadIdx.x;
     if (id >= B * outs) return;
     const uint32_t p = id / outs, o = id - p * outs;
-    const uint32_t half = 1u << (c - 1), mask = (1u << c) - 1u;
+    const uint32_t half = 1u << (c - 1);
     ge_ext acc;
     ge_identity(acc);
 #pragma unroll 1
     for (uint32_t seg = 0; seg < sh.nseg; seg++) {
 #pragma unroll 1
         for (uint32_t k = 0; k < sh.cnt[seg]; k++) {
-            const uint32_t *sp = ACP_PTR(blk, lay, p, sh.sc_off[seg] + o * sh.sc_ostride[seg] + k);
             const uint32_t gen = sh.gen[seg] + k;
             uint32_t s[9];
-            unsigned long long carry = 0;
-#pragma unroll
-            for (int i = 0; i < 8; i++) {
-                carry += (unsigned long long)sp[i] + kc.K[i];
-                s[i] = (uint32_t)carry;
-                carry >>= 32;
-            }
-            s[8] = (uint32_t)carry;
+            s[8] = fb_recode(fb_scalar(blk, lay, sh, p, o, seg, k), kc.K, s);
 #pragma unroll 1
             for (uint32_t w = 0; w < (uint32_t)Wn; w++) {
-                int bit = c * (int)w, limb = bit >> 5, shf = bit & 31;
-                unsigned long long v = s[limb];
-                if (limb + 1 < 9) v |= (unsigned long long)s[limb + 1] << 32;
-                uint32_t u = (uint32_t)(v >> shf) & mask;
-                int d = (w + 1 == (uint32_t)Wn) ? (int)u : (int)u - (int)half;
+                const int d = fb_digit(s, c, Wn, w);
                 if (d == 0) continue;
-                uint32_t mag = d < 0 ? (uint32_t)(-d) : (uint32_t)d;
+                const uint32_t mag = d < 0 ? (uint32_t)(-d) : (uint32_t)d;
                 ge_niels q;
-                ge_niels_load(q, table + FB_ENTRY_U32 * (((size_t)gen * Wn + w) * half + (mag - 1)));
+                ge_niels_load(q, fb_entry(table, gen, Wn, half, w, mag));
                 ge_madd(acc, acc, q, d < 0);
             }
         }
@@ -718,18 +650,7 @@ __global__ void __launch_bounds__(32) k_fb_sum_splits(const uint32_t *__restrict
         ge_load(t, src + 32 * (size_t)z);
         ge_add(acc, acc, t);
     }
-#pragma unroll 1
-    for (int d = 16; d >= 1; d >>= 1) {
-        ge_ext o2;
-#pragma unroll
-        for (int i = 0; i < 8; i++) {
-            o2.X.v[i] = __shfl_down_sync(0xffffffffu, acc.X.v[i], d);
-            o2.Y.v[i] = __shfl_down_sync(0xffffffffu, acc.Y.v[i], d);
-            o2.Z.v[i] = __shfl_down_sync(0xffffffffu, acc.Z.v[i], d);
-            o2.T.v[i] = __shfl_down_sync(0xffffffffu, acc.T.v[i], d);
-        }
-        ge_add_noinline(acc, acc, o2);
-    }
+    ge_warp_sum<true>(acc);
     if (lane == 0) ge_store(dst + 32 * ((size_t)p * pitch + o), acc);
 }
 

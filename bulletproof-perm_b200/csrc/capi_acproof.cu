@@ -21,9 +21,7 @@ struct bpp_circuit {
 
 struct bpp_gens {
     uint32_t n = 0, n_gens = 0;  // gens order: g, h, G[0..n), H[0..n)
-    int c = 8, Wn = 32;
-    uint32_t *d_niels = nullptr, *d_table = nullptr;
-    fb_consts kc;
+    bpp_points *pts = nullptr;   // the n_gens points and their window table (bpp_points_precompute)
 };
 
 struct bpp_acp_batch {
@@ -66,19 +64,13 @@ struct bpp_acp_batch {
     // priority split (bpp_acp_batch_set_priority_split): the table-gather MSMs (k_fb_msm) run on `bulk`, a stream of
     // the lowest priority, so that on an urgent caller's stream the short dependent kernels of this batch win the SM
     // slots against the GPU-filling kernels of a second batch in flight on another stream
-    // large batches: one warp per output point (k_fb_msm_warp) instead of one block; same speed on the A_I shape,
-    // 5 % on the `fixed` mode's prover (two outputs per launch).  BPP_FB_WARP=0 keeps the block form (tuning hook).
-    bool fb_warp_per_output = true;
     bool priority_split = false;
     cudaStream_t bulk = nullptr;
     cudaEvent_t ev_bfork = nullptr, ev_bjoin = nullptr;
     // batch verification by random linear combination (k_rlc_*): scalars of the one MSM over the batch's
     // dynamic points + the shared generators (appended to d_dyn), its compressed result, the fall-back flag
     bool batch_rlc = true;
-    bool fb_stage_scalars = true;   // k_fb_msm_warp<true>: the warp's scalars staged in shared memory (BPP_FB_STAGE=0: off)
     bool decompress_late = false;   // verifier: fork the point decompression after the transcript replay (BPP_DECOMPRESS_LATE=1)
-    bool ipa_fused_tail = true;     // k_ipa_lr_tail for split launches (BPP_IPA_TAIL=0: the three separate launches)
-    bool fb_digits = true;          // k_fb_msm_warp_d: digits staged, c = 16 / 8 (BPP_FB_DIGITS=0: the form above; tuning hook)
     uint32_t *d_rlc_sc = nullptr, *d_rlc_flag = nullptr;
     uint8_t *d_rlc_out = nullptr;
     uint32_t *h_rlc_flag = nullptr;
@@ -277,48 +269,20 @@ extern "C" int bpp_gens_create(bpp_ctx *ctx, const uint8_t g[32], const uint8_t 
     bpp_points *pts = nullptr;
     int rc = bpp_points_upload(ctx, BPP_FMT_COMPRESSED, all.data(), 2 * n + 2, &pts);
     if (rc) return rc;
+    if ((rc = bpp_points_precompute(ctx, pts, window_bits))) {
+        bpp_points_free(ctx, pts);
+        return rc;
+    }
     bpp_gens *gs = new bpp_gens();
     gs->n = (uint32_t)n;
     gs->n_gens = (uint32_t)(2 * n + 2);
-    gs->c = window_bits;
-    gs->Wn = (256 + window_bits - 1) / window_bits;
-    gs->d_niels = pts->niels;
-    pts->niels = nullptr;
-    bpp_points_free(ctx, pts);
-    // K = sum_{w < Wn-1} 2^(c w + c - 1)
-    memset(&gs->kc, 0, sizeof(gs->kc));
-    for (int w = 0; w < gs->Wn - 1; w++) {
-        int bit = gs->c * w + gs->c - 1;
-        gs->kc.K[bit >> 5] |= 1u << (bit & 31);
-    }
-    const size_t half = (size_t)1 << (gs->c - 1);
-    const size_t entries = (size_t)gs->n_gens * gs->Wn * half;
-    if (cudaMalloc((void **)&gs->d_table, entries * FB_ENTRY_U32 * 4) != cudaSuccess) {
-        cudaGetLastError();
-        cudaFree(gs->d_niels);
-        delete gs;
-        return BPP_ERR_OOM;
-    }
-    const uint32_t threads = gs->n_gens * gs->Wn;
-    k_fb_build<<<(threads + 63) / 64, 64, 0, ctx->stream>>>(gs->d_niels, gs->n_gens, gs->c, gs->Wn, gs->d_table);
-    ctx->launches++;
-    cudaError_t e = cudaGetLastError();
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) {
-        ctx->last_error = cudaGetErrorString(e);
-        cudaFree(gs->d_niels);
-        cudaFree(gs->d_table);
-        delete gs;
-        return BPP_ERR_CUDA;
-    }
+    gs->pts = pts;
     *out = gs;
     return BPP_OK;
 }
 extern "C" void bpp_gens_free(bpp_ctx *ctx, bpp_gens *g) {
     if (!g) return;
-    if (ctx) { cudaSetDevice(ctx->device); cudaStreamSynchronize(ctx->stream); }
-    cudaFree(g->d_niels);
-    cudaFree(g->d_table);
+    bpp_points_free(ctx, g->pts);
     delete g;
 }
 
@@ -329,17 +293,6 @@ __global__ void k_compress_strided(const uint32_t *__restrict__ ext, uint32_t pi
 // the same generator set, with fresh scalars per proof.  For such a set the window table of bpp_points_precompute turns
 // every MSM into table look-ups and mixed adds - no buckets, no doublings, so no 253-step dependent chain - and
 // bpp_msm_vartime_batch evaluates `count` of them per launch.
-static bool fb_digits_default() {
-    const char *e = getenv("BPP_FB_DIGITS");
-    return !e || e[0] != '0';
-}
-static void fb_make_K(int c, int Wn, uint32_t K[8]) {   // sum_{w < Wn-1} 2^(c w + c - 1)
-    memset(K, 0, 32);
-    for (int w = 0; w < Wn - 1; w++) {
-        int bit = c * w + c - 1;
-        K[bit >> 5] |= 1u << (bit & 31);
-    }
-}
 extern "C" int bpp_points_precompute(bpp_ctx *ctx, bpp_points *p, int window_bits) {
     if (!ctx || !p || p->n == 0) return BPP_ERR_INVALID_ARG;
     if (window_bits == 0) window_bits = 8;
@@ -365,12 +318,43 @@ extern "C" int bpp_points_precompute(bpp_ctx *ctx, bpp_points *p, int window_bit
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     p->fb_c = window_bits;
     p->fb_Wn = Wn;
-    fb_make_K(window_bits, Wn, p->fb_K);
+    memset(p->fb_K, 0, sizeof(p->fb_K));   // K = sum_{w < Wn-1} 2^(c w + c - 1)
+    for (int w = 0; w < Wn - 1; w++) {
+        const int bit = window_bits * w + window_bits - 1;
+        p->fb_K[bit >> 5] |= 1u << (bit & 31);
+    }
     return BPP_OK;
+}
+// The table-gather MSM's forms: a thread per output (k_fb_msm_small; few terms, many outputs), a warp per output
+// (fb_warp_launch; from 16 outputs per SM: no block tree, no barrier - as fast as a block on the A_I shape, 5 % faster
+// on the `fixed` mode's prover), else a block per output (k_fb_msm), split over `splits` blocks when the outputs alone
+// do not fill the GPU (k_fb_sum_splits adds the partial sums).
+enum fb_form { FB_SMALL, FB_WARP, FB_BLOCK };
+struct fb_plan {
+    fb_form form;
+    uint32_t splits;
+};
+// blocks per output of the block form: 4 blocks per SM in all, at least one work item per thread, at most 256
+static uint32_t fb_split_count(const bpp_ctx *ctx, uint64_t outputs, uint64_t items) {
+    const uint64_t want = 4ull * ctx->sm_count, cap = (items + FB_THREADS - 1) / FB_THREADS;
+    uint64_t sp = outputs >= want ? 1 : (want + outputs - 1) / outputs;
+    if (sp > cap) sp = cap;
+    if (sp > 256) sp = 256;
+    return (uint32_t)(sp ? sp : 1);
+}
+static fb_plan fb_choose(const bpp_ctx *ctx, uint64_t outputs, uint32_t terms, int Wn, bool small_ok, uint32_t max_splits) {
+    if (small_ok && (uint64_t)terms * Wn <= 64 && outputs >= 32ull * ctx->sm_count) return {FB_SMALL, 1};
+    if (outputs >= 16ull * ctx->sm_count) return {FB_WARP, 1};
+    const uint32_t sp = fb_split_count(ctx, outputs, (uint64_t)terms * ((Wn + FB_GROUP - 1) / FB_GROUP));
+    return {FB_BLOCK, sp < max_splits ? sp : max_splits};
+}
+// bpp_msm_vartime_batch: the warp or the block form
+static fb_plan msm_table_plan(const bpp_ctx *ctx, const bpp_points *P, size_t n, size_t count) {
+    return fb_choose(ctx, count, (uint32_t)n, P->fb_Wn, false, 256);
 }
 // d_sc: count x n scalars; d_out32: count x 32.  Stream-ordered, no synchronisation.
 static int msm_table_run(bpp_ctx *ctx, const uint32_t *d_sc, const bpp_points *P, size_t off, size_t n, size_t count, uint8_t *d_out32,
-                         uint32_t *d_ext, uint32_t *d_part, uint32_t sp) {
+                         uint32_t *d_ext, uint32_t *d_part, const fb_plan &pl) {
     acp_layout lay;
     memset(&lay, 0, sizeof(lay));
     lay.stride = (uint32_t)n;          // one "proof block" per MSM: its n scalars
@@ -380,28 +364,21 @@ static int msm_table_run(bpp_ctx *ctx, const uint32_t *d_sc, const bpp_points *P
     fb_consts kc;
     memcpy(kc.K, P->fb_K, 32);
     cudaStream_t st = ctx->stream;
-    if (count >= 16ull * ctx->sm_count) {
-        fb_warp_launch(d_sc, lay, sh, P->fb_table, P->fb_c, P->fb_Wn, kc, (uint32_t)count, 1, (uint32_t)n, d_ext, true, fb_digits_default(), st);
-        LAUNCH_CHECK(ctx);
-    } else if (sp > 1) {
-        k_fb_msm<<<dim3((unsigned)count, 1, sp), FB_THREADS, 0, st>>>(d_sc, lay, sh, P->fb_table, P->fb_c, P->fb_Wn, kc, d_part);
-        LAUNCH_CHECK(ctx);
-        k_fb_sum_splits<<<dim3((unsigned)count, 1), 32, 0, st>>>(d_part, 1, sp, 1, d_ext);
+    if (pl.form == FB_WARP) {
+        fb_warp_launch(d_sc, lay, sh, P->fb_table, P->fb_c, P->fb_Wn, kc, (uint32_t)count, 1, d_ext, st);
         LAUNCH_CHECK(ctx);
     } else {
-        k_fb_msm<<<dim3((unsigned)count, 1), FB_THREADS, 0, st>>>(d_sc, lay, sh, P->fb_table, P->fb_c, P->fb_Wn, kc, d_ext);
+        k_fb_msm<<<dim3((unsigned)count, 1, pl.splits), FB_THREADS, 0, st>>>(d_sc, lay, sh, P->fb_table, P->fb_c, P->fb_Wn, kc,
+                                                                           pl.splits > 1 ? d_part : d_ext);
         LAUNCH_CHECK(ctx);
+        if (pl.splits > 1) {
+            k_fb_sum_splits<<<dim3((unsigned)count, 1), 32, 0, st>>>(d_part, 1, pl.splits, 1, d_ext);
+            LAUNCH_CHECK(ctx);
+        }
     }
     k_compress_strided<<<(unsigned)((count + 127) / 128), 128, 0, st>>>(d_ext, 1, 0, 1, (uint32_t)count, d_out32);
     LAUNCH_CHECK(ctx);
     return BPP_OK;
-}
-static uint32_t msm_table_splits(const bpp_ctx *ctx, const bpp_points *P, size_t n, size_t count) {
-    const uint64_t want = 4ull * ctx->sm_count, items = (uint64_t)n * ((P->fb_Wn + FB_GROUP - 1) / FB_GROUP);
-    uint64_t sp = count >= want ? 1 : (want + count - 1) / count;
-    if (sp > (items + FB_THREADS - 1) / FB_THREADS) sp = (items + FB_THREADS - 1) / FB_THREADS;
-    if (sp > 256) sp = 256;
-    return (uint32_t)(sp ? sp : 1);
 }
 extern "C" int bpp_msm_vartime_batch_dev(bpp_ctx *ctx, const void *d_scalars, size_t count, bpp_points *points, size_t off, size_t n,
                                          void *d_out32) {
@@ -410,11 +387,11 @@ extern "C" int bpp_msm_vartime_batch_dev(bpp_ctx *ctx, const void *d_scalars, si
     CK(ctx, cudaSetDevice(ctx->device));
     int rc;
     if (!points->fb_table && (rc = bpp_points_precompute(ctx, points, 8))) return rc;
-    const uint32_t sp = msm_table_splits(ctx, points, n, count);
-    const size_t ext_b = count * 128, part_b = sp > 1 ? count * sp * 128 : 0;
+    const fb_plan pl = msm_table_plan(ctx, points, n, count);
+    const size_t ext_b = count * 128, part_b = pl.splits > 1 ? count * pl.splits * 128 : 0;
     if ((rc = grow(ctx, &ctx->d_small, &ctx->cap_small, ext_b + part_b))) return rc;
     return msm_table_run(ctx, (const uint32_t *)d_scalars, points, off, n, count, (uint8_t *)d_out32, (uint32_t *)ctx->d_small,
-                         (uint32_t *)(ctx->d_small + ext_b), sp);
+                         (uint32_t *)(ctx->d_small + ext_b), pl);
 }
 extern "C" int bpp_msm_vartime_batch(bpp_ctx *ctx, const uint8_t *scalars, size_t count, bpp_points *points, size_t off, size_t n,
                                      uint8_t *out32) {
@@ -425,13 +402,13 @@ extern "C" int bpp_msm_vartime_batch(bpp_ctx *ctx, const uint8_t *scalars, size_
     CK(ctx, cudaSetDevice(ctx->device));
     int rc;
     if (!points->fb_table && (rc = bpp_points_precompute(ctx, points, 8))) return rc;
-    const uint32_t sp = msm_table_splits(ctx, points, n, count);
-    const size_t sc_b = count * n * 32, ext_b = count * 128, part_b = sp > 1 ? count * sp * 128 : 0, out_b = count * 32;
+    const fb_plan pl = msm_table_plan(ctx, points, n, count);
+    const size_t sc_b = count * n * 32, ext_b = count * 128, part_b = pl.splits > 1 ? count * pl.splits * 128 : 0, out_b = count * 32;
     if ((rc = grow(ctx, &ctx->d_small, &ctx->cap_small, sc_b + ext_b + part_b + out_b))) return rc;
     uint8_t *d = ctx->d_small;
     CK(ctx, cudaMemcpyAsync(d, scalars, sc_b, cudaMemcpyHostToDevice, ctx->stream));
     if ((rc = msm_table_run(ctx, (const uint32_t *)d, points, off, n, count, d + sc_b + ext_b + part_b, (uint32_t *)(d + sc_b),
-                            (uint32_t *)(d + sc_b + ext_b), sp)))
+                            (uint32_t *)(d + sc_b + ext_b), pl)))
         return rc;
     CK(ctx, cudaMemcpyAsync(out32, d + sc_b + ext_b + part_b, out_b, cudaMemcpyDeviceToHost, ctx->stream));
     CK(ctx, cudaStreamSynchronize(ctx->stream));
@@ -548,22 +525,13 @@ extern "C" int bpp_acp_batch_create(bpp_ctx *ctx, const bpp_circuit *cir, const 
     b->ctx = ctx; b->cir = cir; b->gens = gens; b->mode = mode; b->B = (uint32_t)count;
     b->lay = acp_make_layout(cir->n, cir->Q, cir->m, mode);
     b->proof_len = (uint32_t)bpp_acproof_proof_len_mode(cir->n, mode);
-    if (const char *e = getenv("BPP_FB_WARP")) b->fb_warp_per_output = e[0] != '0';
-    if (const char *e = getenv("BPP_FB_STAGE")) b->fb_stage_scalars = e[0] != '0';
-    b->fb_digits = fb_digits_default();
     if (const char *e = getenv("BPP_ACP_TRACE")) b->trace = e[0] == '1';
-    if (const char *e = getenv("BPP_IPA_TAIL")) b->ipa_fused_tail = e[0] != '0';
     if (const char *e = getenv("BPP_DECOMPRESS_LATE")) b->decompress_late = e[0] == '1';
     b->label.assign(label, label + label_len);
     const size_t B = count, lg = b->lay.lg, per = cir->m + 8 + 2 * lg, nch = 6 + lg;   // challenges per proof + the two weights
-    {   // small batches of large circuits: split each fixed-base MSM over several blocks (k_fb_sum_splits adds them)
-        const size_t terms = 2 * (size_t)b->lay.np + 2, want = 4 * (size_t)ctx->sm_count;
-        size_t sp = B >= want ? 1 : (want + B - 1) / B;
-        const size_t max_sp = (terms * 8 + FB_THREADS - 1) / FB_THREADS;   // at least one work item per thread
-        if (sp > max_sp) sp = max_sp;
-        if (sp > 256) sp = 256;
-        b->fb_splits = (uint32_t)(sp ? sp : 1);
-    }
+    // split scratch of the block form: the largest MSM's terms at 8 work items each (c = 8) whatever the table's width,
+    // so that for c < 8 this, not the launch's own item count, caps the split count
+    b->fb_splits = fb_split_count(ctx, B, (2 * (uint64_t)b->lay.np + 2) * 8);
     cudaError_t e = cudaMalloc((void **)&b->d_blk, B * b->lay.stride * 32);
     if (e == cudaSuccess) e = cudaMemsetAsync(b->d_blk, 0, B * b->lay.stride * 32, ctx->stream);
     if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_seeds, B * 32);
@@ -597,7 +565,7 @@ extern "C" int bpp_acp_batch_create(bpp_ctx *ctx, const bpp_circuit *cir, const 
     if (e == cudaSuccess && lg) e = cudaMallocHost((void **)&b->h_tx3, B * 3 * 32);
     if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_ext8, B * 8 * 128);
     if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_dyn, (B * per + gens->n_gens) * 96);   // + the shared generators (RLC batch MSM)
-    if (e == cudaSuccess) e = cudaMemcpyAsync(b->d_dyn + 24 * B * per, gens->d_niels, (size_t)gens->n_gens * 96, cudaMemcpyDeviceToDevice,
+    if (e == cudaSuccess) e = cudaMemcpyAsync(b->d_dyn + 24 * B * per, gens->pts->niels, (size_t)gens->n_gens * 96, cudaMemcpyDeviceToDevice,
                                               ctx->stream);
     if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_rlc_sc, (B * per + gens->n_gens) * 32);
     if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_rlc_flag, 64);
@@ -683,6 +651,11 @@ static void acp_seg(fb_shape &s, uint32_t off, uint32_t ostride, uint32_t gen, u
     s.sc_off[s.nseg] = off; s.sc_ostride[s.nseg] = ostride; s.gen[s.nseg] = gen; s.cnt[s.nseg] = cnt;
     s.nseg++;
 }
+// the form acp_fb runs for this shape: the split scratch holds 8 outputs per proof, so launches with more do not split
+static fb_plan acp_fb_plan(const bpp_acp_batch *b, const fb_shape &sh) {
+    return fb_choose(b->ctx, (uint64_t)b->B * sh.outs, fb_terms(sh), b->gens->pts->fb_Wn, !sh.sel_period,
+                     sh.outs > 8 ? 1 : b->fb_splits);
+}
 // launches the fixed-base MSM; results land in dst[(p * pitch + o)] (raw extended points)
 // on: run on this stream instead of the context's (small batches: independent commitments side by side); part_region:
 // which eighth of the split scratch to use (concurrent split launches must not share it); deferred_splits: when given
@@ -691,17 +664,17 @@ static void acp_seg(fb_shape &s, uint32_t off, uint32_t ostride, uint32_t gen, u
 static int acp_fb(bpp_acp_batch *b, const fb_shape &sh, uint32_t *dst, uint32_t pitch, cudaStream_t on = nullptr,
                   uint32_t part_region = 0, uint32_t *deferred_splits = nullptr) {
     bpp_ctx *ctx = b->ctx;
+    const bpp_points &P = *b->gens->pts;
     if (deferred_splits) *deferred_splits = 1;
     fb_shape s = sh;
-    s.outs = pitch;  // k_fb_msm addresses out_ext + 32 * (p * outs + o)
-    // few (proof, output) pairs: split the terms of each MSM over several blocks so the launch fills the GPU
-    uint32_t terms = 0;
-    for (uint32_t k = 0; k < sh.nseg; k++) terms += sh.cnt[k];
-    if (!sh.sel_period && (uint64_t)terms * b->gens->Wn <= 64 && (uint64_t)b->B * sh.outs >= 32ull * ctx->sm_count) {
-        // few terms per output and plenty of outputs: a thread per output
+    s.outs = pitch;  // the kernels address out_ext + 32 * (p * outs + o)
+    fb_consts kc;
+    memcpy(kc.K, P.fb_K, 32);
+    const fb_plan pl = acp_fb_plan(b, sh);
+    if (pl.form == FB_SMALL) {
         const uint32_t total = b->B * sh.outs;
-        k_fb_msm_small<<<(total + 127) / 128, 128, 0, ctx->stream>>>(b->d_blk, b->lay, s, b->gens->d_table, b->gens->c, b->gens->Wn,
-                                                                    b->gens->kc, b->B, sh.outs, dst);
+        k_fb_msm_small<<<(total + 127) / 128, 128, 0, ctx->stream>>>(b->d_blk, b->lay, s, P.fb_table, P.fb_c, P.fb_Wn, kc, b->B,
+                                                                    sh.outs, dst);
         LAUNCH_CHECK(ctx);
         return BPP_OK;
     }
@@ -711,31 +684,20 @@ static int acp_fb(bpp_acp_batch *b, const fb_shape &sh, uint32_t *dst, uint32_t 
         CK(ctx, cudaEventRecord(b->ev_bfork, ctx->stream));
         CK(ctx, cudaStreamWaitEvent(st, b->ev_bfork, 0));
     }
-    const uint64_t blocks = (uint64_t)b->B * sh.outs, want = 4ull * ctx->sm_count;
-    const uint64_t items = (uint64_t)terms * ((b->gens->Wn + FB_GROUP - 1) / FB_GROUP);
-    uint64_t sp = blocks >= want ? 1 : (want + blocks - 1) / blocks;
-    if (sp > (items + FB_THREADS - 1) / FB_THREADS) sp = (items + FB_THREADS - 1) / FB_THREADS;
-    if (sp > b->fb_splits || sh.outs > 8) sp = sh.outs > 8 ? 1 : b->fb_splits;
-    if (sp == 1 && b->fb_warp_per_output && blocks >= 16ull * ctx->sm_count) {
-        // plenty of outputs: a warp per output (no block tree, no barrier)
-        fb_warp_launch(b->d_blk, b->lay, s, b->gens->d_table, b->gens->c, b->gens->Wn, b->gens->kc, b->B, sh.outs, terms, dst,
-                       b->fb_stage_scalars, b->fb_digits, st);
+    if (pl.form == FB_WARP) {
+        fb_warp_launch(b->d_blk, b->lay, s, P.fb_table, P.fb_c, P.fb_Wn, kc, b->B, sh.outs, dst, st);
         LAUNCH_CHECK(ctx);
-    } else if (sp > 1) {
+    } else {
         uint32_t *part = b->d_part + 32 * (size_t)part_region * b->B * b->fb_splits;
-        k_fb_msm<<<dim3(b->B, sh.outs, (uint32_t)sp), FB_THREADS, 0, st>>>(b->d_blk, b->lay, s, b->gens->d_table,
-                                                                          b->gens->c, b->gens->Wn, b->gens->kc, part);
+        k_fb_msm<<<dim3(b->B, sh.outs, pl.splits), FB_THREADS, 0, st>>>(b->d_blk, b->lay, s, P.fb_table, P.fb_c, P.fb_Wn, kc,
+                                                                       pl.splits > 1 ? part : dst);
         LAUNCH_CHECK(ctx);
-        if (deferred_splits) {
-            *deferred_splits = (uint32_t)sp;
-        } else {
-            k_fb_sum_splits<<<dim3(b->B, sh.outs), 32, 0, st>>>(part, sh.outs, (uint32_t)sp, pitch, dst);
+        if (pl.splits > 1 && deferred_splits) {
+            *deferred_splits = pl.splits;
+        } else if (pl.splits > 1) {
+            k_fb_sum_splits<<<dim3(b->B, sh.outs), 32, 0, st>>>(part, sh.outs, pl.splits, pitch, dst);
             LAUNCH_CHECK(ctx);
         }
-    } else {
-        k_fb_msm<<<dim3(b->B, sh.outs), FB_THREADS, 0, st>>>(b->d_blk, b->lay, s, b->gens->d_table, b->gens->c,
-                                                            b->gens->Wn, b->gens->kc, dst);
-        LAUNCH_CHECK(ctx);
     }
     if (b->priority_split && !on) {
         CK(ctx, cudaEventRecord(b->ev_bjoin, st));
@@ -1006,7 +968,7 @@ static int acp_prove_ipa(bpp_acp_batch *b) {
         acp_seg(sh, L.vH, 0, gH, np); sh.sel[1] = 2;    // <b_R s^-1 y^-n, H_L> for L, <b_L .., H_R> for R
         acp_seg(sh, L.cl, 1, 0, 1);   sh.sel[2] = 0;    // c_L Q, c_R Q with Q = w g
         // small batches with device transcripts: split sums, compression, transcript and u^-1 in one launch
-        const bool fuse_tail = !b->host_transcripts && B <= 1023 && b->ipa_fused_tail;
+        const bool fuse_tail = !b->host_transcripts && B <= 1023;
         uint32_t split_n = 1;
         if ((rc = acp_fb(b, sh, b->d_lrext + 32 * 2 * (size_t)j, 2 * lg, nullptr, 0, fuse_tail ? &split_n : nullptr))) return rc;
         if (split_n > 1) {
@@ -1472,9 +1434,8 @@ extern "C" int bpp_acp_batch_time_commit_msm(bpp_acp_batch *b, int reps, float *
     cudaEventDestroy(e0);
     cudaEventDestroy(e1);
     *ms_avg = ms / reps;
-    if (mixed_adds) *mixed_adds = (uint64_t)b->B * (1 + 2 * L.n) * b->gens->Wn;
-    const bool warp_form = b->fb_warp_per_output && (uint64_t)b->B >= 16ull * ctx->sm_count;
-    if (full_adds) *full_adds = (uint64_t)b->B * (warp_form ? 31 : FB_THREADS - 1);
+    if (mixed_adds) *mixed_adds = (uint64_t)b->B * (1 + 2 * L.n) * b->gens->pts->fb_Wn;
+    if (full_adds) *full_adds = (uint64_t)b->B * (acp_fb_plan(b, sh).form == FB_WARP ? 31 : FB_THREADS - 1);
     return BPP_OK;
 }
 

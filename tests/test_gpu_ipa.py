@@ -253,14 +253,13 @@ def test_generator_fold_operator_matches_the_oracle_and_the_scalar_fold_form(bac
     table.free()
 
 
-@pytest.mark.parametrize("window_bits,digits", [(16, "1"), (8, "1"), (16, "0")])
-def test_large_batch_uses_the_warp_per_output_msm_and_stays_byte_identical(backend, monkeypatch, window_bits, digits):
-    """From 16 outputs per SM the commitments go through the warp-per-output fixed-base kernels (k_fb_msm_warp_d: digits
-    staged in shared memory, the inner-product rounds' L / R selection compacted while staging; BPP_FB_DIGITS=0: the
-    scalar-staged form).  A 5-card `fixed` batch of 2400 proofs with different prover seeds: a sample of proofs must equal
-    the CPU restatement byte for byte, and every proof must verify."""
+@pytest.mark.parametrize("window_bits", [16, 8, 11])
+def test_large_batch_uses_the_warp_per_output_msm_and_stays_byte_identical(backend, window_bits):
+    """From 16 outputs per SM the commitments go through the warp-per-output fixed-base kernels (c = 16, 8:
+    k_fb_msm_warp_d, digits staged in shared memory, the inner-product rounds' L / R selection compacted while staging;
+    c = 11: k_fb_msm_warp<true>, the scalar-staged form).  A 5-card `fixed` batch of 2400 proofs with different prover
+    seeds: a sample of proofs must equal the CPU restatement byte for byte, and every proof must verify."""
     from bpperm_b200 import acproof as G
-    monkeypatch.setenv("BPP_FB_DIGITS", digits)
     core, prover, V, cir, gens, inst = _setup(backend, 5, 71, window_bits)
     B = 2400
     seeds = [(7000 + i).to_bytes(4, "little") * 8 for i in range(B)]

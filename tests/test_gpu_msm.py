@@ -454,7 +454,9 @@ def test_precomputed_points_single_msm_matches_the_bucket_path_and_the_oracle(ba
     table.free()
 
 
-@pytest.mark.parametrize("n,count", [(2, 1), (2, 5000), (105, 7), (209, 300), (209, 2500), (33, 1)])
+# count >= 16 per SM (148 SMs): a warp per output, at c = 8 digit-staged (209), scalar-staged (350: the digit stage,
+# 50 432 B, exceeds 48 KB) and unstaged (400: the scalar stage, 51 200 B, does too)
+@pytest.mark.parametrize("n,count", [(2, 1), (2, 5000), (105, 7), (209, 300), (209, 2500), (33, 1), (350, 2400), (400, 2400)])
 def test_batched_msm_over_shared_points_matches_the_c_restatement(backend, n, count):
     import numpy as np
     from oracle import cref

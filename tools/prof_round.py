@@ -59,7 +59,6 @@ fb_ms, fb_madd, _ = batch.time_commit_msm(10)
 import os
 row = {"k": k, "mode": mode, "batch": B, "table_window_bits": cb, "prove_ms": tp, "verify_ms": tv, "a_i_msm_ms": fb_ms,
        "a_i_msm_frac_of_imad_limit": fb_madd * 504 / (fb_ms * 1e-3) / be.imad_pipe_limit(), "lib": os.environ.get("BPPERM_LIB", "product"),
-       "stage": os.environ.get("BPP_FB_STAGE", "1"),
        "proofs_per_s": B / ((tp + tv) * 1e-3), "accepted": batch.download_accept() == b"\x01" * B}
 print(json.dumps(row), flush=True)
 if out:
