@@ -6,7 +6,7 @@ is not a valid Python identifier).
 from ._lib import BppError, LIB_PATH, SYMBOLS, load  # noqa: F401
 from .backend import Backend, Points, FMT_AFFINE, FMT_COMPRESSED, FMT_DALEK_XYZT, scalars_to_bytes  # noqa: F401
 from .util import Ops  # noqa: F401
-from . import acproof, weights  # noqa: F401
+from . import acproof, ipa, weights  # noqa: F401
 
 try:  # torch is only needed for the multi-GPU plumbing
     from . import parallel  # noqa: F401

@@ -28,6 +28,8 @@ SYMBOLS = [
     "bpp_acp_batch_upload_witness", "bpp_acp_batch_commit", "bpp_acp_batch_upload_commitments", "bpp_acp_batch_gen_shuffle_witness", "bpp_acp_batch_prove", "bpp_acp_batch_download_proofs",
     "bpp_acp_batch_upload_proofs", "bpp_acp_batch_verify", "bpp_acp_batch_download_accept",
     "bpp_acp_batch_time_commit_msm", "bpp_acp_batch_set_host_transcripts", "bpp_transcript_script", "bpp_ipa_fold_generators", "bpp_acp_batch_set_batch_rlc", "bpp_acp_batch_set_priority_split",
+    "bpp_transcript_new", "bpp_transcript_append_message", "bpp_transcript_challenge_bytes",
+    "bpp_ipa_proof_len", "bpp_ipa_batch_create", "bpp_ipa_batch_free", "bpp_ipa_batch_prove", "bpp_ipa_batch_verify",
 ]
 
 _lib = None
@@ -154,5 +156,16 @@ def load() -> ctypes.CDLL:
     lib.bpp_transcript_script.argtypes = [vp, u8p, sz, c.c_char_p, sz]
     lib.bpp_acp_batch_time_commit_msm.argtypes = [vp, c.c_int, c.POINTER(c.c_float), c.POINTER(c.c_uint64),
                                                   c.POINTER(c.c_uint64)]
+    # transcripts (host only) and the stand-alone inner-product batch; in/out buffers as char* (ctypes string buffers)
+    lib.bpp_transcript_new.argtypes = [u8p, sz, c.c_char_p]
+    lib.bpp_transcript_append_message.argtypes = [c.c_char_p, u8p, sz, u8p, sz]
+    lib.bpp_transcript_challenge_bytes.argtypes = [c.c_char_p, u8p, sz, c.c_char_p, sz]
+    lib.bpp_ipa_proof_len.argtypes = [sz]
+    lib.bpp_ipa_proof_len.restype = sz
+    lib.bpp_ipa_batch_create.argtypes = [vp, vp, sz, sz, sz, sz, sz, c.POINTER(vp)]
+    lib.bpp_ipa_batch_free.argtypes = [vp]
+    lib.bpp_ipa_batch_free.restype = None
+    lib.bpp_ipa_batch_prove.argtypes = [vp, u8p, u8p, u8p, u8p, u8p, c.c_char_p, c.c_char_p]
+    lib.bpp_ipa_batch_verify.argtypes = [vp, u8p, u8p, u8p, u8p, u8p, c.c_char_p, c.c_char_p]
     _lib = lib
     return lib

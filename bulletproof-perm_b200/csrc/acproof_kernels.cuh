@@ -1206,14 +1206,8 @@ __global__ void __launch_bounds__(DYN_W) k_dyn_window_sums(const uint32_t *__res
 
 // phase 2.  Thread per proof: Horner over the 64 window sums (4 doublings each), add the fixed-base
 // part, test for the identity and fold in the scalar check t == <l, r>.
-__global__ void __launch_bounds__(64) k_dyn_horner_accept(acp_layout lay, uint32_t B, const uint32_t *__restrict__ blk,
-                                                          const uint32_t *__restrict__ wsum,
-                                                          const uint32_t *__restrict__ stat_ext /* B x 32 */,
-                                                          const uint32_t *__restrict__ bad, int check_t,
-                                                          uint8_t *__restrict__ accept) {
-    uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
-    if (p >= B) return;
-    ge_ext acc, t;
+FE_INLINE void dyn_horner(ge_ext &acc, const uint32_t *__restrict__ wsum, uint32_t p) {
+    ge_ext t;
     ge_load(acc, wsum + 32 * ((size_t)p * DYN_W + DYN_W - 1));
 #pragma unroll 1
     for (int w = DYN_W - 2; w >= 0; w--) {
@@ -1222,6 +1216,16 @@ __global__ void __launch_bounds__(64) k_dyn_horner_accept(acp_layout lay, uint32
         ge_load(t, wsum + 32 * ((size_t)p * DYN_W + w));
         ge_add(acc, acc, t);
     }
+}
+__global__ void __launch_bounds__(64) k_dyn_horner_accept(acp_layout lay, uint32_t B, const uint32_t *__restrict__ blk,
+                                                          const uint32_t *__restrict__ wsum,
+                                                          const uint32_t *__restrict__ stat_ext /* B x 32 */,
+                                                          const uint32_t *__restrict__ bad, int check_t,
+                                                          uint8_t *__restrict__ accept) {
+    uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= B) return;
+    ge_ext acc, t;
+    dyn_horner(acc, wsum, p);
     ge_load(t, stat_ext + 32 * (size_t)p);
     ge_add(acc, acc, t);
     bool ident = fe_is_zero(acc.X) || fe_is_zero(acc.Y);  // the Ristretto identity coset

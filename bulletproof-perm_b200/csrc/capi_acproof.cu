@@ -2,6 +2,7 @@
 // The driver re-expresses the seven-step state machine of
 // /root/reference/bp-perm/src/circuit_lib.rs (call order lib.rs:219-231) for B proofs in lock-step:
 // one kernel launch per protocol step for the whole batch, Fiat-Shamir transcripts on host threads.
+#include <functional>
 #include <thread>
 
 #include "bpperm_internal.hpp"
@@ -656,49 +657,55 @@ static fb_plan acp_fb_plan(const bpp_acp_batch *b, const fb_shape &sh) {
     return fb_choose(b->ctx, (uint64_t)b->B * sh.outs, fb_terms(sh), b->gens->pts->fb_Wn, !sh.sel_period,
                      sh.outs > 8 ? 1 : b->fb_splits);
 }
-// launches the fixed-base MSM; results land in dst[(p * pitch + o)] (raw extended points)
-// on: run on this stream instead of the context's (small batches: independent commitments side by side); part_region:
-// which eighth of the split scratch to use (concurrent split launches must not share it); deferred_splits: when given
-// and the launch is split, the partial sums are left in the scratch for the caller's own tail kernel (their count is
-// written there; 1 = the result is complete in dst).
-static int acp_fb(bpp_acp_batch *b, const fb_shape &sh, uint32_t *dst, uint32_t pitch, cudaStream_t on = nullptr,
-                  uint32_t part_region = 0, uint32_t *deferred_splits = nullptr) {
-    bpp_ctx *ctx = b->ctx;
-    const bpp_points &P = *b->gens->pts;
+// The fixed-base MSM launch over B proof blocks of layout `lay` in the form `pl`: results land in dst[(p * pitch + o)]
+// (raw extended points).  part: the split scratch of the block form (B x outs x pl.splits partial sums); deferred_splits:
+// when given and the launch is split, the partial sums are left there for the caller's own tail kernel (their count is
+// written; 1 = the result is complete in dst).
+static int fb_launch(bpp_ctx *ctx, const uint32_t *blk, const acp_layout &lay, uint32_t B, const bpp_points &P, const fb_shape &sh,
+                     const fb_plan &pl, uint32_t *dst, uint32_t pitch, cudaStream_t st, uint32_t *part, uint32_t *deferred_splits) {
     if (deferred_splits) *deferred_splits = 1;
     fb_shape s = sh;
     s.outs = pitch;  // the kernels address out_ext + 32 * (p * outs + o)
     fb_consts kc;
     memcpy(kc.K, P.fb_K, 32);
-    const fb_plan pl = acp_fb_plan(b, sh);
     if (pl.form == FB_SMALL) {
-        const uint32_t total = b->B * sh.outs;
-        k_fb_msm_small<<<(total + 127) / 128, 128, 0, ctx->stream>>>(b->d_blk, b->lay, s, P.fb_table, P.fb_c, P.fb_Wn, kc, b->B,
-                                                                    sh.outs, dst);
+        const uint32_t total = B * sh.outs;
+        k_fb_msm_small<<<(total + 127) / 128, 128, 0, st>>>(blk, lay, s, P.fb_table, P.fb_c, P.fb_Wn, kc, B, sh.outs, dst);
         LAUNCH_CHECK(ctx);
-        return BPP_OK;
+    } else if (pl.form == FB_WARP) {
+        fb_warp_launch(blk, lay, s, P.fb_table, P.fb_c, P.fb_Wn, kc, B, sh.outs, dst, st);
+        LAUNCH_CHECK(ctx);
+    } else {
+        k_fb_msm<<<dim3(B, sh.outs, pl.splits), FB_THREADS, 0, st>>>(blk, lay, s, P.fb_table, P.fb_c, P.fb_Wn, kc,
+                                                                    pl.splits > 1 ? part : dst);
+        LAUNCH_CHECK(ctx);
+        if (pl.splits > 1 && deferred_splits) {
+            *deferred_splits = pl.splits;
+        } else if (pl.splits > 1) {
+            k_fb_sum_splits<<<dim3(B, sh.outs), 32, 0, st>>>(part, sh.outs, pl.splits, pitch, dst);
+            LAUNCH_CHECK(ctx);
+        }
     }
+    return BPP_OK;
+}
+// fb_launch over this batch's proof blocks.  on: run on this stream instead of the context's (small batches: independent
+// commitments side by side); part_region: which eighth of the split scratch to use (concurrent split launches must not
+// share it).  With the priority split, the GPU-filling forms go to the low-priority stream.
+static int acp_fb(bpp_acp_batch *b, const fb_shape &sh, uint32_t *dst, uint32_t pitch, cudaStream_t on = nullptr,
+                  uint32_t part_region = 0, uint32_t *deferred_splits = nullptr) {
+    bpp_ctx *ctx = b->ctx;
+    const bpp_points &P = *b->gens->pts;
+    const fb_plan pl = acp_fb_plan(b, sh);
+    uint32_t *part = b->d_part + 32 * (size_t)part_region * b->B * b->fb_splits;
+    if (pl.form == FB_SMALL) return fb_launch(ctx, b->d_blk, b->lay, b->B, P, sh, pl, dst, pitch, ctx->stream, part, deferred_splits);
     cudaStream_t st = on ? on : ctx->stream;
     if (b->priority_split && !on) {   // the GPU-filling launch goes to the low-priority stream, bracketed by events
         st = b->bulk;
         CK(ctx, cudaEventRecord(b->ev_bfork, ctx->stream));
         CK(ctx, cudaStreamWaitEvent(st, b->ev_bfork, 0));
     }
-    if (pl.form == FB_WARP) {
-        fb_warp_launch(b->d_blk, b->lay, s, P.fb_table, P.fb_c, P.fb_Wn, kc, b->B, sh.outs, dst, st);
-        LAUNCH_CHECK(ctx);
-    } else {
-        uint32_t *part = b->d_part + 32 * (size_t)part_region * b->B * b->fb_splits;
-        k_fb_msm<<<dim3(b->B, sh.outs, pl.splits), FB_THREADS, 0, st>>>(b->d_blk, b->lay, s, P.fb_table, P.fb_c, P.fb_Wn, kc,
-                                                                       pl.splits > 1 ? part : dst);
-        LAUNCH_CHECK(ctx);
-        if (pl.splits > 1 && deferred_splits) {
-            *deferred_splits = pl.splits;
-        } else if (pl.splits > 1) {
-            k_fb_sum_splits<<<dim3(b->B, sh.outs), 32, 0, st>>>(part, sh.outs, pl.splits, pitch, dst);
-            LAUNCH_CHECK(ctx);
-        }
-    }
+    int rc = fb_launch(ctx, b->d_blk, b->lay, b->B, P, sh, pl, dst, pitch, st, part, deferred_splits);
+    if (rc) return rc;
     if (b->priority_split && !on) {
         CK(ctx, cudaEventRecord(b->ev_bjoin, st));
         CK(ctx, cudaStreamWaitEvent(ctx->stream, b->ev_bjoin, 0));
@@ -930,6 +937,60 @@ static int acp_challenge_dependent_scalars(bpp_acp_batch *b) {
     return BPP_OK;
 }
 
+// The prover's inner-product rounds (scalar folding, ipa_kernels.cuh), shared by the `fixed` mode and the stand-alone
+// batch.  On entry the transcripts stand after innerproduct_domain_sep and the block holds a, b (lay.l, lay.r), the
+// H factors (lay.yninv), the G factors (lay.yn, io.gf only) and the Q scalar (lay.wq).  G = gens[gG ..), H = gens[gH ..),
+// Q = gens[gQ].  fb(shape, dst, pitch, split_n) launches the fixed-base MSM (acp_fb's contract); host_u(j), when set,
+// draws u_j on host transcripts from the compressed L_j, R_j and leaves u_j, u_j^-1 in the block.  Without it the
+// transcripts are the device states io.tr: batches of up to 1023 proofs run each round's split sums, compression and
+// challenge in one launch (k_ipa_lr_tail), larger ones through k_compress_strided + k_ipa_challenge.
+struct ipa_rounds_io {
+    uint32_t *blk, *lrext, *part;
+    uint8_t *lr;        // B x 2 lg x 32: the compressed L_j, R_j
+    uint64_t *tr;
+    uint32_t gG, gH, gQ;
+    bool gf;
+};
+template <class FB>
+static int ipa_prove_rounds(bpp_ctx *ctx, const acp_layout &L, uint32_t B, const ipa_rounds_io &io, FB fb,
+                            const std::function<int(uint32_t)> &host_u) {
+    const uint32_t np = L.np, lg = L.lg;
+    cudaStream_t s = ctx->stream;
+    int rc;
+    CK(ctx, ipa_round_launch(L, -1, io.blk, B, s, io.gf));   // s table = {1}, c_L, c_R and the MSM scalars of round 0
+    ctx->launches++;
+    for (uint32_t j = 0; j < lg; j++) {
+        const uint32_t nj = np >> j;
+        fb_shape sh = acp_shape(2);
+        sh.sel_period = nj;
+        acp_seg(sh, L.vG, 0, io.gG, np); sh.sel[0] = 1;    // <a_L s, G_R> for L, <a_R s, G_L> for R
+        acp_seg(sh, L.vH, 0, io.gH, np); sh.sel[1] = 2;    // <b_R s^-1 y^-n, H_L> for L, <b_L .., H_R> for R
+        acp_seg(sh, L.cl, 1, io.gQ, 1);  sh.sel[2] = 0;    // c_L Q, c_R Q
+        // small batches with device transcripts: split sums, compression, transcript and u^-1 in one launch
+        const bool fuse_tail = !host_u && B <= 1023;
+        uint32_t split_n = 1;
+        if ((rc = fb(sh, io.lrext + 32 * 2 * (size_t)j, 2 * lg, fuse_tail ? &split_n : nullptr))) return rc;
+        if (split_n > 1) {
+            k_ipa_lr_tail<<<B, 64, 0, s>>>(io.part, split_n, io.lrext, io.lr, L, (int)j, io.tr, io.blk);
+            LAUNCH_CHECK(ctx);
+            CK(ctx, ipa_round_launch(L, (int)j, io.blk, B, s, io.gf));
+            ctx->launches++;
+            continue;
+        }
+        k_compress_strided<<<(2 * B + 127) / 128, 128, 0, s>>>(io.lrext, 2 * lg, 2 * j, 2, B, io.lr);
+        LAUNCH_CHECK(ctx);
+        if (!host_u) {
+            TR_LAUNCH_AT(tr_warp_max() < 1023 ? tr_warp_max() : 1023, k_ipa_challenge, B, s, io.lr, L, B, (int)j, io.tr, io.blk);
+            LAUNCH_CHECK(ctx);
+        } else if ((rc = host_u(j))) {
+            return rc;
+        }
+        CK(ctx, ipa_round_launch(L, (int)j, io.blk, B, s, io.gf));   // fold a, b; s table; next round's c_L, c_R and MSM scalars
+        ctx->launches++;
+    }
+    return BPP_OK;
+}
+
 // `fixed` mode tail of the prover (bulletproofs 4.0.0 inner_product_proof.rs create() behind dalek's R1CS glue):
 // append t_x, t_x_blinding, e_blinding -> w; lg rounds of (L_j, R_j) -> u_j with a, b folded in place.
 static int acp_prove_ipa(bpp_acp_batch *b) {
@@ -957,33 +1018,16 @@ static int acp_prove_ipa(bpp_acp_batch *b) {
         });
         if ((rc = acp_put_challenges(b, L.wq, 1))) return rc;
     }
-    CK(ctx, ipa_round_launch(L, -1, b->d_blk, B, s));   // s table = {1}, c_L, c_R and the MSM scalars of round 0
-    ctx->launches++;
-    const uint32_t gH = 2 + b->gens->n;
-    for (uint32_t j = 0; j < lg; j++) {
-        const uint32_t nj = np >> j;
-        fb_shape sh = acp_shape(2);
-        sh.sel_period = nj;
-        acp_seg(sh, L.vG, 0, 2, np);  sh.sel[0] = 1;    // <a_L s, G_R> for L, <a_R s, G_L> for R
-        acp_seg(sh, L.vH, 0, gH, np); sh.sel[1] = 2;    // <b_R s^-1 y^-n, H_L> for L, <b_L .., H_R> for R
-        acp_seg(sh, L.cl, 1, 0, 1);   sh.sel[2] = 0;    // c_L Q, c_R Q with Q = w g
-        // small batches with device transcripts: split sums, compression, transcript and u^-1 in one launch
-        const bool fuse_tail = !b->host_transcripts && B <= 1023;
-        uint32_t split_n = 1;
-        if ((rc = acp_fb(b, sh, b->d_lrext + 32 * 2 * (size_t)j, 2 * lg, nullptr, 0, fuse_tail ? &split_n : nullptr))) return rc;
-        if (split_n > 1) {
-            k_ipa_lr_tail<<<B, 64, 0, s>>>(b->d_part, split_n, b->d_lrext, b->d_lr, L, (int)j, b->d_tr, b->d_blk);
-            LAUNCH_CHECK(ctx);
-            CK(ctx, ipa_round_launch(L, (int)j, b->d_blk, B, s));
-            ctx->launches++;
-            continue;
-        }
-        k_compress_strided<<<(2 * B + 127) / 128, 128, 0, s>>>(b->d_lrext, 2 * lg, 2 * j, 2, B, b->d_lr);
-        LAUNCH_CHECK(ctx);
-        if (!b->host_transcripts) {
-            TR_LAUNCH_AT(tr_warp_max() < 1023 ? tr_warp_max() : 1023, k_ipa_challenge, B, s, b->d_lr, L, B, (int)j, b->d_tr, b->d_blk);
-            LAUNCH_CHECK(ctx);
-        } else {
+    ipa_rounds_io io;
+    io.blk = b->d_blk; io.lr = b->d_lr; io.lrext = b->d_lrext; io.part = b->d_part; io.tr = b->d_tr;
+    io.gG = 2; io.gH = 2 + b->gens->n; io.gQ = 0;   // Q = w g
+    io.gf = false;
+    auto fb = [&](const fb_shape &sh, uint32_t *dst, uint32_t pitch, uint32_t *split_n) {
+        return acp_fb(b, sh, dst, pitch, nullptr, 0, split_n);
+    };
+    std::function<int(uint32_t)> host_u;
+    if (b->host_transcripts)
+        host_u = [&](uint32_t j) -> int {
             CK(ctx, cudaMemcpy2DAsync(b->h_pts8, 64, b->d_lr + 64 * (size_t)j, 64 * (size_t)lg, 64, B, cudaMemcpyDeviceToHost, s));
             CK(ctx, cudaStreamSynchronize(s));
             acp_parallel_for(B, [&](uint32_t p) {
@@ -992,13 +1036,13 @@ static int acp_prove_ipa(bpp_acp_batch *b) {
                 t.append_point("R", b->h_pts8 + 64 * (size_t)p + 32);
                 t.challenge_wide("u", b->h_wide + 64 * (size_t)p);
             });
-            if ((rc = acp_put_challenges(b, L.u + j, 1))) return rc;
+            int rc2 = acp_put_challenges(b, L.u + j, 1);
+            if (rc2) return rc2;
             k_ipa_uinv<<<(B + 63) / 64, 64, 0, s>>>(L, B, j, b->d_blk);
             LAUNCH_CHECK(ctx);
-        }
-        CK(ctx, ipa_round_launch(L, (int)j, b->d_blk, B, s));   // fold a, b; s table; next round's c_L, c_R and MSM scalars
-        ctx->launches++;
-    }
+            return BPP_OK;
+        };
+    if ((rc = ipa_prove_rounds(ctx, L, B, io, fb, host_u))) return rc;
     k_acp_pack_fixed<<<dim3((b->proof_len / 32 + 127) / 128, B), 128, 0, s>>>(L, b->d_pts8, b->d_lr, b->d_blk, b->d_proofs,
                                                                              b->proof_len);
     LAUNCH_CHECK(ctx);
@@ -1213,7 +1257,7 @@ static int acp_verify_fixed(bpp_acp_batch *b, const uint8_t *verifier_seed) {
         CK(ctx, cudaMemsetAsync(b->d_bad, 0, (size_t)B * 4, b->aux));
         k_acp_decompress<<<(B * (m + 8) + 127) / 128, 128, 0, b->aux>>>(b->d_V, b->d_pts8, m, B, per, b->d_dyn, b->d_bad);
         LAUNCH_CHECK(ctx);
-        k_acp_decompress_lr<<<(B * 2 * lg + 127) / 128, 128, 0, b->aux>>>(b->d_lr, m, lg, B, b->d_dyn, b->d_bad);
+        k_acp_decompress_lr<<<(B * 2 * lg + 127) / 128, 128, 0, b->aux>>>(b->d_lr, 2 * lg, 2 * lg, m + 8, per, B, b->d_dyn, b->d_bad);
         LAUNCH_CHECK(ctx);
         CK(ctx, cudaEventRecord(b->ev_join, b->aux));
         return BPP_OK;
@@ -1277,7 +1321,7 @@ static int acp_verify_fixed(bpp_acp_batch *b, const uint8_t *verifier_seed) {
     if ((rc = acp_challenge_dependent_scalars(b))) return rc;
     acp_dots_launch(L, 9, 1, B, b->d_blk, s);   // sigma
     LAUNCH_CHECK(ctx);
-    k_ipa_vprep<<<(B + 63) / 64, 64, 0, s>>>(L, B, b->d_blk);
+    k_ipa_vprep<<<(B + 63) / 64, 64, 0, s>>>(L, B, m + 8, b->d_blk);
     LAUNCH_CHECK(ctx);
     k_ipa_stable_full<<<B, np >= IPA_ROUND_THREADS ? IPA_ROUND_THREADS : (np < 128 ? 128 : np), 0, s>>>(L, b->d_blk);
     LAUNCH_CHECK(ctx);
@@ -1542,5 +1586,293 @@ extern "C" int bpp_transcript_script(bpp_ctx *ctx, const uint8_t *script, size_t
         ctx->last_error = cudaGetErrorString(e);
         return BPP_ERR_CUDA;
     }
+    return BPP_OK;
+}
+
+// ---- transcript state across the C ABI (host only) ------------------------------------------------------------
+// merlin::Transcript cannot be serialised, so a transcript crosses the ABI as BPP_TRANSCRIPT_BYTES: the 25 Keccak lanes
+// and pos | pos_begin << 8 | cur_flags << 16, 26 little-endian u64 - host_merlin.hpp export_state, merlin_dev.cuh load.
+static_assert(BPP_TRANSCRIPT_BYTES == 8 * MERLIN_STATE_WORDS, "transcript state layout");
+static bool tr_state_ok(const uint8_t *state) {
+    uint64_t w[MERLIN_STATE_WORDS];
+    memcpy(w, state, sizeof(w));
+    return bpp_host::Strobe128::state_valid(w);
+}
+extern "C" int bpp_transcript_new(const uint8_t *label, size_t label_len, uint8_t state[BPP_TRANSCRIPT_BYTES]) {
+    if ((!label && label_len) || !state || label_len >= (1ull << 32)) return BPP_ERR_INVALID_ARG;
+    bpp_host::Transcript t(label, label_len);
+    uint64_t w[MERLIN_STATE_WORDS];
+    t.export_state(w);
+    memcpy(state, w, sizeof(w));
+    return BPP_OK;
+}
+extern "C" int bpp_transcript_append_message(uint8_t state[BPP_TRANSCRIPT_BYTES], const uint8_t *label, size_t label_len,
+                                             const uint8_t *msg, size_t msg_len) {
+    if (!state || (!label && label_len) || (!msg && msg_len) || msg_len >= (1ull << 32)) return BPP_ERR_INVALID_ARG;
+    if (!tr_state_ok(state)) return BPP_ERR_INVALID_ARG;
+    uint64_t w[MERLIN_STATE_WORDS];
+    memcpy(w, state, sizeof(w));
+    bpp_host::Transcript t(w);
+    t.append_message((const char *)label, label_len, msg, msg_len);
+    t.export_state(w);
+    memcpy(state, w, sizeof(w));
+    return BPP_OK;
+}
+extern "C" int bpp_transcript_challenge_bytes(uint8_t state[BPP_TRANSCRIPT_BYTES], const uint8_t *label, size_t label_len,
+                                              uint8_t *out, size_t out_len) {
+    if (!state || (!label && label_len) || (!out && out_len) || out_len >= (1ull << 32)) return BPP_ERR_INVALID_ARG;
+    if (!tr_state_ok(state)) return BPP_ERR_INVALID_ARG;
+    uint64_t w[MERLIN_STATE_WORDS];
+    memcpy(w, state, sizeof(w));
+    bpp_host::Transcript t(w);
+    t.challenge_bytes((const char *)label, label_len, out, out_len);
+    t.export_state(w);
+    memcpy(state, w, sizeof(w));
+    return BPP_OK;
+}
+
+// ---- stand-alone inner-product argument, batched (bulletproofs 4.0.0 inner_product_proof.rs) -----------------------
+// The prover runs the scalar-fold rounds of the `fixed` mode (ipa_prove_rounds) over a block holding only the
+// inner-product fields (ipa_make_layout); the verifier evaluates dalek's verify as one MSM per proof: the 2 n + 1
+// generator terms through the window table, the 2 lg n + 1 proof points through k_dyn_window_sums.
+struct bpp_ipa_batch {
+    bpp_ctx *ctx = nullptr;
+    bpp_points *gens = nullptr;
+    uint32_t g_off = 0, h_off = 0, q_off = 0, n = 0, lg = 0, B = 0, fb_splits = 1;
+    acp_layout lay;
+    uint32_t *d_blk = nullptr, *d_lrext = nullptr, *d_part = nullptr, *d_stat = nullptr, *d_wsum = nullptr, *d_bad = nullptr,
+             *d_dyn = nullptr;
+    uint8_t *d_in = nullptr;       // staged inputs: a | b | G factors | H factors (B x n x 32 each) | q (B x 32) | P (B x 32)
+    uint8_t *d_lr = nullptr;       // B x (2 lg + 1) x 32: L_j, R_j (prover: the first 2 lg per proof, pitch 2 lg), then P
+    uint8_t *d_proofs = nullptr, *d_accept = nullptr;
+    uint64_t *d_tr = nullptr;
+    // BPP_ACP_TRACE=1: stage timeline of prove / verify on the context's stream, printed to stderr (as bpp_acp_batch's)
+    bool trace = false;
+    std::vector<std::pair<const char *, cudaEvent_t>> marks;
+};
+static void ipa_mark(bpp_ipa_batch *b, const char *name) {
+    if (!b->trace) return;
+    cudaEvent_t e;
+    cudaEventCreate(&e);
+    cudaEventRecord(e, b->ctx->stream);
+    b->marks.emplace_back(name, e);
+}
+// after the call's synchronisation
+static void ipa_marks_dump(bpp_ipa_batch *b, const char *what) {
+    if (!b->trace || b->marks.empty()) return;
+    fprintf(stderr, "[ipa trace] %s:", what);
+    for (size_t i = 1; i < b->marks.size(); i++) {
+        float ms = 0;
+        cudaEventElapsedTime(&ms, b->marks[i - 1].second, b->marks[i].second);
+        fprintf(stderr, " %s %.0f us |", b->marks[i].first, ms * 1e3f);
+    }
+    fprintf(stderr, "\n");
+    for (auto &m : b->marks) cudaEventDestroy(m.second);
+    b->marks.clear();
+}
+
+static acp_layout ipa_make_layout(uint32_t n) {
+    acp_layout L;
+    memset(&L, 0, sizeof(L));
+    uint32_t o = 0;
+    auto take = [&](uint32_t cnt) { uint32_t r = o; o += cnt; return r; };
+    L.n = n; L.np = n; L.lg = acp_log2(n);
+    L.l = take(n); L.r = take(n); L.yn = take(n); L.yninv = take(n); L.vG = take(n); L.vH = take(n);
+    L.stab = take(2 * n);
+    L.u = take(L.lg); L.uinv = take(L.lg); L.vd = take(2 * L.lg + 1);
+    L.wq = take(1); L.cl = take(2); L.pa = take(1); L.pb = take(1);
+    L.stride = (o + 3) & ~3u;
+    return L;
+}
+
+extern "C" size_t bpp_ipa_proof_len(size_t n) {
+    if (n == 0 || (n & (n - 1))) return 0;
+    size_t lg = 0;
+    while (((size_t)1 << lg) < n) lg++;
+    return 32 * (2 * lg + 2);
+}
+
+extern "C" void bpp_ipa_batch_free(bpp_ipa_batch *b) {
+    if (!b) return;
+    cudaSetDevice(b->ctx->device);
+    cudaStreamSynchronize(b->ctx->stream);
+    void *dev[] = {b->d_blk, b->d_lrext, b->d_part, b->d_stat, b->d_wsum, b->d_bad, b->d_dyn, b->d_in, b->d_lr, b->d_proofs,
+                   b->d_accept, b->d_tr};
+    for (void *p : dev)
+        if (p) cudaFree(p);
+    for (auto &m : b->marks) cudaEventDestroy(m.second);
+    delete b;
+}
+
+#define IPA_MAX_N 8192   // the large deck's n' (4096 cards): the largest shape the tables and tests cover
+extern "C" int bpp_ipa_batch_create(bpp_ctx *ctx, bpp_points *gens, size_t g_off, size_t h_off, size_t q_off, size_t n, size_t count,
+                                    bpp_ipa_batch **out) {
+    if (!ctx || !gens || !out || count == 0 || count > (1u << 24) || n == 0 || n > IPA_MAX_N || (n & (n - 1)))
+        return BPP_ERR_INVALID_ARG;
+    *out = nullptr;
+    if (g_off > gens->n || n > gens->n - g_off || h_off > gens->n || n > gens->n - h_off || q_off >= gens->n)
+        return BPP_ERR_LENGTH_MISMATCH;
+    CK(ctx, cudaSetDevice(ctx->device));
+    bpp_ipa_batch *b = new bpp_ipa_batch();
+    b->ctx = ctx; b->gens = gens;
+    b->g_off = (uint32_t)g_off; b->h_off = (uint32_t)h_off; b->q_off = (uint32_t)q_off;
+    b->n = (uint32_t)n; b->B = (uint32_t)count;
+    b->lay = ipa_make_layout(b->n);
+    b->lg = b->lay.lg;
+    if (const char *e = getenv("BPP_ACP_TRACE")) b->trace = e[0] == '1';
+    const size_t B = count, lg = b->lg;
+    b->fb_splits = fb_split_count(ctx, B, (2 * (uint64_t)n + 2) * 8);   // as bpp_acp_batch_create sizes its scratch
+    cudaError_t e = cudaMalloc((void **)&b->d_blk, B * b->lay.stride * 32);
+    if (e == cudaSuccess) e = cudaMemsetAsync(b->d_blk, 0, B * b->lay.stride * 32, ctx->stream);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_in, B * (4 * n + 2) * 32);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_lr, B * (2 * lg + 1) * 32);
+    if (e == cudaSuccess && lg) e = cudaMalloc((void **)&b->d_lrext, B * 2 * lg * 128);
+    if (e == cudaSuccess && b->fb_splits > 1) e = cudaMalloc((void **)&b->d_part, B * 2 * b->fb_splits * 128);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_stat, B * 128);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_wsum, B * DYN_W * 128);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_bad, B * 4);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_dyn, B * (2 * lg + 1) * 96);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_proofs, B * bpp_ipa_proof_len(n));
+    if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_accept, B);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&b->d_tr, B * BPP_TRANSCRIPT_BYTES);
+    if (e != cudaSuccess) {
+        ctx->last_error = cudaGetErrorString(e);
+        bool oom = e == cudaErrorMemoryAllocation;
+        cudaGetLastError();
+        bpp_ipa_batch_free(b);
+        return oom ? BPP_ERR_OOM : BPP_ERR_CUDA;
+    }
+    *out = b;
+    return BPP_OK;
+}
+
+// canonical (< l) scalars; nearly every one is decided by its top byte
+static bool ipa_all_canonical(const uint8_t *s, size_t cnt) {
+    for (size_t i = 0; i < cnt; i++)
+        if (s[32 * i + 31] >= 0x10 && !acp_scalar_is_canonical(s + 32 * i)) return false;
+    return true;
+}
+// the checks prove and verify share; 0 or the status to return
+static int ipa_check_inputs(const bpp_ipa_batch *b, const uint8_t *q, const uint8_t *gf, const uint8_t *hf, const uint8_t *transcripts) {
+    const size_t B = b->B, n = b->n;
+    for (size_t p = 0; p < B; p++)
+        if (!tr_state_ok(transcripts + BPP_TRANSCRIPT_BYTES * p)) return BPP_ERR_INVALID_ARG;
+    if ((q && !ipa_all_canonical(q, B)) || (gf && !ipa_all_canonical(gf, B * n)) || (hf && !ipa_all_canonical(hf, B * n)))
+        return BPP_ERR_SCALAR_RANGE;
+    return BPP_OK;
+}
+// uploads q and the factors (NULL = ones) and the transcripts, places them in the proof blocks
+static int ipa_upload_common(bpp_ipa_batch *b, const uint8_t *q, const uint8_t *gf, const uint8_t *hf, const uint8_t *transcripts,
+                             const uint32_t *d_a, const uint32_t *d_b) {
+    bpp_ctx *ctx = b->ctx;
+    cudaStream_t s = ctx->stream;
+    const size_t B = b->B, n = b->n, vec = B * n * 32;
+    uint8_t *d_gf = b->d_in + 2 * vec, *d_hf = b->d_in + 3 * vec, *d_q = b->d_in + 4 * vec;
+    if (gf) CK(ctx, cudaMemcpyAsync(d_gf, gf, vec, cudaMemcpyHostToDevice, s));
+    if (hf) CK(ctx, cudaMemcpyAsync(d_hf, hf, vec, cudaMemcpyHostToDevice, s));
+    if (q) CK(ctx, cudaMemcpyAsync(d_q, q, B * 32, cudaMemcpyHostToDevice, s));
+    CK(ctx, cudaMemcpyAsync(b->d_tr, transcripts, B * BPP_TRANSCRIPT_BYTES, cudaMemcpyHostToDevice, s));
+    k_ipa_place<<<dim3((4 * b->n + 1 + 127) / 128, b->B), 128, 0, s>>>(d_a, d_b, gf ? (const uint32_t *)d_gf : nullptr,
+                                                                     hf ? (const uint32_t *)d_hf : nullptr,
+                                                                     q ? (const uint32_t *)d_q : nullptr, b->lay, b->d_blk);
+    LAUNCH_CHECK(ctx);
+    return BPP_OK;
+}
+static fb_plan ipa_fb_plan(const bpp_ipa_batch *b, const fb_shape &sh) {
+    return fb_choose(b->ctx, (uint64_t)b->B * sh.outs, fb_terms(sh), b->gens->fb_Wn, !sh.sel_period, sh.outs > 8 ? 1 : b->fb_splits);
+}
+
+extern "C" int bpp_ipa_batch_prove(bpp_ipa_batch *b, const uint8_t *q, const uint8_t *G_factors, const uint8_t *H_factors,
+                                   const uint8_t *a, const uint8_t *b_vec, uint8_t *transcripts, uint8_t *proofs_out) {
+    if (!b || !a || !b_vec || !transcripts || !proofs_out) return BPP_ERR_INVALID_ARG;
+    bpp_ctx *ctx = b->ctx;
+    const size_t B = b->B, n = b->n, vec = B * n * 32;
+    int rc;
+    if ((rc = ipa_check_inputs(b, q, G_factors, H_factors, transcripts))) return rc;
+    if (!ipa_all_canonical(a, B * n) || !ipa_all_canonical(b_vec, B * n)) return BPP_ERR_SCALAR_RANGE;
+    CK(ctx, cudaSetDevice(ctx->device));
+    if (!b->gens->fb_table && (rc = bpp_points_precompute(ctx, b->gens, 8))) return rc;
+    cudaStream_t s = ctx->stream;
+    const acp_layout &L = b->lay;
+    ipa_mark(b, "start");
+    CK(ctx, cudaMemcpyAsync(b->d_in, a, vec, cudaMemcpyHostToDevice, s));
+    CK(ctx, cudaMemcpyAsync(b->d_in + vec, b_vec, vec, cudaMemcpyHostToDevice, s));
+    if ((rc = ipa_upload_common(b, q, G_factors, H_factors, transcripts, (const uint32_t *)b->d_in, (const uint32_t *)(b->d_in + vec))))
+        return rc;
+    ipa_mark(b, "upload");
+    TR_LAUNCH(k_ipa_start, b->B, s, b->n, b->B, b->d_tr);
+    LAUNCH_CHECK(ctx);
+    ipa_mark(b, "dom-sep");
+    if (b->lg) {
+        ipa_rounds_io io;
+        io.blk = b->d_blk; io.lr = b->d_lr; io.lrext = b->d_lrext; io.part = b->d_part; io.tr = b->d_tr;
+        io.gG = b->g_off; io.gH = b->h_off; io.gQ = b->q_off;
+        io.gf = true;
+        auto fb = [&](const fb_shape &sh, uint32_t *dst, uint32_t pitch, uint32_t *split_n) {
+            return fb_launch(ctx, b->d_blk, L, b->B, *b->gens, sh, ipa_fb_plan(b, sh), dst, pitch, s, b->d_part, split_n);
+        };
+        if ((rc = ipa_prove_rounds(ctx, L, b->B, io, fb, std::function<int(uint32_t)>()))) return rc;
+    }
+    ipa_mark(b, "inner-product rounds");
+    const size_t plen = bpp_ipa_proof_len(n);
+    k_ipa_pack<<<(unsigned)((B * (plen / 32) + 127) / 128), 128, 0, s>>>(L, b->d_lr, b->d_blk, b->B, b->d_proofs);
+    LAUNCH_CHECK(ctx);
+    CK(ctx, cudaMemcpyAsync(proofs_out, b->d_proofs, B * plen, cudaMemcpyDeviceToHost, s));
+    CK(ctx, cudaMemcpyAsync(transcripts, b->d_tr, B * BPP_TRANSCRIPT_BYTES, cudaMemcpyDeviceToHost, s));
+    ipa_mark(b, "pack+download");
+    CK(ctx, cudaStreamSynchronize(s));
+    ipa_marks_dump(b, "prove");
+    return BPP_OK;
+}
+
+extern "C" int bpp_ipa_batch_verify(bpp_ipa_batch *b, const uint8_t *q, const uint8_t *G_factors, const uint8_t *H_factors,
+                                    const uint8_t *P, const uint8_t *proofs, uint8_t *transcripts, uint8_t *accept) {
+    if (!b || !P || !proofs || !transcripts || !accept) return BPP_ERR_INVALID_ARG;
+    bpp_ctx *ctx = b->ctx;
+    const size_t B = b->B, n = b->n, lg = b->lg, plen = bpp_ipa_proof_len(n), per = 2 * lg + 1;
+    int rc;
+    if ((rc = ipa_check_inputs(b, q, G_factors, H_factors, transcripts))) return rc;
+    CK(ctx, cudaSetDevice(ctx->device));
+    if (!b->gens->fb_table && (rc = bpp_points_precompute(ctx, b->gens, 8))) return rc;
+    cudaStream_t s = ctx->stream;
+    const acp_layout &L = b->lay;
+    ipa_mark(b, "start");
+    // the proofs go where the prover stages a and b, P after q
+    uint8_t *d_pr = b->d_in, *d_P = b->d_in + (4 * n + 1) * B * 32;
+    CK(ctx, cudaMemcpyAsync(d_pr, proofs, B * plen, cudaMemcpyHostToDevice, s));
+    CK(ctx, cudaMemcpyAsync(d_P, P, B * 32, cudaMemcpyHostToDevice, s));
+    if ((rc = ipa_upload_common(b, q, G_factors, H_factors, transcripts, nullptr, nullptr))) return rc;
+    CK(ctx, cudaMemsetAsync(b->d_bad, 0, B * 4, s));
+    ipa_mark(b, "upload");
+    k_ipa_unpack<<<(unsigned)((B * (plen / 32) + 127) / 128), 128, 0, s>>>(L, d_pr, d_P, b->B, b->d_blk, b->d_lr, b->d_bad);
+    LAUNCH_CHECK(ctx);
+    k_acp_decompress_lr<<<(unsigned)((B * per + 127) / 128), 128, 0, s>>>(b->d_lr, (uint32_t)per, 2 * b->lg, 0, (uint32_t)per, b->B,
+                                                                         b->d_dyn, b->d_bad);
+    LAUNCH_CHECK(ctx);
+    TR_LAUNCH(k_ipa_vtranscript, b->B, s, b->d_lr, L, b->B, b->d_tr, b->d_blk);
+    LAUNCH_CHECK(ctx);
+    k_ipa_vprep<<<(b->B + 63) / 64, 64, 0, s>>>(L, b->B, 0, b->d_blk);
+    LAUNCH_CHECK(ctx);
+    k_ipa_stable_full<<<b->B, n >= IPA_ROUND_THREADS ? IPA_ROUND_THREADS : (n < 128 ? 128 : (unsigned)n), 0, s>>>(L, b->d_blk);
+    LAUNCH_CHECK(ctx);
+    k_ipa_vscal<<<dim3((b->n + 1 + 127) / 128, b->B), 128, 0, s>>>(L, b->d_blk);
+    LAUNCH_CHECK(ctx);
+    {
+        fb_shape sh = acp_shape(1);
+        acp_seg(sh, L.vG, 0, b->g_off, b->n);
+        acp_seg(sh, L.vH, 0, b->h_off, b->n);
+        acp_seg(sh, L.cl, 0, b->q_off, 1);
+        if ((rc = fb_launch(ctx, b->d_blk, L, b->B, *b->gens, sh, ipa_fb_plan(b, sh), b->d_stat, 1, s, b->d_part, nullptr))) return rc;
+    }
+    k_dyn_window_sums<<<b->B, DYN_W, 0, s>>>(b->d_blk, L, b->d_dyn, (uint32_t)per, b->d_wsum);
+    LAUNCH_CHECK(ctx);
+    k_ipa_accept<<<(b->B + 63) / 64, 64, 0, s>>>(b->B, b->d_wsum, b->d_stat, b->d_bad, b->d_accept);
+    LAUNCH_CHECK(ctx);
+    ipa_mark(b, "check");
+    CK(ctx, cudaMemcpyAsync(accept, b->d_accept, B, cudaMemcpyDeviceToHost, s));
+    CK(ctx, cudaMemcpyAsync(transcripts, b->d_tr, B * BPP_TRANSCRIPT_BYTES, cudaMemcpyDeviceToHost, s));
+    ipa_mark(b, "download");
+    CK(ctx, cudaStreamSynchronize(s));
+    ipa_marks_dump(b, "verify");
     return BPP_OK;
 }

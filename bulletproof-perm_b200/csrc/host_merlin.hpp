@@ -51,6 +51,11 @@ class Strobe128 {
         cur_flags_ = 0;
         meta_ad((const uint8_t *)protocol_label, strlen(protocol_label), false);
     }
+    // the state of export_state, continued (bpp_transcript_* carry a transcript across the C ABI in this form)
+    explicit Strobe128(const uint64_t in[26]) : pos_(0), pos_begin_(0), cur_flags_(0) {
+        memset(st_, 0, 200);
+        import_state(in);
+    }
     void meta_ad(const uint8_t *d, size_t n, bool more) { begin_op(kM | kA, more); absorb(d, n); }
     void ad(const uint8_t *d, size_t n, bool more) { begin_op(kA, more); absorb(d, n); }
     void prf(uint8_t *out, size_t n, bool more) { begin_op(kI | kA | kC, more); squeeze(out, n); }
@@ -58,6 +63,21 @@ class Strobe128 {
     void export_state(uint64_t out[26]) const {
         memcpy(out, st_, 200);
         out[25] = (uint64_t)pos_ | ((uint64_t)pos_begin_ << 8) | ((uint64_t)cur_flags_ << 16);
+    }
+    // false for a word 25 no export could have written (pos, pos_begin beyond the rate, high bits set)
+    static bool state_valid(const uint64_t in[26]) {
+        const uint64_t w = in[25];
+        return !(w >> 24) && (w & 0xff) < kR && ((w >> 8) & 0xff) <= kR;
+    }
+    // false (state unchanged) if !state_valid(in)
+    bool import_state(const uint64_t in[26]) {
+        if (!state_valid(in)) return false;
+        const uint64_t w = in[25];
+        memcpy(st_, in, 200);
+        pos_ = (uint8_t)w;
+        pos_begin_ = (uint8_t)(w >> 8);
+        cur_flags_ = (uint8_t)(w >> 16);
+        return true;
     }
 
   private:
@@ -107,9 +127,12 @@ class Strobe128 {
 class Transcript {
   public:
     Transcript(const uint8_t *label, size_t n) : strobe_("Merlin v1.0") { append_message("dom-sep", label, n); }
-    void append_message(const char *label, const uint8_t *msg, size_t n) {
+    explicit Transcript(const uint64_t state[26]) : strobe_(state) {}
+    void append_message(const char *label, const uint8_t *msg, size_t n) { append_message(label, strlen(label), msg, n); }
+    // labels with an explicit length (merlin's labels are &'static [u8]: any bytes, NUL included)
+    void append_message(const char *label, size_t label_len, const uint8_t *msg, size_t n) {
         uint8_t len[4] = {(uint8_t)n, (uint8_t)(n >> 8), (uint8_t)(n >> 16), (uint8_t)(n >> 24)};
-        strobe_.meta_ad((const uint8_t *)label, strlen(label), false);
+        strobe_.meta_ad((const uint8_t *)label, label_len, false);
         strobe_.meta_ad(len, 4, true);
         strobe_.ad(msg, n, false);
     }
@@ -118,9 +141,10 @@ class Transcript {
         for (int i = 0; i < 8; i++) b[i] = (uint8_t)(x >> (8 * i));
         append_message(label, b, 8);
     }
-    void challenge_bytes(const char *label, uint8_t *out, size_t n) {
+    void challenge_bytes(const char *label, uint8_t *out, size_t n) { challenge_bytes(label, strlen(label), out, n); }
+    void challenge_bytes(const char *label, size_t label_len, uint8_t *out, size_t n) {
         uint8_t len[4] = {(uint8_t)n, (uint8_t)(n >> 8), (uint8_t)(n >> 16), (uint8_t)(n >> 24)};
-        strobe_.meta_ad((const uint8_t *)label, strlen(label), false);
+        strobe_.meta_ad((const uint8_t *)label, label_len, false);
         strobe_.meta_ad(len, 4, true);
         strobe_.prf(out, n, false);
     }
@@ -142,6 +166,7 @@ class Transcript {
     // (k_scalar_from_wide) or through reduce_wide() below for single values.
     void challenge_wide(const char *label, uint8_t out64[64]) { challenge_bytes(label, out64, 64); }
     void export_state(uint64_t out[26]) const { strobe_.export_state(out); }
+    bool import_state(const uint64_t in[26]) { return strobe_.import_state(in); }
 
   private:
     Strobe128 strobe_;

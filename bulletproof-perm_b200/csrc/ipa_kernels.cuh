@@ -82,7 +82,11 @@ SC_INLINE uint32_t *ipa_stab(uint32_t *blk, const acp_layout &lay, uint32_t p, u
 // fold happens (a, b are l[0], r[0]).  The two barriers are cluster barriers (release/acquire at cluster scope: the
 // folded vectors and the table written by one CTA are read by the others); the CTAs' partial inner products meet in
 // rank 0 through distributed shared memory.
-__global__ void __launch_bounds__(IPA_ROUND_THREADS) k_ipa_round(acp_layout lay, int round, uint32_t *__restrict__ blk) {
+// GF: the stand-alone inner-product batch (bpp_ipa_batch_*), whose G generators carry per-proof factors (dalek's G_factors,
+// held at lay.yn there): the G-side MSM scalars are multiplied by them as the H side's are by lay.yninv.  k_ipa_round (the
+// `fixed` mode, G_factors = 1) is the GF = false instance.
+template <bool GF>
+__device__ __forceinline__ void ipa_round_body(const acp_layout &lay, int round, uint32_t *__restrict__ blk) {
     namespace cg = cooperative_groups;
     __shared__ __align__(16) uint32_t sh[32 * 8];
     __shared__ __align__(16) uint32_t part[2 * 8];     // this CTA's share of the two inner products (Montgomery sums)
@@ -152,6 +156,11 @@ __global__ void __launch_bounds__(IPA_ROUND_THREADS) k_ipa_round(acp_layout lay,
         sc_load(b, ACP_PTR(blk, lay, p, lay.r + ip));
         sc_load(yi, ACP_PTR(blk, lay, p, lay.yninv + g));
         sc_mont(r, a, s);                              // a * s_t (s in Montgomery form -> standard result)
+        if (GF) {
+            sc gf;
+            sc_load(gf, ACP_PTR(blk, lay, p, lay.yn + g));
+            sc_mul(r, r, gf);
+        }
         sc_store(ACP_PTR(blk, lay, p, lay.vG + g), r);
         sc_mont(r, b, sinv);
         sc_mul(r, r, yi);
@@ -175,14 +184,21 @@ __global__ void __launch_bounds__(IPA_ROUND_THREADS) k_ipa_round(acp_layout lay,
     }
     cluster.sync();                                    // no CTA leaves while rank 0 reads its shared memory
 }
-// launch: cluster of `C` CTAs per proof
-static inline cudaError_t ipa_round_launch(acp_layout lay, int round, uint32_t *blk, uint32_t B, cudaStream_t s) {
+__global__ void __launch_bounds__(IPA_ROUND_THREADS) k_ipa_round(acp_layout lay, int round, uint32_t *__restrict__ blk) {
+    ipa_round_body<false>(lay, round, blk);
+}
+__global__ void __launch_bounds__(IPA_ROUND_THREADS) k_ipa_round_gf(acp_layout lay, int round, uint32_t *__restrict__ blk) {
+    ipa_round_body<true>(lay, round, blk);
+}
+// launch: cluster of `C` CTAs per proof; gf: the k_ipa_round_gf instance
+static inline cudaError_t ipa_round_launch(acp_layout lay, int round, uint32_t *blk, uint32_t B, cudaStream_t s, bool gf = false) {
     const uint32_t np = lay.np;
     const unsigned threads = np >= IPA_ROUND_THREADS ? IPA_ROUND_THREADS : (np < 128 ? 128 : np);
     unsigned C = 1;
     while (C < 8 && (size_t)C * 1024 < np) C <<= 1;
+    void (*kern)(acp_layout, int, uint32_t *) = gf ? k_ipa_round_gf : k_ipa_round;
     if (C == 1) {
-        k_ipa_round<<<B, threads, 0, s>>>(lay, round, blk);
+        kern<<<B, threads, 0, s>>>(lay, round, blk);
         return cudaGetLastError();
     }
     cudaLaunchConfig_t cfg = {};
@@ -196,7 +212,7 @@ static inline cudaError_t ipa_round_launch(acp_layout lay, int round, uint32_t *
     at[0].val.clusterDim.z = 1;
     cfg.attrs = at;
     cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, k_ipa_round, lay, round, blk);
+    return cudaLaunchKernelEx(&cfg, kern, lay, round, blk);
 }
 // ---- K7: explicit generator folding (SURVEY 2.3 / D.3; bulletproofs 4.0.0 inner_product_proof.rs create():
 // G'_i = u^-1 G_i + u G_{i + n/2}).  NOT on the prover's path - the rounds above fold the scalars and keep the original
@@ -351,8 +367,9 @@ __global__ void k_acp_put_wide_strided(const uint32_t *__restrict__ wide, acp_la
     const uint32_t off = k == 0 ? lay.y : k == 1 ? lay.z : k == 2 ? lay.x : k == 3 ? lay.wq : lay.u + (k - 4);
     sc_store(ACP_PTR(blk, lay, p, off), r);
 }
-// thread per proof: u_j^-1 for all rounds with one inversion; u, uinv in Montgomery form; usq, uinvsq standard
-__global__ void __launch_bounds__(64) k_ipa_vprep(acp_layout lay, uint32_t B, uint32_t *__restrict__ blk) {
+// thread per proof: u_j^-1 for all rounds with one inversion; u, uinv in Montgomery form; usq, uinvsq standard at
+// lay.vd + first + 2 k, + 1 (`fixed` mode: first = m + 8, after the commitments and the eight proof points)
+__global__ void __launch_bounds__(64) k_ipa_vprep(acp_layout lay, uint32_t B, uint32_t first, uint32_t *__restrict__ blk) {
     uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= B) return;
     uint32_t *u = ACP_PTR(blk, lay, p, lay.u), *ui = ACP_PTR(blk, lay, p, lay.uinv);
@@ -382,10 +399,10 @@ __global__ void __launch_bounds__(64) k_ipa_vprep(acp_layout lay, uint32_t B, ui
         sc_store(ui + 8 * (size_t)k, r);
         sc_mont_noinline(sq, e, e);
         sc_from_mont(sq, sq);
-        sc_store(ACP_PTR(blk, lay, p, lay.vd + lay.m + 8 + 2 * k), sq);          // L_k: u_k^2
+        sc_store(ACP_PTR(blk, lay, p, lay.vd + first + 2 * k), sq);              // L_k: u_k^2
         sc_mont_noinline(sq, r, r);
         sc_from_mont(sq, sq);
-        sc_store(ACP_PTR(blk, lay, p, lay.vd + lay.m + 8 + 2 * k + 1), sq);      // R_k: u_k^-2
+        sc_store(ACP_PTR(blk, lay, p, lay.vd + first + 2 * k + 1), sq);          // R_k: u_k^-2
     }
 }
 // Scalars of the fused check (SURVEY D.1, `fixed` layout; rho = per-proof verifier weight on check 2):
@@ -488,19 +505,20 @@ __global__ void __launch_bounds__(128) k_acp_vscal_fixed(acp_layout lay, uint32_
         for (int k = 0; k < 3; k++) sc_store(ACP_PTR(blk, lay, p, lay.vd + lay.m + 5 + k), xp[k + 1]);
     }
 }
-// extra dynamic points of `fixed` mode: L_k, R_k (an identity encoding is rejected like
-// validate_and_append_point, an invalid one like decompress() = None)
-__global__ void __launch_bounds__(128) k_acp_decompress_lr(const uint8_t *__restrict__ lr, uint32_t m, uint32_t lg, uint32_t B,
-                                                           uint32_t *__restrict__ dyn, uint32_t *__restrict__ bad) {
-    const uint32_t per = m + 8 + 2 * lg;
+// extra dynamic points: `cnt` encodings per proof (lr: B x cnt x 32) into slots first .. first + cnt of the proof's `per`
+// dynamic points.  `fixed` mode: L_k, R_k after the commitments and the eight proof points; the stand-alone
+// inner-product verifier: L_k, R_k, P.  Entries below `nonzero` reject an identity encoding (validate_and_append_point),
+// every entry an invalid one (decompress() = None).
+__global__ void __launch_bounds__(128) k_acp_decompress_lr(const uint8_t *__restrict__ lr, uint32_t cnt, uint32_t nonzero, uint32_t first,
+                                                           uint32_t per, uint32_t B, uint32_t *__restrict__ dyn, uint32_t *__restrict__ bad) {
     uint32_t id = blockIdx.x * blockDim.x + threadIdx.x;
-    if (id >= B * 2 * lg) return;
-    const uint32_t p = id / (2 * lg), k = id - p * 2 * lg;
+    if (id >= B * cnt) return;
+    const uint32_t p = id / cnt, k = id - p * cnt;
     const uint8_t *src = lr + 32 * (size_t)id;
     uint32_t any = 0;
     for (int b = 0; b < 32; b++) any |= src[b];
     fe x, y;
-    bool ok = ge_decompress(x, y, src) && any != 0;
+    bool ok = ge_decompress(x, y, src) && (any != 0 || k >= nonzero);
     if (!ok) {
         atomicOr(&bad[p], 1u);
         fe_set0(x);
@@ -508,5 +526,119 @@ __global__ void __launch_bounds__(128) k_acp_decompress_lr(const uint8_t *__rest
     }
     ge_niels q;
     ge_affine_to_niels(q, x, y);
-    ge_niels_store(dyn + 24 * ((size_t)p * per + m + 8 + k), q);
+    ge_niels_store(dyn + 24 * ((size_t)p * per + first + k), q);
+}
+
+// ---- stand-alone inner-product batch (bpp_ipa_batch_*; bulletproofs 4.0.0 inner_product_proof.rs create / verify) ----
+// The proof block holds the inner-product fields of acp_layout only (ipa_make_layout, capi_acproof.cu): a, b at lay.l,
+// lay.r (folded in place by the prover; lay.pa, lay.pb for the verifier), H_factors at lay.yninv, G_factors at lay.yn
+// (k_ipa_round_gf), q at lay.wq - so that k_ipa_round's "w c_L" is the Q coefficient of Q = q gens[q_off] - and the
+// round state u, uinv, stab, vG, vH, cl.  The verifier's dynamic scalars sit at lay.vd: u_k^2, u_k^-2 (k_ipa_vprep with
+// first = 0), then -1 for P.
+
+// contiguous staged inputs (count x n scalars each; q: count x 1) -> proof blocks.  A null a / b is skipped (verifier),
+// a null factor vector or q stands for all ones.  Grid (ceil((4 n + 1) / 128), B).
+__global__ void __launch_bounds__(128) k_ipa_place(const uint32_t *__restrict__ a, const uint32_t *__restrict__ b,
+                                                   const uint32_t *__restrict__ gf, const uint32_t *__restrict__ hf,
+                                                   const uint32_t *__restrict__ q, acp_layout lay, uint32_t *__restrict__ blk) {
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x, p = blockIdx.y, n = lay.np;
+    if (j > 4 * n) return;
+    const uint32_t which = j == 4 * n ? 4 : j / n, i = j - which * n;
+    const uint32_t *src = which == 0 ? a : which == 1 ? b : which == 2 ? gf : which == 3 ? hf : q;
+    if (!src && which < 2) return;
+    const uint32_t dst = which == 0 ? lay.l : which == 1 ? lay.r : which == 2 ? lay.yn : which == 3 ? lay.yninv : lay.wq;
+    sc v;
+    if (src) sc_load(v, src + 8 * ((size_t)p * (which == 4 ? 1 : n) + i));
+    else sc_set_u32(v, 1);
+    sc_store(ACP_PTR(blk, lay, p, dst + i), v);
+}
+// prover: proof p = L_0 R_0 .. L_{lg-1} R_{lg-1} a b (InnerProductProof::to_bytes); lr: B x 2 lg x 32
+__global__ void __launch_bounds__(128) k_ipa_pack(acp_layout lay, const uint8_t *__restrict__ lr, const uint32_t *__restrict__ blk,
+                                                  uint32_t B, uint8_t *__restrict__ out) {
+    const uint32_t words = 2 * lay.lg + 2, id = blockIdx.x * blockDim.x + threadIdx.x;
+    if (id >= B * words) return;
+    const uint32_t p = id / words, i = id - p * words;
+    const uint4 *s = i < 2 * lay.lg ? reinterpret_cast<const uint4 *>(lr + 32 * ((size_t)p * 2 * lay.lg + i))
+                                    : reinterpret_cast<const uint4 *>(ACP_PTR(blk, lay, p, i == 2 * lay.lg ? lay.l : lay.r));
+    uint4 *d = reinterpret_cast<uint4 *>(out + 32 * (size_t)id);
+    d[0] = s[0];
+    d[1] = s[1];
+}
+// verifier: proofs (B x (2 lg + 2) x 32) and P (B x 32) -> lrp (B x (2 lg + 1) x 32: L_0 R_0 .. P) and a, b at lay.pa,
+// lay.pb.  An a or b >= l rejects the proof (InnerProductProof::from_bytes refuses it): bad[p] |= 1.
+__global__ void __launch_bounds__(128) k_ipa_unpack(acp_layout lay, const uint8_t *__restrict__ proofs, const uint8_t *__restrict__ P,
+                                                    uint32_t B, uint32_t *__restrict__ blk, uint8_t *__restrict__ lrp,
+                                                    uint32_t *__restrict__ bad) {
+    const uint32_t words = 2 * lay.lg + 2, id = blockIdx.x * blockDim.x + threadIdx.x;
+    if (id >= B * words) return;
+    const uint32_t p = id / words, i = id - p * words;
+    if (i == words - 1) {   // b's thread also copies P
+        const uint4 *s = reinterpret_cast<const uint4 *>(P + 32 * (size_t)p);
+        uint4 *d = reinterpret_cast<uint4 *>(lrp + 32 * ((size_t)p * (words - 1) + words - 2));
+        d[0] = s[0];
+        d[1] = s[1];
+    }
+    const uint4 *s = reinterpret_cast<const uint4 *>(proofs + 32 * (size_t)id);
+    const uint4 lo = s[0], hi = s[1];
+    if (i < 2 * lay.lg) {
+        uint4 *d = reinterpret_cast<uint4 *>(lrp + 32 * ((size_t)p * (words - 1) + i));
+        d[0] = lo;
+        d[1] = hi;
+        return;
+    }
+    sc v;
+    v.v[0] = lo.x; v.v[1] = lo.y; v.v[2] = lo.z; v.v[3] = lo.w; v.v[4] = hi.x; v.v[5] = hi.y; v.v[6] = hi.z; v.v[7] = hi.w;
+    uint32_t l8[8], t[8];
+#pragma unroll
+    for (int k = 0; k < 8; k++) l8[k] = SC_L[k];
+    if (!sc_sub8(t, v.v, l8)) atomicOr(&bad[p], 1u);   // no borrow: v >= l
+    sc_reduce256(v, v);
+    sc_store(ACP_PTR(blk, lay, p, i == 2 * lay.lg ? lay.pa : lay.pb), v);
+}
+// verifier scalars of  -a s_i gf_i G_i - b s_i^-1 hf_i H_i - a b q Q + sum_k (u_k^2 L_k + u_k^-2 R_k) + P  (= identity iff
+// dalek's verify accepts): vG, vH (n each), cl[0] (Q), and vd[2 lg] = 1 (P).  s from k_ipa_stable_full.  Grid
+// (ceil((n + 1) / 128), B).
+__global__ void __launch_bounds__(128) k_ipa_vscal(acp_layout lay, uint32_t *__restrict__ blk) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x, p = blockIdx.y, n = lay.np;
+    if (i > n) return;
+    sc pa, pb, t, f;
+    sc_load(pa, ACP_PTR(blk, lay, p, lay.pa));
+    sc_load(pb, ACP_PTR(blk, lay, p, lay.pb));
+    if (i == n) {
+        sc_mul(t, pa, pb);
+        sc_load(f, ACP_PTR(blk, lay, p, lay.wq));
+        sc_mul(t, t, f);
+        sc_neg(t, t);
+        sc_store(ACP_PTR(blk, lay, p, lay.cl), t);
+        sc_set_u32(t, 1);
+        sc_store(ACP_PTR(blk, lay, p, lay.vd + 2 * lay.lg), t);
+        return;
+    }
+    sc s;
+    const uint32_t *st = ipa_stab(blk, lay, p, lay.lg);
+    sc_load(s, st + 8 * (size_t)i);
+    sc_mont(t, pa, s);                           // a s_i
+    sc_load(f, ACP_PTR(blk, lay, p, lay.yn + i));
+    sc_mul(t, t, f);
+    sc_neg(t, t);
+    sc_store(ACP_PTR(blk, lay, p, lay.vG + i), t);
+    sc_load(s, st + 8 * (size_t)(n - 1 - i));
+    sc_mont(t, pb, s);                           // b s_i^-1
+    sc_load(f, ACP_PTR(blk, lay, p, lay.yninv + i));
+    sc_mul(t, t, f);
+    sc_neg(t, t);
+    sc_store(ACP_PTR(blk, lay, p, lay.vH + i), t);
+}
+// thread per proof: the dynamic part (k_dyn_window_sums) plus the fixed-base part must be the identity, and no encoding or
+// scalar may have been refused
+__global__ void __launch_bounds__(64) k_ipa_accept(uint32_t B, const uint32_t *__restrict__ wsum, const uint32_t *__restrict__ stat_ext,
+                                                   const uint32_t *__restrict__ bad, uint8_t *__restrict__ accept) {
+    uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= B) return;
+    ge_ext acc, t;
+    dyn_horner(acc, wsum, p);
+    ge_load(t, stat_ext + 32 * (size_t)p);
+    ge_add(acc, acc, t);
+    const bool ident = fe_is_zero(acc.X) || fe_is_zero(acc.Y);  // the Ristretto identity coset
+    accept[p] = (ident && bad[p] == 0) ? 1 : 0;
 }

@@ -221,6 +221,44 @@ __global__ void __launch_bounds__(64) k_ipa_lr_tail(const uint32_t *__restrict__
     }
 }
 
+// Stand-alone inner-product batch (bpp_ipa_batch_*): the caller's transcripts, uploaded in `states`, get
+// innerproduct_domain_sep(n) - dom-sep "ipp v1", u64 "n" - in place (InnerProductProof::create and
+// verification_scalars both start so).
+template <class T>
+__global__ void __launch_bounds__(TR_THREADS) k_ipa_start(uint32_t n, uint32_t B, uint64_t *__restrict__ states) {
+    const uint32_t p = tr_index<T>();
+    if (p >= B) return;
+    T t;
+    t.load(states + MERLIN_STATE_WORDS * (size_t)p);
+    t.append_message(MERLIN_LABEL("dom-sep"), (const uint8_t *)"ipp v1", 6);
+    t.append_u64(MERLIN_LABEL("n"), n);
+    t.store(states + MERLIN_STATE_WORDS * (size_t)p);
+}
+// Its verifier: verification_scalars' transcript steps on the uploaded states - the domain separator, then L_j, R_j ->
+// u_j (standard form at lay.u + j) for every round.  lrp: B x (2 lg + 1) x 32 (k_ipa_unpack).  An all-zero L_j or R_j
+// (validate_and_append_point refuses it) rejects the proof in k_acp_decompress_lr; the state is then left as if the
+// point had been appended, which dalek does not define.
+template <class T>
+__global__ void __launch_bounds__(TR_THREADS) k_ipa_vtranscript(const uint8_t *__restrict__ lrp, acp_layout lay, uint32_t B,
+                                                                uint64_t *__restrict__ states, uint32_t *__restrict__ blk) {
+    const uint32_t p = tr_index<T>();
+    if (p >= B) return;
+    T t;
+    t.load(states + MERLIN_STATE_WORDS * (size_t)p);
+    t.append_message(MERLIN_LABEL("dom-sep"), (const uint8_t *)"ipp v1", 6);
+    t.append_u64(MERLIN_LABEL("n"), lay.np);
+    sc c;
+#pragma unroll 1
+    for (uint32_t j = 0; j < lay.lg; j++) {
+        const uint8_t *q = lrp + 32 * ((size_t)(2 * lay.lg + 1) * p + 2 * j);
+        t.append_message(MERLIN_LABEL("L"), q, 32);
+        t.append_message(MERLIN_LABEL("R"), q + 32, 32);
+        t.challenge_scalar(MERLIN_LABEL("u"), c);
+        if (t.lane == 0) sc_store(ACP_PTR(blk, lay, p, lay.u + j), c);
+    }
+    t.store(states + MERLIN_STATE_WORDS * (size_t)p);
+}
+
 // Verifier: replays the whole transcript of one proof and leaves its final state in `states` (k_tr_weights continues
 // it).  tx3 (B x 3 x 32: t_x, t_x_blinding, e_blinding, reduced) and lr are used in `fixed` mode only (lay.lg > 0).
 template <class T>

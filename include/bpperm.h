@@ -330,6 +330,52 @@ int bpp_transcript_script(bpp_ctx *ctx, const uint8_t *script, size_t len, uint8
 /* measurement hook: the A_I-shaped fixed-base MSM kernel alone, timed with CUDA events over `reps` launches */
 int bpp_acp_batch_time_commit_msm(bpp_acp_batch *b, int reps, float *ms_avg, uint64_t *mixed_adds, uint64_t *full_adds);
 
+/* ---- transcripts across the ABI (host only: no context, no device) ------------------------------------------
+ * merlin 3.0.0 Transcript (the `&mut Transcript` of bulletproofs' inner_product_proof.rs) as a caller-held state of
+ * BPP_TRANSCRIPT_BYTES: 26 little-endian u64, the 25 Keccak-f[1600] lanes of the STROBE-128 sponge, then
+ * pos | pos_begin << 8 | cur_flags << 16.  A state no transcript could be in (pos or pos_begin beyond the rate)
+ * is BPP_ERR_INVALID_ARG.  Labels are byte strings of label_len bytes (merlin's &'static [u8]). */
+#define BPP_TRANSCRIPT_BYTES 208
+/* Transcript::new(label) */
+int bpp_transcript_new(const uint8_t *label, size_t label_len, uint8_t state[BPP_TRANSCRIPT_BYTES]);
+/* Transcript::append_message(label, msg) */
+int bpp_transcript_append_message(uint8_t state[BPP_TRANSCRIPT_BYTES], const uint8_t *label, size_t label_len,
+                                  const uint8_t *msg, size_t msg_len);
+/* Transcript::challenge_bytes(label, out) */
+int bpp_transcript_challenge_bytes(uint8_t state[BPP_TRANSCRIPT_BYTES], const uint8_t *label, size_t label_len,
+                                   uint8_t *out, size_t out_len);
+
+/* ---- stand-alone inner-product argument, batched ---------------------------------------------------------------
+ * bulletproofs 4.0.0 InnerProductProof::create / verify (inner_product_proof.rs; the crate keeps the module private)
+ * for `count` independent proofs of length n over caller generators and caller transcripts - what a caller needs to
+ * replace the 2n scalars l, r that circuit_lib.rs:464-468 sends in the clear by a proof of 2 lg n + 2 words.
+ * For proof p: G = gens[g_off .. g_off + n), H = gens[h_off .. h_off + n), Q_p = q_p * gens[q_off] (every use in dalek:
+ * the R1CS and range-proof verifiers take Q = w * B; an arbitrary per-proof Q is not supported).  gens is one tabled
+ * point set: the c = 8 window table is built on first use unless bpp_points_precompute ran.  n is a power of two, at
+ * most 8192.  Scalars are 32-byte little-endian; factor vectors are count x n x 32 (NULL = all ones), q count x 32
+ * (NULL = ones), transcripts count x BPP_TRANSCRIPT_BYTES, read and written back.  Host buffers; each call ends with one
+ * synchronisation.
+ * Errors, before any device work: n not a power of two or > 8192, NULL arguments, count == 0: BPP_ERR_INVALID_ARG; an
+ * offset range outside gens: BPP_ERR_LENGTH_MISMATCH; a scalar input >= l: BPP_ERR_SCALAR_RANGE. */
+typedef struct bpp_ipa_batch bpp_ipa_batch;
+/* 32 (2 lg n + 2): L_0 R_0 .. L_{lg n - 1} R_{lg n - 1} a b (InnerProductProof::to_bytes); 0 unless n is a power of two */
+size_t bpp_ipa_proof_len(size_t n);
+int bpp_ipa_batch_create(bpp_ctx *ctx, bpp_points *gens, size_t g_off, size_t h_off, size_t q_off, size_t n, size_t count,
+                         bpp_ipa_batch **out);
+void bpp_ipa_batch_free(bpp_ipa_batch *b);
+/* InnerProductProof::create(transcript, Q, G_factors, H_factors, G, H, a, b): from each transcript state, the domain
+ * separator ("dom-sep" "ipp v1", u64 "n") and the rounds; proofs_out count x bpp_ipa_proof_len(n); every transcript is
+ * left as create leaves it. */
+int bpp_ipa_batch_prove(bpp_ipa_batch *b, const uint8_t *q, const uint8_t *G_factors, const uint8_t *H_factors,
+                        const uint8_t *a, const uint8_t *b_vec, uint8_t *transcripts, uint8_t *proofs_out);
+/* InnerProductProof::verify(n, transcript, G_factors, H_factors, P, Q, G, H): P count x 32 compressed; accept[p] = 1 iff
+ * P_p = a b Q_p + sum a s_i gf_i G_i + sum b s_i^-1 hf_i H_i - sum u_j^2 L_j - sum u_j^-2 R_j.  A proof is rejected (0,
+ * not an error) when its a or b is >= l (from_bytes refuses it), an L_j or R_j is the all-zero encoding
+ * (validate_and_append_point) or L_j, R_j or P fails decoding.  The transcripts of accepted proofs are left as verify
+ * leaves them. */
+int bpp_ipa_batch_verify(bpp_ipa_batch *b, const uint8_t *q, const uint8_t *G_factors, const uint8_t *H_factors,
+                         const uint8_t *P, const uint8_t *proofs, uint8_t *transcripts, uint8_t *accept);
+
 /* ---- measurement helpers --------------------------------------------------------------------- */
 /* IMAD.WIDE.U32 peak microbenchmark: returns wide multiply-adds per second over all SMs. */
 int bpp_bench_imad_peak(bpp_ctx *ctx, int iters, double *ops_per_sec, double *ms);

@@ -79,6 +79,68 @@ impl GeneratorSet {
 }
 impl Drop for GeneratorSet { fn drop(&mut self) { with_ctx(|c| unsafe { sys::bpp_points_free(c, self.pts) }) } }
 
+/// A merlin `Transcript` held as the library's state (bpperm.h: bpp_transcript_*).  merlin::Transcript cannot be
+/// exported, so a caller that hands its protocol's inner-product argument to `InnerProductBatch` runs the transcript
+/// here: every append it makes to its own `Transcript` before the argument must be mirrored into this one.
+#[derive(Clone)]
+pub struct GpuTranscript { state: [u8; sys::BPP_TRANSCRIPT_BYTES] }
+impl GpuTranscript {
+    pub fn new(label: &'static [u8]) -> Self {
+        let mut state = [0u8; sys::BPP_TRANSCRIPT_BYTES];
+        assert_eq!(unsafe { sys::bpp_transcript_new(label.as_ptr(), label.len(), state.as_mut_ptr()) }, 0);
+        GpuTranscript { state }
+    }
+    pub fn append_message(&mut self, label: &'static [u8], message: &[u8]) {
+        assert_eq!(unsafe { sys::bpp_transcript_append_message(self.state.as_mut_ptr(), label.as_ptr(), label.len(), message.as_ptr(),
+                                                               message.len()) }, 0);
+    }
+    pub fn append_u64(&mut self, label: &'static [u8], x: u64) { self.append_message(label, &x.to_le_bytes()) }
+    pub fn challenge_bytes(&mut self, label: &'static [u8], dest: &mut [u8]) {
+        assert_eq!(unsafe { sys::bpp_transcript_challenge_bytes(self.state.as_mut_ptr(), label.as_ptr(), label.len(), dest.as_mut_ptr(),
+                                                                dest.len()) }, 0);
+    }
+}
+
+/// `count` inner-product proofs of length n (bulletproofs 4.0.0 `InnerProductProof::create` / `verify`) over a
+/// `GeneratorSet`: G = set[g_off..g_off + n), H = set[h_off..h_off + n), Q_p = q_p * set[q_off].
+pub struct InnerProductBatch { b: *mut sys::bpp_ipa_batch, count: usize, n: usize, proof_len: usize }
+impl InnerProductBatch {
+    pub fn new(gens: &GeneratorSet, g_off: usize, h_off: usize, q_off: usize, n: usize, count: usize) -> Self {
+        let mut b = std::ptr::null_mut();
+        let rc = with_ctx(|c| unsafe { sys::bpp_ipa_batch_create(c, gens.pts, g_off, h_off, q_off, n, count, &mut b) });
+        assert_eq!(rc, 0);
+        InnerProductBatch { b, count, n, proof_len: unsafe { sys::bpp_ipa_proof_len(n) } }
+    }
+    fn states(ts: &[GpuTranscript]) -> Vec<u8> { ts.iter().flat_map(|t| t.state.to_vec()).collect() }
+    fn opt(v: Option<&[Scalar]>) -> *const u8 { v.map_or(std::ptr::null(), |s| bytes_of(s).as_ptr()) }
+    /// create for every proof; a, b, factors: count x n (row-major), q: count; None = ones.  The transcripts advance as
+    /// create advances them.  Returns count proofs of `proof_len` bytes (InnerProductProof::to_bytes).
+    pub fn prove(&mut self, transcripts: &mut [GpuTranscript], q: Option<&[Scalar]>, g_factors: Option<&[Scalar]>,
+                 h_factors: Option<&[Scalar]>, a: &[Scalar], b: &[Scalar]) -> Vec<u8> {
+        assert!(transcripts.len() == self.count && a.len() == self.count * self.n && b.len() == self.count * self.n);
+        let mut st = Self::states(transcripts);
+        let mut proofs = vec![0u8; self.count * self.proof_len];
+        assert_eq!(unsafe { sys::bpp_ipa_batch_prove(self.b, Self::opt(q), Self::opt(g_factors), Self::opt(h_factors), bytes_of(a).as_ptr(),
+                                                     bytes_of(b).as_ptr(), st.as_mut_ptr(), proofs.as_mut_ptr()) }, 0);
+        for (t, s) in transcripts.iter_mut().zip(st.chunks_exact(sys::BPP_TRANSCRIPT_BYTES)) { t.state.copy_from_slice(s) }
+        proofs
+    }
+    /// verify for every proof; one Result per proof.  The transcripts of accepted proofs advance as verify advances them.
+    pub fn verify(&mut self, transcripts: &mut [GpuTranscript], q: Option<&[Scalar]>, g_factors: Option<&[Scalar]>,
+                  h_factors: Option<&[Scalar]>, p: &[CompressedRistretto], proofs: &[u8]) -> Vec<Result<(), ProofError>> {
+        assert!(transcripts.len() == self.count && p.len() == self.count && proofs.len() == self.count * self.proof_len);
+        let mut st = Self::states(transcripts);
+        let mut acc = vec![0u8; self.count];
+        assert_eq!(unsafe { sys::bpp_ipa_batch_verify(self.b, Self::opt(q), Self::opt(g_factors), Self::opt(h_factors),
+                                                      p.as_ptr() as *const u8, proofs.as_ptr(), st.as_mut_ptr(), acc.as_mut_ptr()) }, 0);
+        for ((t, s), a) in transcripts.iter_mut().zip(st.chunks_exact(sys::BPP_TRANSCRIPT_BYTES)).zip(&acc) {
+            if *a == 1 { t.state.copy_from_slice(s) }
+        }
+        acc.into_iter().map(|a| if a == 1 { Ok(()) } else { Err(ProofError::VerificationError) }).collect()
+    }
+}
+impl Drop for InnerProductBatch { fn drop(&mut self) { unsafe { sys::bpp_ipa_batch_free(self.b) } } }
+
 fn bytes_of(v: &[Scalar]) -> &[u8] { unsafe { std::slice::from_raw_parts(v.as_ptr() as *const u8, v.len() * 32) } }
 
 /// util.rs:84-94 (same panic text on a length mismatch)

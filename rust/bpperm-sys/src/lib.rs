@@ -8,6 +8,7 @@ use std::os::raw::{c_char, c_int};
 #[repr(C)] pub struct bpp_circuit { _p: [u8; 0] }
 #[repr(C)] pub struct bpp_gens { _p: [u8; 0] }
 #[repr(C)] pub struct bpp_acp_batch { _p: [u8; 0] }
+#[repr(C)] pub struct bpp_ipa_batch { _p: [u8; 0] }
 
 pub const BPP_OK: c_int = 0;
 pub const BPP_ERR_LENGTH_MISMATCH: c_int = -4;
@@ -17,6 +18,8 @@ pub const BPP_FMT_DALEK_XYZT: c_int = 2; // 160 B EdwardsPoint { X, Y, Z, T: Fie
 pub const MODE_REFERENCE: c_int = 0;
 pub const MODE_REFERENCE_FIXED: c_int = 1;
 pub const MODE_FIXED: c_int = 2;
+/// merlin Transcript state across the ABI: 25 Keccak lanes + pos | pos_begin << 8 | cur_flags << 16, little-endian u64
+pub const BPP_TRANSCRIPT_BYTES: usize = 208;
 
 extern "C" {
     pub fn bpp_init(device: c_int, out: *mut *mut bpp_ctx) -> c_int;
@@ -125,4 +128,18 @@ extern "C" {
     pub fn bpp_acp_batch_set_host_transcripts(b: *mut bpp_acp_batch, on: c_int) -> c_int;
     pub fn bpp_acp_batch_set_batch_rlc(b: *mut bpp_acp_batch, on: c_int) -> c_int;
     pub fn bpp_acp_batch_set_priority_split(b: *mut bpp_acp_batch, on: c_int) -> c_int;
+
+    // transcripts across the ABI (host only) and the stand-alone inner-product argument (inner_product_proof.rs)
+    pub fn bpp_transcript_new(label: *const u8, label_len: usize, state: *mut u8) -> c_int;
+    pub fn bpp_transcript_append_message(state: *mut u8, label: *const u8, label_len: usize, msg: *const u8, msg_len: usize) -> c_int;
+    pub fn bpp_transcript_challenge_bytes(state: *mut u8, label: *const u8, label_len: usize, out: *mut u8, out_len: usize) -> c_int;
+    pub fn bpp_ipa_proof_len(n: usize) -> usize;
+    pub fn bpp_ipa_batch_create(ctx: *mut bpp_ctx, gens: *mut bpp_points, g_off: usize, h_off: usize, q_off: usize, n: usize,
+                                count: usize, out: *mut *mut bpp_ipa_batch) -> c_int;
+    pub fn bpp_ipa_batch_free(b: *mut bpp_ipa_batch);
+    /// q, G_factors, H_factors nullable (= ones); transcripts: count x BPP_TRANSCRIPT_BYTES, in/out
+    pub fn bpp_ipa_batch_prove(b: *mut bpp_ipa_batch, q: *const u8, g_factors: *const u8, h_factors: *const u8, a: *const u8,
+                               b_vec: *const u8, transcripts: *mut u8, proofs_out: *mut u8) -> c_int;
+    pub fn bpp_ipa_batch_verify(b: *mut bpp_ipa_batch, q: *const u8, g_factors: *const u8, h_factors: *const u8, p: *const u8,
+                                proofs: *const u8, transcripts: *mut u8, accept: *mut u8) -> c_int;
 }

@@ -1,0 +1,177 @@
+"""Stand-alone inner-product batch (bpp_ipa_batch_*): prove and verify times at (count, n) = (4096, 128), (4096, 8) and
+(1, 8192), beside the inner-product rounds of the `fixed` mode prover on the same padded shape (52, 4 and 4096 cards),
+taken from its BPP_ACP_TRACE=1 stage timeline.  prove / verify: host clock around the C calls, which end in a device
+synchronisation (host input checks, pageable uploads and downloads included), after a warm-up; stage_median_ms: the
+batch's own BPP_ACP_TRACE=1 timeline (device events) in separate runs.  Inputs seeded.  Writes one JSON file (argv[1]) with the card name and power limit beside the numbers."""
+import ctypes
+import json
+import os
+import re
+import subprocess
+import sys
+import tempfile
+import time
+
+import numpy as np
+
+sys.path.insert(0, ".")
+import bpperm_b200  # noqa: E402
+
+L = 2 ** 252 + 27742317777372353535851937790883648493
+SHAPES = [(4096, 128), (4096, 8), (1, 8192)]
+REPS = int(os.environ.get("IPA_BENCH_REPS", "10"))
+
+
+def card():
+    try:
+        out = subprocess.check_output(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                                      text=True).strip().splitlines()[0]
+        name, pl, clk = [x.strip() for x in out.split(",")]
+        return {"gpu": name, "power_limit": pl, "max_sm_clock": clk}
+    except Exception as e:  # noqa: BLE001
+        return {"gpu": "unknown", "error": str(e)}
+
+
+def scalars(rs, cnt):
+    s = rs.randint(0, 256, size=(cnt, 32), dtype=np.uint8)
+    s[:, 31] &= 0x0F   # < 2^252 < l
+    return s
+
+
+def stderr_of(fn) -> str:
+    """what the library prints to file descriptor 2 while fn runs (its BPP_ACP_TRACE=1 stage lines)"""
+    with tempfile.TemporaryFile(mode="w+b") as f:
+        sys.stderr.flush()
+        saved = os.dup(2)
+        os.dup2(f.fileno(), 2)
+        try:
+            fn()
+        finally:
+            os.dup2(saved, 2)
+            os.close(saved)
+        f.seek(0)
+        return f.read().decode(errors="replace")
+
+
+def timed(fn, reps):
+    fn()   # warm-up
+    ts = []
+    for _ in range(reps):
+        t0 = time.perf_counter()
+        fn()
+        ts.append(time.perf_counter() - t0)
+    return {"median_ms": 1e3 * float(np.median(ts)), "min_ms": 1e3 * min(ts), "max_ms": 1e3 * max(ts), "reps": reps}
+
+
+def ipa_shape(be, count, n, rs):
+    Ipa = bpperm_b200.ipa
+    pts = be.points_from_uniform(rs.randint(0, 256, size=(2 * n + 1, 64), dtype=np.uint8).tobytes())   # G | H | Q
+    a, b = scalars(rs, count * n), scalars(rs, count * n)
+    A = a.reshape(count, n, 32)
+    Bv = b.reshape(count, n, 32)
+    # P = <a, G> + <b, H> + <a, b> Q through the library's batched table MSM
+    c = []
+    for p in range(count):
+        av = [int.from_bytes(A[p, i].tobytes(), "little") for i in range(n)]
+        bv = [int.from_bytes(Bv[p, i].tobytes(), "little") for i in range(n)]
+        c.append((sum(x * y for x, y in zip(av, bv)) % L).to_bytes(32, "little"))
+    msm_sc = b"".join(A[p].tobytes() + Bv[p].tobytes() + c[p] for p in range(count))
+    P = be.msm_batch(msm_sc, pts, 2 * n + 1, count)
+    bt = Ipa.InnerProductBatch(be, pts, 0, n, 2 * n, n, count)
+    states = Ipa.Transcript(b"ipa-bench").state * count
+    st = ctypes.create_string_buffer(len(states))
+    proofs = ctypes.create_string_buffer(bt.proof_len * count)
+    acc = ctypes.create_string_buffer(count)
+    ab, bb = a.tobytes(), b.tobytes()
+    lib = be._lib
+
+    def prove():   # the C call alone: the states are reset in place, nothing else is converted
+        ctypes.memmove(st, states, len(states))
+        be._check(lib.bpp_ipa_batch_prove(bt._h, None, None, None, ab, bb, st, proofs))
+
+    def verify():
+        ctypes.memmove(st, states, len(states))
+        be._check(lib.bpp_ipa_batch_verify(bt._h, None, None, None, P, proofs.raw, st, acc))
+
+    tp = timed(prove, REPS)
+    tv = timed(verify, REPS)
+    # stage timeline (device events) in a run of its own: the rounds alone, comparable with the `fixed` prover's stage
+    os.environ["BPP_ACP_TRACE"] = "1"
+    bt2 = Ipa.InnerProductBatch(be, pts, 0, n, 2 * n, n, count)
+    del os.environ["BPP_ACP_TRACE"]
+    bt2_h = bt2._h
+
+    def traced():
+        for _ in range(REPS + 1):
+            ctypes.memmove(st, states, len(states))
+            be._check(lib.bpp_ipa_batch_prove(bt2_h, None, None, None, ab, bb, st, proofs))
+            ctypes.memmove(st, states, len(states))
+            be._check(lib.bpp_ipa_batch_verify(bt2_h, None, None, None, P, proofs.raw, st, acc))
+    log = stderr_of(traced)
+    bt2.free()
+    stages = {}
+    for what in ("prove", "verify"):
+        lines = [ln for ln in log.splitlines() if ln.startswith(f"[ipa trace] {what}:")][1:]   # the first is the warm-up
+        for ln in lines:
+            for name, us in re.findall(r" ([^|:]+?) (\d+) us \|", ln):
+                stages.setdefault(f"{what}: {name}", []).append(float(us))
+    stage_ms = {k: float(np.median(v)) / 1e3 for k, v in stages.items()}
+    row = {"count": count, "n": n, "proof_bytes": bt.proof_len, "prove": tp, "verify": tv,
+           "all_accepted": acc.raw == b"\x01" * count, "stage_median_ms": stage_ms}
+    bt.free()
+    pts.free()
+    return row
+
+
+def fixed_rounds(be, count, npad, rs):
+    """median time of the `fixed` prover's "inner-product rounds" stage (BPP_ACP_TRACE=1) on count proofs of the
+    shuffle whose n pads to npad"""
+    G, W = bpperm_b200.acproof, bpperm_b200.weights
+    k = {128: 52, 8: 4, 8192: 4096}[npad]
+    n, Q, m, WL, WR, WO, WV, cv = W.shuffle_circuit(k)
+    ng = G.next_pow2(n)
+    pts = be.points_from_uniform(rs.randint(0, 256, size=(2 * ng + 2, 64), dtype=np.uint8).tobytes())
+    enc = be.compress_points(pts)
+    cir = G.Circuit(be, n, Q, m, WL, WR, WO, WV, cv)
+    gens = G.Generators(be, enc[:32], enc[32:64], [enc[64 + 32 * i: 96 + 32 * i] for i in range(ng)],
+                        [enc[64 + 32 * (ng + i): 96 + 32 * (ng + i)] for i in range(ng)])
+    sb = lambda vals: b"".join(int(x).to_bytes(32, "little") for x in vals)  # noqa: E731
+    v, a_L, a_R, a_O = W.shuffle_witness(k, rs.permutation(k), int.from_bytes(rs.bytes(31), "little"))
+    os.environ["BPP_ACP_TRACE"] = "1"
+    batch = G.Batch(be, cir, gens, count, "fixed", b"test")
+    del os.environ["BPP_ACP_TRACE"]
+    batch.upload_witness(sb(a_L) * count, sb(a_R) * count, sb(a_O) * count, scalars(rs, count * m).tobytes(),
+                         rs.randint(0, 256, size=(count, 32), dtype=np.uint8).tobytes())
+    batch.commit(sb(v) * count, want=False)
+    def run():
+        for _ in range(REPS + 1):
+            batch.prove()
+            be.synchronize()
+    log = stderr_of(run)
+    us = [float(x) for x in re.findall(r"inner-product rounds (\d+) us", log)][1:]   # the first prove is the warm-up
+    batch.free()
+    gens.free()
+    cir.free()
+    return {"cards": k, "padded_n": ng, "count": count, "rounds_median_ms": float(np.median(us)) / 1e3 if us else None,
+            "samples": len(us)}
+
+
+def main():
+    be = bpperm_b200.Backend(0)
+    rs = np.random.RandomState(2026)
+    res = {"card": card(), "reps": REPS, "rows": []}
+    for count, n in SHAPES:
+        row = ipa_shape(be, count, n, rs)
+        row["fixed_mode_rounds"] = fixed_rounds(be, count, n, rs)
+        fr = row["fixed_mode_rounds"]["rounds_median_ms"]
+        own = row["stage_median_ms"].get("prove: inner-product rounds")
+        row["rounds_over_fixed_rounds"] = own / fr if fr and own else None
+        print(json.dumps(row), flush=True)
+        res["rows"].append(row)
+    out = sys.argv[1] if len(sys.argv) > 1 else "ipa_bench.json"
+    os.makedirs(os.path.dirname(out) or ".", exist_ok=True)
+    json.dump(res, open(out, "w"), indent=1)
+
+
+if __name__ == "__main__":
+    main()
