@@ -130,6 +130,8 @@ static int grow(bpp_ctx *ctx, T **p, size_t *cap, size_t need_elems) {
 // defined in capi_core.cu
 int comm_all_gather(bpp_ctx *ctx, const void *d_send, void *d_recv, size_t bytes_per_rank, cudaStream_t stream);
 int msm_wait_pending(bpp_ctx *ctx, bool keep_latest = false);
+// groups: number of window groups, split evenly (0 = the library's partition for n, which minimises the latency of one
+// call; bpp_set_msm_groups / bpp_set_msm_partition override it)
 int msm_enqueue(bpp_ctx *ctx, const uint32_t *d_scalars, const bpp_points *pts, size_t off, size_t n, uint8_t *d_out,
-                int do_compress, bool join = true);
+                int do_compress, bool join = true, int groups = 0);
 

@@ -1221,7 +1221,12 @@ static int acp_verify_rlc(bpp_acp_batch *b, uint32_t per, int check_t, bool *dec
     view.niels = b->d_dyn;
     view.n = N;
     acp_mark(b, "rlc-scalars");
-    int rc = msm_enqueue(ctx, b->d_rlc_sc, &view, 0, N, b->d_rlc_out, 1, true);
+    // One window group: shaped for throughput, not for the latency of one call.  With several batches in flight the short
+    // dependent kernels of one batch hide behind the GPU-filling kernels of another, so what counts is the SM time the
+    // MSM takes: one sort, one accumulate grid without a partial wave per group, one merge + Horner chain.  Against the
+    // four groups pick_partition gives 4096 x 113 + 210 points: 612 K -> 695 K proofs/s in the 52-card step with six
+    // batches in flight, B200 at 1000 W (DESIGN.md section 3.2).
+    int rc = msm_enqueue(ctx, b->d_rlc_sc, &view, 0, N, b->d_rlc_out, 1, true, 1);
     view.niels = nullptr;
     if (rc) return rc;
     acp_mark(b, "rlc-msm");

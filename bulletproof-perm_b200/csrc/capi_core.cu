@@ -348,7 +348,7 @@ static int msm_pipeline_init(bpp_ctx *ctx) {
 // caller's stream).  Measured on B200 (tools/msm_groups.py, tools/msm_trace.py): the pipeline pays once the
 // accumulate of one group is long enough to hide the dependent tail (fix-up, node merges, Horner) of the previous
 // one; a small first group starts the accumulate early and a small last group leaves a short tail.
-static int pick_partition(const bpp_ctx *ctx, size_t n, int W, bool join, int part[BPP_MAX_GROUPS]) {
+static int pick_partition(const bpp_ctx *ctx, size_t n, int W, bool join, int groups, int part[BPP_MAX_GROUPS]) {
     if (ctx->n_forced_part && !ctx->profiling) {
         int sum = 0;
         for (int i = 0; i < ctx->n_forced_part; i++) sum += ctx->forced_part[i];
@@ -357,7 +357,7 @@ static int pick_partition(const bpp_ctx *ctx, size_t n, int W, bool join, int pa
             return ctx->n_forced_part;
         }
     }
-    if (!ctx->forced_groups && !ctx->profiling && W >= 8 &&
+    if (!ctx->forced_groups && !groups && !ctx->profiling && W >= 8 &&
         n >= (join ? BPP_PIPELINE_MIN_POINTS : BPP_PIPELINE_MIN_POINTS_SUBMIT)) {
         // measured best of the partitions tried at 2^18..2^22 points (profiles/r1_msm_partitions.md): an eighth of the
         // windows first and last, the rest in two halves (16 windows: 2, 6, 6, 2)
@@ -369,7 +369,7 @@ static int pick_partition(const bpp_ctx *ctx, size_t n, int W, bool join, int pa
         part[0] = edge; part[1] = (mid + 1) / 2; part[2] = mid / 2; part[3] = edge;
         return 4;
     }
-    int G = ctx->forced_groups ? ctx->forced_groups : 1;
+    int G = ctx->forced_groups ? ctx->forced_groups : (groups ? groups : 1);
     if (G > W) G = W;
     if (G > BPP_MAX_GROUPS) G = BPP_MAX_GROUPS;
     if (ctx->profiling || G < 1) G = 1;  // the per-phase events describe the in-order pipeline
@@ -407,7 +407,7 @@ static size_t msm_acc_pad_smem() {
 // valid after bpp_msm_wait, and up to two submitted MSMs are in flight (the tail of one beside the sort and
 // accumulate of the next).
 int msm_enqueue(bpp_ctx *ctx, const uint32_t *d_scalars, const bpp_points *pts, size_t off, size_t n, uint8_t *d_out,
-                int do_compress, bool join) {
+                int do_compress, bool join, int groups) {
     const int c = ctx->forced_c ? ctx->forced_c : pick_window(n);
     const int W = (256 + c - 1) / c;
     const uint32_t B = 1u << (c - 1);
@@ -435,7 +435,7 @@ int msm_enqueue(bpp_ctx *ctx, const uint32_t *d_scalars, const bpp_points *pts, 
     // window groups of the pipelined form (each at its own level at any moment) never share storage
     const size_t node_elems = (size_t)W * max_T_out * 32;
     int part[BPP_MAX_GROUPS];
-    const int G = pick_partition(ctx, n, W, join, part);
+    const int G = pick_partition(ctx, n, W, join, groups, part);
     int rc;
     if (G > 1 && (rc = msm_pipeline_init(ctx))) return rc;
     ctx->slot ^= 1;
