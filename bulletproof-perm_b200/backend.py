@@ -9,6 +9,7 @@ here in its canonical 32-byte encoding.
 """
 from __future__ import annotations
 
+import array
 import ctypes
 import weakref
 from typing import Iterable, Sequence, Union
@@ -223,6 +224,43 @@ class Backend:
         out = ctypes.create_string_buffer(32 * count)
         self._check(self._lib.bpp_msm_vartime_batch(self._ctx, bytes(scalars), count, points._h, off, n, out))
         return out.raw
+
+    # -- many independent MSMs over caller points (bpp_msm_multi*): MSM j takes the next sizes[j] terms ----------
+    @staticmethod
+    def _sizes(sizes):
+        sizes = [int(x) for x in sizes]
+        return (ctypes.c_uint32 * max(1, len(sizes)))(*sizes), len(sizes), sum(sizes)
+
+    def msm_multi(self, scalars: bytes, points_enc: bytes, sizes):
+        """`len(sizes)` MSMs over T x 32 scalars and T x 32 encodings -> (encodings, ok flags).  An undecodable point
+        fails only its own MSM (ok False, 32 zero bytes)."""
+        arr, count, T = self._sizes(sizes)
+        if len(scalars) != 32 * T or len(points_enc) != 32 * T:
+            raise ValueError("scalars and points: sum(sizes) x 32 bytes each")
+        out, ok = ctypes.create_string_buffer(32 * count), ctypes.create_string_buffer(count)
+        self._check(self._lib.bpp_msm_multi(self._ctx, count, arr, bytes(scalars), bytes(points_enc), out, ok))
+        return [out.raw[32 * j:32 * j + 32] for j in range(count)], [b != 0 for b in ok.raw]
+
+    def msm_multi_indexed(self, scalars: bytes, points: Points, index, sizes):
+        """`len(sizes)` MSMs with P_t = points[index[t]] -> list of encodings."""
+        arr, count, T = self._sizes(sizes)
+        raw = index.tobytes() if hasattr(index, "tobytes") else array.array("I", index).tobytes()   # uint32 each
+        if len(scalars) != 32 * T or len(raw) != 4 * T:
+            raise ValueError("scalars: sum(sizes) x 32 bytes, index: sum(sizes) uint32 entries")
+        ix = (ctypes.c_uint32 * max(1, T)).from_buffer_copy(raw or bytes(4))
+        out = ctypes.create_string_buffer(32 * count)
+        self._check(self._lib.bpp_msm_multi_indexed(self._ctx, count, arr, bytes(scalars), points._h, ix, out))
+        return [out.raw[32 * j:32 * j + 32] for j in range(count)]
+
+    def msm_multi_dev(self, sizes, d_scalars: int, d_points_enc: int, d_out32: int, d_ok: int):
+        arr, count, _ = self._sizes(sizes)
+        self._check(self._lib.bpp_msm_multi_dev(self._ctx, count, arr, ctypes.c_void_p(d_scalars), ctypes.c_void_p(d_points_enc),
+                                                ctypes.c_void_p(d_out32), ctypes.c_void_p(d_ok)))
+
+    def msm_multi_indexed_dev(self, sizes, d_scalars: int, points: Points, d_index: int, d_out32: int):
+        arr, count, _ = self._sizes(sizes)
+        self._check(self._lib.bpp_msm_multi_indexed_dev(self._ctx, count, arr, ctypes.c_void_p(d_scalars), points._h,
+                                                        ctypes.c_void_p(d_index), ctypes.c_void_p(d_out32)))
 
     # device-pointer forms (pointers are ints, e.g. torch.Tensor.data_ptr())
     def msm_dev(self, d_scalars: int, points: Points, off: int, n: int, d_out: int):

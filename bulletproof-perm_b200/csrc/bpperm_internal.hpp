@@ -66,6 +66,8 @@ struct bpp_ctx {
     uint8_t *h_pinned = nullptr; size_t cap_pinned = 0;         // pinned staging for host scalars
     uint8_t *d_vec = nullptr; size_t cap_vec = 0;               // arena of the scalar-vector operators
     uint8_t *d_small = nullptr; size_t cap_small = 0;           // arena of bpp_msm_vartime_batch
+    uint8_t *d_multi = nullptr; size_t cap_multi = 0;           // arena of bpp_msm_multi*
+    std::vector<uint8_t> mm_host;                               // host plan of the last bpp_msm_multi* call
     // pipelined MSM: window groups on side streams (msm_pipeline_init)
     bool pipe_ready = false;
     int forced_groups = 0;

@@ -55,7 +55,7 @@ extern "C" void bpp_free(bpp_ctx *ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
     cudaDeviceSynchronize();
-    void *ptrs[] = {ctx->d_scalars, ctx->d_out, ctx->d_stage, ctx->d_flag, ctx->d_vec, ctx->d_small};
+    void *ptrs[] = {ctx->d_scalars, ctx->d_out, ctx->d_stage, ctx->d_flag, ctx->d_vec, ctx->d_small, ctx->d_multi};
     for (void *p : ptrs)
         if (p) cudaFree(p);
     for (auto &sc : ctx->scr) {

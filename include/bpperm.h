@@ -201,6 +201,30 @@ int bpp_msm_vartime_batch(bpp_ctx *ctx, const uint8_t *scalars, size_t count, bp
 int bpp_msm_vartime_batch_dev(bpp_ctx *ctx, const void *d_scalars, size_t count, bpp_points *points, size_t off, size_t n,
                               void *d_out32);
 
+/* ---- batched MSMs over caller points: many independent vartime_multiscalar_mul calls in one call ----------
+ * MSM j has sizes[j] terms; the terms of all MSMs are stored one after another.  With T = sum sizes and
+ * start_j = sum_{i<j} sizes[i], MSM j = sum_{t = start_j}^{start_j + sizes[j] - 1} s_t * P_t.  sizes is host memory (the
+ * launch plan is made from it).  out32[j] is the canonical encoding of MSM j; sizes[j] == 0 gives the identity (32 zero
+ * bytes).  Scalars are 32-byte little-endian with bit 255 clear; non-canonical scalars below 2^255 are accepted, as dalek
+ * accepts them.  A few launches per call whatever count is, all on the context's stream; results depend on the inputs
+ * only (not on the batch's composition or order).
+ * Errors, host forms, before any device work: NULL pointers or count == 0, or T >= 2^31: BPP_ERR_INVALID_ARG; an
+ * index[t] >= bpp_points_len(points): BPP_ERR_LENGTH_MISMATCH; a scalar with bit 255 set: BPP_ERR_SCALAR_RANGE.  The _dev
+ * forms check what the host sees (NULL pointers, count, T); device data cannot make them fault: bit 255 of a scalar is read
+ * as zero and an index outside the set is clamped into it (the -DBPP_DEBUG_BOUNDS build asserts instead). */
+/* points as 32-byte RFC 9496 encodings (T x 32).  An undecodable encoding fails only its own MSM:
+ * ok[j] = 0 and out32[j] = 32 zero bytes (dalek: optional_multiscalar_mul -> None); ok[j] = 1 otherwise. */
+int bpp_msm_multi(bpp_ctx *ctx, size_t count, const uint32_t *sizes, const uint8_t *scalars /* T x 32 */,
+                  const uint8_t *points_enc /* T x 32 */, uint8_t *out32 /* count x 32 */, uint8_t *ok /* count */);
+/* points from a resident set: P_t = points[index[t]]; no decoding. */
+int bpp_msm_multi_indexed(bpp_ctx *ctx, size_t count, const uint32_t *sizes, const uint8_t *scalars,
+                          const bpp_points *points, const uint32_t *index /* T */, uint8_t *out32);
+/* _dev: scalars, encodings / index, out32, ok are device pointers; stream-ordered on the context's stream, no synchronisation */
+int bpp_msm_multi_dev(bpp_ctx *ctx, size_t count, const uint32_t *sizes, const void *d_scalars,
+                      const void *d_points_enc, void *d_out32, void *d_ok);
+int bpp_msm_multi_indexed_dev(bpp_ctx *ctx, size_t count, const uint32_t *sizes, const void *d_scalars,
+                              const bpp_points *points, const void *d_index, void *d_out32);
+
 /* ---- the arithmetic-circuit (shuffle) proof, batched ------------------------------------------------
  * Replaces the group/scalar arithmetic of ACProof::ArithmeticCircuitProof (circuit_lib.rs:133-585) for
  * `count` independent proofs that share one circuit and one generator set, driven in the reference's

@@ -42,6 +42,26 @@ impl VartimeMultiscalarMul for GpuRistretto {
         CompressedRistretto(out).decompress()
     }
 }
+impl GpuRistretto {
+    /// Many independent `optional_multiscalar_mul` calls in one `bpp_msm_multi`: call k is (scalars, points), the
+    /// results come back in call order.  A call whose points do not all decode gives `None`, as a single call does;
+    /// the other calls are unaffected.
+    pub fn optional_multiscalar_mul_many(calls: &[(Vec<Scalar>, Vec<CompressedRistretto>)]) -> Vec<Option<RistrettoPoint>> {
+        if calls.is_empty() { return Vec::new(); }
+        let sizes: Vec<u32> = calls.iter().map(|(s, p)| { assert_eq!(s.len(), p.len()); s.len() as u32 }).collect();
+        let s: Vec<u8> = calls.iter().flat_map(|(s, _)| s.iter().flat_map(|x| x.to_bytes().to_vec())).collect();
+        let enc: Vec<u8> = calls.iter().flat_map(|(_, p)| p.iter().flat_map(|q| q.to_bytes().to_vec())).collect();
+        let mut out = vec![0u8; 32 * calls.len()];
+        let mut ok = vec![0u8; calls.len()];
+        let rc = with_ctx(|c| unsafe {
+            sys::bpp_msm_multi(c, calls.len(), sizes.as_ptr(), s.as_ptr(), enc.as_ptr(), out.as_mut_ptr(), ok.as_mut_ptr())
+        });
+        assert_eq!(rc, 0);
+        out.chunks_exact(32).zip(ok.iter())
+            .map(|(o, &k)| if k == 1 { CompressedRistretto(<[u8; 32]>::try_from(o).unwrap()).decompress() } else { None })
+            .collect()
+    }
+}
 
 /// The reference's 15 call sites always multiply sub-ranges of the same generators (g, h, G_vec, H_vec: lib.rs:164-180).
 /// Upload them once, attach the window table once; every later MSM is table look-ups + mixed adds, and
@@ -73,6 +93,18 @@ impl GeneratorSet {
         assert_eq!(scalars.len(), count * n);
         let mut out = vec![0u8; 32 * count];
         let rc = with_ctx(|c| unsafe { sys::bpp_msm_vartime_batch(c, bytes_of(scalars).as_ptr(), count, self.pts, off, n, out.as_mut_ptr()) });
+        assert_eq!(rc, 0);
+        out.chunks_exact(32).map(|c| CompressedRistretto(<[u8; 32]>::try_from(c).unwrap())).collect()
+    }
+    /// Independent MSMs over points of this set chosen per term: MSM j = sum scalars[t] * points[index[t]] over its
+    /// sizes[j] terms (terms of all MSMs one after another).  No table: any mix of sub-ranges and sizes, one call.
+    pub fn msm_many_indexed(&self, sizes: &[u32], scalars: &[Scalar], index: &[u32]) -> Vec<CompressedRistretto> {
+        let total: usize = sizes.iter().map(|&n| n as usize).sum();
+        assert!(scalars.len() == total && index.len() == total && !sizes.is_empty());
+        let mut out = vec![0u8; 32 * sizes.len()];
+        let rc = with_ctx(|c| unsafe {
+            sys::bpp_msm_multi_indexed(c, sizes.len(), sizes.as_ptr(), bytes_of(scalars).as_ptr(), self.pts, index.as_ptr(), out.as_mut_ptr())
+        });
         assert_eq!(rc, 0);
         out.chunks_exact(32).map(|c| CompressedRistretto(<[u8; 32]>::try_from(c).unwrap())).collect()
     }

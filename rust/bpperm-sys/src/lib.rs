@@ -55,6 +55,17 @@ extern "C" {
                                  out32: *mut u8) -> c_int;
     pub fn bpp_msm_vartime_batch_dev(ctx: *mut bpp_ctx, d_scalars: *const core::ffi::c_void, count: usize, points: *mut bpp_points,
                                      off: usize, n: usize, d_out32: *mut core::ffi::c_void) -> c_int;
+    // many independent MSMs over caller points: MSM j takes the next sizes[j] terms (sizes: host memory)
+    pub fn bpp_msm_multi(ctx: *mut bpp_ctx, count: usize, sizes: *const u32, scalars: *const u8, points_enc: *const u8,
+                         out32: *mut u8, ok: *mut u8) -> c_int;
+    pub fn bpp_msm_multi_indexed(ctx: *mut bpp_ctx, count: usize, sizes: *const u32, scalars: *const u8,
+                                 points: *const bpp_points, index: *const u32, out32: *mut u8) -> c_int;
+    pub fn bpp_msm_multi_dev(ctx: *mut bpp_ctx, count: usize, sizes: *const u32, d_scalars: *const core::ffi::c_void,
+                             d_points_enc: *const core::ffi::c_void, d_out32: *mut core::ffi::c_void,
+                             d_ok: *mut core::ffi::c_void) -> c_int;
+    pub fn bpp_msm_multi_indexed_dev(ctx: *mut bpp_ctx, count: usize, sizes: *const u32, d_scalars: *const core::ffi::c_void,
+                                     points: *const bpp_points, d_index: *const core::ffi::c_void,
+                                     d_out32: *mut core::ffi::c_void) -> c_int;
     // multi-GPU: one process per GPU, NCCL inside the library
     pub fn bpp_comm_unique_id(id: *mut u8) -> c_int;                      // 128 bytes, made on rank 0
     pub fn bpp_comm_init(ctx: *mut bpp_ctx, nranks: c_int, rank: c_int, id: *const u8) -> c_int;
