@@ -32,6 +32,8 @@ struct acp_layout {
     uint32_t wq, u, uinv, cl, pa, pb, ptab;        // `fixed` mode: challenge w, u_j / u_j^-1 (lg each), w*c_L, w*c_R,
                                                    // the proof's a and b, 3 x IPA_MAX_LG squarings for the power tables
     uint32_t stab;                                 // `fixed` mode: 2 x n' table of the s_t (ipa_kernels.cuh)
+    uint32_t vr, nx;                               // shuffle-shaped circuits: a_R = v' - x as written by the witness
+                                                   // kernels, v' (n - 2) and -x (1); none otherwise
 };
 
 #define ACP_PTR(base, lay, p, off) ((base) + 8 * ((size_t)(p) * (lay).stride + (off)))
@@ -91,7 +93,15 @@ __global__ void __launch_bounds__(128) k_acp_place_witness(const uint32_t *__res
 // padding multipliers 2k - 2, 2k - 1 are zero.  Block per (chain, proof): each thread multiplies up a run of consecutive
 // factors, the run totals are scanned through shared memory (Hillis-Steele), so a 4096-card chain is 8 + 9 + 8
 // dependent multiplications deep instead of 4095.  Products in Montgomery form until the final store.
+// Both forms also write a_R in its structured form: v'[gb + i] = v[vb + i + 1] and -x (sc_sub(0, x)), so that the prover
+// can commit <a_R, H> as <v', H> + (-x) H_sum (bpp_acp_batch_prove).
 #define WIT_THREADS 256
+SC_INLINE void acp_store_neg_x(uint32_t *blk, const acp_layout &lay, uint32_t p, const sc &x) {
+    sc z, nx;
+    sc_set0(z);
+    sc_sub(nx, z, x);
+    sc_store(ACP_PTR(blk, lay, p, lay.nx), nx);
+}
 __global__ void __launch_bounds__(WIT_THREADS) k_shuffle_witness(const uint32_t *__restrict__ deck /* k x 8 */,
                                                                  const uint32_t *__restrict__ perm /* B x k */,
                                                                  const uint32_t *__restrict__ xs /* B x 8 */, uint32_t k,
@@ -119,6 +129,7 @@ __global__ void __launch_bounds__(WIT_THREADS) k_shuffle_witness(const uint32_t 
     sc acc = one, f, t;
     for (uint32_t i = i0; i < i1; i++) {
         f = value(i + 1);
+        sc_store(ACP_PTR(blk, lay, p, lay.vr + gb + i), f);
         sc_sub(f, f, x);
         sc_store(ACP_PTR(blk, lay, p, lay.aR + gb + i), f);
         sc_mont(t, f, r2);
@@ -132,6 +143,7 @@ __global__ void __launch_bounds__(WIT_THREADS) k_shuffle_witness(const uint32_t 
         sc_mont(acc, acc, t);
         if (c == 0) {
             sc_store(vp + 8 * (size_t)(2 * k), x);
+            acp_store_neg_x(blk, lay, p, x);
             sc z;
             sc_set0(z);
             for (uint32_t q = 2 * k - 2; q < 2 * k; q++) {
@@ -201,6 +213,7 @@ __global__ void __launch_bounds__(64) k_shuffle_witness_serial(const uint32_t *_
         BPP_ASSERT(!c || pp[i + 1] < k);
         sc_load(v, deck + 8 * (size_t)(c ? pp[i + 1] : i + 1));
         sc_store(vp + 8 * (size_t)(vb + i + 1), v);
+        sc_store(ACP_PTR(blk, lay, p, lay.vr + gb + i), v);
         sc_sub(f, v, x);
         sc_store(ACP_PTR(blk, lay, p, lay.aR + gb + i), f);
         if (i) sc_store(ACP_PTR(blk, lay, p, lay.aL + gb + i), P);   // a_L[gb + i] = a_O[gb + i - 1]
@@ -210,6 +223,7 @@ __global__ void __launch_bounds__(64) k_shuffle_witness_serial(const uint32_t *_
     }
     if (c == 0) {
         sc_store(vp + 8 * (size_t)(2 * k), x);
+        acp_store_neg_x(blk, lay, p, x);
         sc z;
         sc_set0(z);
         for (uint32_t q = 2 * k - 2; q < 2 * k; q++) {
@@ -294,6 +308,13 @@ struct fb_shape {
     uint32_t outs;           // outputs per proof (gridDim.y)
     uint32_t sel_period;     // 0 = off.  IPA rounds (ipa_kernels.cuh): term k of a segment belongs to output 0 (L) or
     uint32_t sel[4];         // 1 (R) by the half of its period it lies in: sel 1 = upper half -> L, 2 = lower half -> L
+};
+// k_fb_msm_warp_d<C, true> only (fb_warp_d_fits), kept out of fb_shape so that the other table kernels' parameters stay
+// as they were measured: segments of mask `alt` index alt_table (a table of the same width) instead of the launch's
+// table, and terms with at most FB_SPARSE_MAX non-zero digits are spread over all lanes
+struct fb_sparse {
+    uint32_t on, alt;
+    const uint32_t *alt_table;
 };
 struct fb_consts {
     uint32_t K[8];  // sum_{w < Wn-1} half * 2^(c w)
@@ -517,12 +538,32 @@ __global__ void __launch_bounds__(FB_THREADS, FB_WARP_MINBLOCKS) k_fb_msm_warp(c
 // table entry - and, since the lane stride 32 is a multiple of the window count, a lane keeps the same window for its
 // whole life (ww = lane mod Wn): items are single (term, window) pairs, so lanes differ by at most one mixed add
 // (the 4-window items above: by four).  Dynamic shared memory: (FB_THREADS / 32) x total_terms x 36 B.
+//
+// SPARSE (launches with sp.on set): a term with at most FB_SPARSE_MAX non-zero digits - a small scalar, such as a
+// card value of the shuffle witness, has one - would put all its work on the lanes of those windows (lanes 0 and 16 for
+// a value below 2^15) while the other 30 lanes idle.  Such terms are not staged as digits: while staging, each of
+// their non-zero digits becomes one word (entry << 1 | sign) of a per-warp list, compacted with ballot + popc, and the
+// lanes take that list round-robin after their dense items, continuing the lane order where the dense items stop, so the
+// mixed adds per lane differ by at most one (skipped zero digits aside).  Terms of an `alt` segment (their generator
+// index carries FB_ALT) read sp.alt_table and always stay dense.  The list is sized for the worst case: 2 words per
+// term, (FB_THREADS / 32) x total_terms x 8 B more dynamic shared memory.
 #ifndef FB_STAGE_MAX_BYTES
 #define FB_STAGE_MAX_BYTES (48u * 1024u)   // dynamic shared memory without an opt-in attribute
 #endif
+#define FB_SPARSE_MAX 2
+#define FB_ALT 0x80000000u
+// 32-bit words per warp of the digit-staged form's stage: s' (8 per term) and the generator index, rounded up to 16
+// bytes; with SPARSE the list after them
+static __host__ __device__ __forceinline__ uint32_t fb_stage_d_words(uint32_t terms, bool sparse) {
+    return ((9 * terms + 3) & ~3u) + (sparse ? FB_SPARSE_MAX * terms : 0);
+}
 template <int C>
+__device__ __forceinline__ uint32_t fb_field(const uint32_t (&s)[8], uint32_t w) {   // w: a compile-time constant after unrolling
+    return C == 16 ? (s[w >> 1] >> (16 * (w & 1))) & 0xffffu : (s[w >> 2] >> (8 * (w & 3))) & 0xffu;
+}
+template <int C, bool SPARSE>
 __global__ void __launch_bounds__(FB_THREADS, FB_WARP_MINBLOCKS) k_fb_msm_warp_d(const uint32_t *__restrict__ blk, acp_layout lay, fb_shape sh,
-                                                              const uint32_t *__restrict__ table, fb_consts kc,
+                                                              const uint32_t *__restrict__ table, fb_consts kc, fb_sparse sp,
                                                               uint32_t B, uint32_t outs /* per proof; sh.outs = pitch */,
                                                               uint32_t *__restrict__ out_ext /* [p][pitch] x 32 */) {
     constexpr uint32_t WN = (256 + C - 1) / C, LOG_WN = WN == 32 ? 5 : 4, HALF = 1u << (C - 1);
@@ -532,28 +573,60 @@ __global__ void __launch_bounds__(FB_THREADS, FB_WARP_MINBLOCKS) k_fb_msm_warp_d
     if (wid >= B * outs) return;   // whole warps leave together
     const uint32_t p = wid / outs, o = wid - p * outs;
     const uint32_t total_terms = fb_terms(sh);
-    // per warp: total_terms x 8 words of s', then the generator indices (region rounded up to 16 bytes)
-    uint32_t *stage = fb_stage + (size_t)(threadIdx.x >> 5) * ((9 * total_terms + 3) & ~3u);
+    const uint32_t lt = (1u << lane) - 1u;
+    // per warp: total_terms x 8 words of s', then the generator indices (region rounded up to 16 bytes), then the list
+    uint32_t *stage = fb_stage + (size_t)(threadIdx.x >> 5) * fb_stage_d_words(total_terms, SPARSE);
     uint32_t *sgen = stage + 8 * (size_t)total_terms;
-    uint32_t n_act = 0;
+    uint32_t *slist = stage + fb_stage_d_words(total_terms, false);
+    uint32_t n_act = 0, n_sp = 0;
     for (uint32_t t0 = 0; t0 < total_terms; t0 += 32) {
         const uint32_t t = t0 + lane;
         bool act = t < total_terms;
-        uint32_t seg = 0, k = t;
+        uint32_t seg = 0, k = t, gen = 0;
+        uint32_t s[8];
         if (act) {
             fb_locate_term(sh, t, seg, k);
             act = fb_term_selected(sh, seg, k, o);
         }
+        if (act) {
+            const uint32_t carry = fb_recode(fb_scalar(blk, lay, sh, p, o, seg, k), kc.K, s);
+            BPP_ASSERT(carry == 0);   // s' < 2^256 (s < 2^255, K < 2^(C (WN - 1)))
+            (void)carry;
+            gen = sh.gen[seg] + k;
+            if (SPARSE && ((sp.alt >> seg) & 1u)) gen |= FB_ALT;
+        }
+        if (SPARSE) {
+            uint32_t nz = 0;
+            if (act && !(gen & FB_ALT)) {
+#pragma unroll
+                for (uint32_t w = 0; w < WN; w++) nz += fb_field<C>(s, w) != (w == WN - 1 ? 0u : HALF);
+            }
+            const bool sp = act && !(gen & FB_ALT) && nz <= FB_SPARSE_MAX;
+            static_assert(FB_SPARSE_MAX == 2, "the list positions below count terms of one and of two digits");
+            const uint32_t b1 = __ballot_sync(0xffffffffu, sp && nz == 1), b2 = __ballot_sync(0xffffffffu, sp && nz == 2);
+            if (sp) {
+                uint32_t pos = n_sp + __popc(b1 & lt) + 2 * __popc(b2 & lt);
+#pragma unroll
+                for (uint32_t w = 0; w < WN; w++) {
+                    const uint32_t u = fb_field<C>(s, w);
+                    const int d = w == WN - 1 ? (int)u : (int)u - (int)HALF;
+                    if (d != 0) {
+                        const uint32_t mag = d < 0 ? (uint32_t)(-d) : (uint32_t)d;
+                        BPP_ASSERT(pos < FB_SPARSE_MAX * total_terms);
+                        slist[pos++] = ((((gen << LOG_WN) + w) << (C - 1)) + (mag - 1)) << 1 | (d < 0 ? 1u : 0u);
+                    }
+                }
+            }
+            n_sp += __popc(b1) + 2 * __popc(b2);
+            act = act && !sp;
+        }
         const uint32_t bal = __ballot_sync(0xffffffffu, act);
         if (act) {
-            const uint32_t idx = n_act + __popc(bal & ((1u << lane) - 1u));
-            uint32_t s[8];
-            const uint32_t carry = fb_recode(fb_scalar(blk, lay, sh, p, o, seg, k), kc.K, s);
-            BPP_ASSERT(carry == 0 && idx < total_terms);   // s' < 2^256 (s < 2^255, K < 2^(C (WN - 1)))
-            (void)carry;
+            const uint32_t idx = n_act + __popc(bal & lt);
+            BPP_ASSERT(idx < total_terms);
             *reinterpret_cast<uint4 *>(stage + 8 * (size_t)idx) = make_uint4(s[0], s[1], s[2], s[3]);
             *reinterpret_cast<uint4 *>(stage + 8 * (size_t)idx + 4) = make_uint4(s[4], s[5], s[6], s[7]);
-            sgen[idx] = sh.gen[seg] + k;
+            sgen[idx] = gen;
         }
         n_act += __popc(bal);
     }
@@ -563,9 +636,17 @@ __global__ void __launch_bounds__(FB_THREADS, FB_WARP_MINBLOCKS) k_fb_msm_warp_d
     const bool top = ww == WN - 1;                      // the top window's digit is unsigned
     const uint32_t lane_entry = ww << (C - 1);          // entry = (gen * WN + ww) * HALF + mag - 1
     uint32_t it = lane;
+    uint32_t js = (lane - items) & 31u;                 // list word js goes to lane (items + js) mod 32
     auto advance = [&](const uint32_t *&ptr, bool &neg) -> bool {
         for (;;) {
-            if (it >= items) return false;
+            if (it >= items) {
+                if (!SPARSE || js >= n_sp) return false;
+                const uint32_t wd = slist[js];
+                js += 32;
+                ptr = table + (size_t)(wd >> 1) * FB_ENTRY_U32;
+                neg = wd & 1u;
+                return true;
+            }
             const uint32_t term = it >> LOG_WN;
             it += 32;
             uint32_t u;
@@ -574,9 +655,10 @@ __global__ void __launch_bounds__(FB_THREADS, FB_WARP_MINBLOCKS) k_fb_msm_warp_d
             const int d = top ? (int)u : (int)u - (int)HALF;
             if (d == 0) continue;
             const uint32_t mag = d < 0 ? (uint32_t)(-d) : (uint32_t)d;
-            const uint32_t entry = ((sgen[term] << LOG_WN) << (C - 1)) + lane_entry + (mag - 1);
+            const uint32_t g = sgen[term];
+            const uint32_t entry = ((g << LOG_WN) << (C - 1)) + lane_entry + (mag - 1);   // the shift drops FB_ALT
             BPP_ASSERT(mag >= 1 && mag <= HALF && term < n_act);
-            ptr = table + (size_t)entry * FB_ENTRY_U32;
+            ptr = (SPARSE && (g & FB_ALT) ? sp.alt_table : table) + (size_t)entry * FB_ENTRY_U32;
             neg = d < 0;
             return true;
         }
@@ -586,19 +668,33 @@ __global__ void __launch_bounds__(FB_THREADS, FB_WARP_MINBLOCKS) k_fb_msm_warp_d
     ge_warp_sum<false>(acc);
     if (lane == 0) ge_store(out_ext + 32 * ((size_t)p * sh.outs + o), acc);
 }
-// host side: the warp-per-output launch.  The digit-staged form where the window width has one, its stage fits and the
-// entry indices fit 32 bits; else the scalar-staged form where its stage fits; else the unstaged form.
+// whether fb_warp_launch runs shape sh in the digit-staged form: the window width has one, its stage fits and the entry
+// indices fit 32 bits (31 with SPARSE: the list words carry the sign beside them; the alt table has generator 0 only)
+static inline bool fb_warp_d_fits(const fb_shape &sh, const fb_sparse &sp, int c, int Wn) {
+    uint64_t gen_end = 0;
+    for (uint32_t k = 0; k < sh.nseg; k++) {
+        const uint64_t e = ((sp.alt >> k) & 1u) ? 1 : (uint64_t)sh.gen[k] + sh.cnt[k];
+        gen_end = gen_end > e ? gen_end : e;
+    }
+    const bool fits = ((gen_end * Wn) << (c - 1)) < (sp.on ? 1ull << 31 : 1ull << 32);
+    const size_t stage_d = (size_t)(FB_THREADS / 32) * fb_stage_d_words(fb_terms(sh), sp.on != 0) * 4;
+    return fits && stage_d <= FB_STAGE_MAX_BYTES && (c == 16 || c == 8);
+}
+// host side: the warp-per-output launch.  The digit-staged form where fb_warp_d_fits; else the scalar-staged form where
+// its stage fits; else the unstaged form.  A launch with sp.on or sp.alt set only runs in the digit-staged form (the
+// caller checks fb_warp_d_fits).
 static inline void fb_warp_launch(const uint32_t *d_sc, const acp_layout &lay, const fb_shape &sh, const uint32_t *table, int c, int Wn,
-                                  const fb_consts &kc, uint32_t B, uint32_t outs, uint32_t *d_ext, cudaStream_t st) {
+                                  const fb_consts &kc, uint32_t B, uint32_t outs, uint32_t *d_ext, cudaStream_t st,
+                                  const fb_sparse &sp = fb_sparse{}) {
     const uint32_t n_out = B * outs, terms = fb_terms(sh);
     const unsigned grid = (n_out + FB_THREADS / 32 - 1) / (FB_THREADS / 32);
-    const size_t stage_d = (size_t)(FB_THREADS / 32) * ((9 * terms + 3) & ~3u) * 4, stage_b = (size_t)(FB_THREADS / 32) * terms * 32;
-    uint64_t gen_end = 0;
-    for (uint32_t k = 0; k < sh.nseg; k++) gen_end = gen_end > (uint64_t)sh.gen[k] + sh.cnt[k] ? gen_end : (uint64_t)sh.gen[k] + sh.cnt[k];
-    const bool fits32 = ((gen_end * Wn) << (c - 1)) < (1ull << 32);
-    if (fits32 && stage_d <= FB_STAGE_MAX_BYTES && (c == 16 || c == 8)) {
-        if (c == 16) k_fb_msm_warp_d<16><<<grid, FB_THREADS, stage_d, st>>>(d_sc, lay, sh, table, kc, B, outs, d_ext);
-        else k_fb_msm_warp_d<8><<<grid, FB_THREADS, stage_d, st>>>(d_sc, lay, sh, table, kc, B, outs, d_ext);
+    const size_t stage_d = (size_t)(FB_THREADS / 32) * fb_stage_d_words(terms, sp.on != 0) * 4,
+                 stage_b = (size_t)(FB_THREADS / 32) * terms * 32;
+    if (fb_warp_d_fits(sh, sp, c, Wn)) {
+        if (sp.on && c == 16) k_fb_msm_warp_d<16, true><<<grid, FB_THREADS, stage_d, st>>>(d_sc, lay, sh, table, kc, sp, B, outs, d_ext);
+        else if (sp.on) k_fb_msm_warp_d<8, true><<<grid, FB_THREADS, stage_d, st>>>(d_sc, lay, sh, table, kc, sp, B, outs, d_ext);
+        else if (c == 16) k_fb_msm_warp_d<16, false><<<grid, FB_THREADS, stage_d, st>>>(d_sc, lay, sh, table, kc, sp, B, outs, d_ext);
+        else k_fb_msm_warp_d<8, false><<<grid, FB_THREADS, stage_d, st>>>(d_sc, lay, sh, table, kc, sp, B, outs, d_ext);
     } else if (stage_b <= FB_STAGE_MAX_BYTES) {
         k_fb_msm_warp<true><<<grid, FB_THREADS, stage_b, st>>>(d_sc, lay, sh, table, c, Wn, kc, B, outs, d_ext);
     } else {
@@ -652,6 +748,21 @@ __global__ void __launch_bounds__(32) k_fb_sum_splits(const uint32_t *__restrict
     }
     ge_warp_sum<true>(acc);
     if (lane == 0) ge_store(dst + 32 * ((size_t)p * pitch + o), acc);
+}
+
+// one warp: out = the sum of the points niels[first .. first + cnt) (one-time: H_sum of bpp_acp_batch_create)
+__global__ void __launch_bounds__(32) k_point_sum(const uint32_t *__restrict__ niels, uint32_t first, uint32_t cnt,
+                                                  uint32_t *__restrict__ out_ext) {
+    ge_ext acc;
+    ge_identity(acc);
+#pragma unroll 1
+    for (uint32_t i = threadIdx.x; i < cnt; i += 32) {
+        ge_niels q;
+        ge_niels_load(q, niels + 24 * (size_t)(first + i));
+        ge_madd(acc, acc, q, false);
+    }
+    ge_warp_sum<true>(acc);
+    if (threadIdx.x == 0) ge_store(out_ext, acc);
 }
 
 // thread per point: ext (raw limbs) -> 32-byte encoding

@@ -23,6 +23,11 @@ struct bpp_circuit {
 struct bpp_gens {
     uint32_t n = 0, n_gens = 0;  // gens order: g, h, G[0..n), H[0..n)
     bpp_points *pts = nullptr;   // the n_gens points and their window table (bpp_points_precompute)
+    // sums of generator ranges with their own window table (acp_gens_sum: H_sum of the shuffle prover's A_I), built once
+    // per (range, window width) for all batches over these generators and freed with them
+    struct range_sum { uint32_t first, cnt; bpp_points *pts; };
+    std::vector<range_sum> sums;
+    std::mutex mu;
 };
 
 struct bpp_acp_batch {
@@ -60,6 +65,10 @@ struct bpp_acp_batch {
     cudaEvent_t ev_join3 = nullptr;
     uint32_t *d_vwit = nullptr, *d_wgen = nullptr;   // bpp_acp_batch_gen_shuffle_witness: v (B x m), staging of its inputs
     bool have_vwit = false;
+    // the resident witness came from bpp_acp_batch_gen_shuffle_witness (v', -x are in the block): A_I may take the
+    // structured shape (acp_ai_shape) over H_sum = H_0 + .. + H_{n-3}, whose table hsum is (owned by the generators)
+    bool shuffle_wit = false;
+    const bpp_points *hsum = nullptr;
     bool have_V = false;            // commitments resident (bpp_acp_batch_commit / _upload_commitments / _upload_proofs)
     uint8_t *h_V = nullptr;         // host transcripts only: pinned copy of the commitments
     // priority split (bpp_acp_batch_set_priority_split): the table-gather MSMs (k_fb_msm) run on `bulk`, a stream of
@@ -106,6 +115,8 @@ static void acp_marks_dump(bpp_acp_batch *b, const char *what) {
     for (auto &m : b->marks) cudaEventDestroy(m.second);
     b->marks.clear();
 }
+// the shape of bpp_circuit_create_shuffle's circuit, which bpp_acp_batch_gen_shuffle_witness needs: n = 2k, m = 2k + 1, k >= 2
+static bool acp_shuffle_shaped(uint32_t n, uint32_t m) { return n >= 4 && !(n & 1u) && m == n + 1; }
 static acp_layout acp_make_layout(uint32_t n_, uint32_t Q, uint32_t m, int mode) {
     acp_layout L;
     uint32_t o = 0;
@@ -128,6 +139,8 @@ static acp_layout acp_make_layout(uint32_t n_, uint32_t Q, uint32_t m, int mode)
     L.ptab = take(mode == 2 ? 3 * IPA_MAX_LG : 0);
     L.stab = take(mode == 2 ? 2 * np : 0);
     L.rho = take(1);
+    const bool shuffle = acp_shuffle_shaped(n, m);
+    L.vr = take(shuffle ? n - 2 : 0); L.nx = take(shuffle ? 1 : 0);
     L.stride = (o + 3) & ~3u;
     return L;
 }
@@ -283,6 +296,7 @@ extern "C" int bpp_gens_create(bpp_ctx *ctx, const uint8_t g[32], const uint8_t 
 }
 extern "C" void bpp_gens_free(bpp_ctx *ctx, bpp_gens *g) {
     if (!g) return;
+    for (auto &e : g->sums) bpp_points_free(ctx, e.pts);
     bpp_points_free(ctx, g->pts);
     delete g;
 }
@@ -510,6 +524,8 @@ extern "C" void bpp_acp_batch_free(bpp_acp_batch *b) {
     delete b;
 }
 
+static int acp_prepare_hsum(bpp_acp_batch *b);
+
 // mode 0 = "reference" (bit-for-bit what circuit_lib.rs does, defects included; verification never
 // accepts), mode 1 = "reference-fixed" (SURVEY A.3), mode 2 = "fixed" (standard powers + inner-product argument,
 // ipa_kernels.cuh; needs next_pow2(n) generators).  label = the Transcript::new label (lib.rs:172: b"test").
@@ -591,6 +607,10 @@ extern "C" int bpp_acp_batch_create(bpp_ctx *ctx, const bpp_circuit *cir, const 
         bpp_acp_batch_free(b);
         return oom ? BPP_ERR_OOM : BPP_ERR_CUDA;
     }
+    if (int rc = acp_prepare_hsum(b)) {
+        bpp_acp_batch_free(b);
+        return rc;
+    }
     *out = b;
     return BPP_OK;
 }
@@ -657,13 +677,88 @@ static fb_plan acp_fb_plan(const bpp_acp_batch *b, const fb_shape &sh) {
     return fb_choose(b->ctx, (uint64_t)b->B * sh.outs, fb_terms(sh), b->gens->pts->fb_Wn, !sh.sel_period,
                      sh.outs > 8 ? 1 : b->fb_splits);
 }
+// A_I = alpha*h + <a_L,G> + <a_R,H>.  For a witness of bpp_acp_batch_gen_shuffle_witness, a_R[i] = v'[i] - x on the first
+// n - 2 multipliers and 0 on the last two, so (the group has prime order) <a_R,H> = <v',H> + (-x) H_sum with H_sum =
+// H_0 + .. + H_{n-3}: the same point.  Card values are small integers, so v' has one non-zero digit where a_R has
+// Wn, and the digit-staged warp kernel spreads those digits over all lanes (fb_sparse): A_I costs (1 + n/2) x Wn
+// + (n - 2) + Wn table adds per proof instead of (1 + n) x Wn for a small deck (52 cards, c = 16: 1766 instead of
+// 3280).  structured: that shape, which only the digit-staged warp form runs (acp_ai_structured_ok).
+static fb_shape acp_ai_shape(const bpp_acp_batch *b, bool structured, fb_sparse *sp = nullptr) {
+    const acp_layout &L = b->lay;
+    const uint32_t gH = 2 + b->gens->n;   // first H generator (gens order g, h, G[..], H[..])
+    fb_shape sh = acp_shape(1);
+    acp_seg(sh, L.alpha, 0, 1, 1); acp_seg(sh, L.aL, 0, 2, L.n);
+    if (!structured) {
+        acp_seg(sh, L.aR, 0, gH, L.n);
+        return sh;
+    }
+    acp_seg(sh, L.vr, 0, gH, L.n - 2); acp_seg(sh, L.nx, 0, 0, 1);
+    if (sp) *sp = fb_sparse{1, 1u << 3, b->hsum ? b->hsum->fb_table : nullptr};
+    return sh;
+}
+static bool acp_ai_structured_ok(const bpp_acp_batch *b) {
+    if (!acp_shuffle_shaped(b->lay.n, b->lay.m)) return false;
+    const bpp_points &P = *b->gens->pts;
+    fb_sparse sp;
+    const fb_shape sh = acp_ai_shape(b, true, &sp);
+    return acp_fb_plan(b, sh).form == FB_WARP && fb_warp_d_fits(sh, sp, P.fb_c, P.fb_Wn);
+}
+// H_sum's table for batches that can use the structured A_I, shared by every batch over the same generators: built on
+// first use (one warp sums the points, the sum goes through compression and bpp_points_upload, then gets its own table
+// at the generators' width), looked up under the generators' lock afterwards.
+static int acp_prepare_hsum(bpp_acp_batch *b) {
+    if (!acp_ai_structured_ok(b)) return BPP_OK;
+    bpp_ctx *ctx = b->ctx;
+    bpp_gens *g = const_cast<bpp_gens *>(b->gens);
+    const uint32_t first = 2 + g->n, cnt = b->lay.n - 2;
+    const int c = g->pts->fb_c;
+    std::lock_guard<std::mutex> lock(g->mu);
+    for (const auto &e : g->sums)
+        if (e.first == first && e.cnt == cnt && e.pts->fb_c == c) {
+            b->hsum = e.pts;
+            return BPP_OK;
+        }
+    uint32_t *d = nullptr;
+    CK(ctx, cudaMalloc((void **)&d, 128 + 32));
+    uint8_t enc[32];
+    k_point_sum<<<1, 32, 0, ctx->stream>>>(g->pts->niels, first, cnt, d);
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess) {
+        k_compress_batch<<<1, 128, 0, ctx->stream>>>(d, 1, (uint8_t *)(d + 32));
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(enc, d + 32, 32, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    cudaFree(d);
+    if (e != cudaSuccess) {
+        ctx->last_error = cudaGetErrorString(e);
+        return BPP_ERR_CUDA;
+    }
+    ctx->launches += 2;
+    bpp_points *pts = nullptr;
+    int rc = bpp_points_upload(ctx, BPP_FMT_COMPRESSED, enc, 1, &pts);
+    if (rc) return rc;
+    if ((rc = bpp_points_precompute(ctx, pts, c))) {
+        bpp_points_free(ctx, pts);
+        return rc;
+    }
+    g->sums.push_back({first, cnt, pts});
+    b->hsum = pts;
+    return BPP_OK;
+}
+
 // The fixed-base MSM launch over B proof blocks of layout `lay` in the form `pl`: results land in dst[(p * pitch + o)]
 // (raw extended points).  part: the split scratch of the block form (B x outs x pl.splits partial sums); deferred_splits:
 // when given and the launch is split, the partial sums are left there for the caller's own tail kernel (their count is
 // written; 1 = the result is complete in dst).
 static int fb_launch(bpp_ctx *ctx, const uint32_t *blk, const acp_layout &lay, uint32_t B, const bpp_points &P, const fb_shape &sh,
-                     const fb_plan &pl, uint32_t *dst, uint32_t pitch, cudaStream_t st, uint32_t *part, uint32_t *deferred_splits) {
+                     const fb_plan &pl, uint32_t *dst, uint32_t pitch, cudaStream_t st, uint32_t *part, uint32_t *deferred_splits,
+                     const fb_sparse &sp = fb_sparse{}) {
     if (deferred_splits) *deferred_splits = 1;
+    if ((sp.on || sp.alt) && !(pl.form == FB_WARP && fb_warp_d_fits(sh, sp, P.fb_c, P.fb_Wn))) {
+        ctx->last_error = "fixed-base MSM: a sparse / two-table shape needs the digit-staged warp form";
+        return BPP_ERR_INVALID_ARG;
+    }
     fb_shape s = sh;
     s.outs = pitch;  // the kernels address out_ext + 32 * (p * outs + o)
     fb_consts kc;
@@ -673,7 +768,7 @@ static int fb_launch(bpp_ctx *ctx, const uint32_t *blk, const acp_layout &lay, u
         k_fb_msm_small<<<(total + 127) / 128, 128, 0, st>>>(blk, lay, s, P.fb_table, P.fb_c, P.fb_Wn, kc, B, sh.outs, dst);
         LAUNCH_CHECK(ctx);
     } else if (pl.form == FB_WARP) {
-        fb_warp_launch(blk, lay, s, P.fb_table, P.fb_c, P.fb_Wn, kc, B, sh.outs, dst, st);
+        fb_warp_launch(blk, lay, s, P.fb_table, P.fb_c, P.fb_Wn, kc, B, sh.outs, dst, st, sp);
         LAUNCH_CHECK(ctx);
     } else {
         k_fb_msm<<<dim3(B, sh.outs, pl.splits), FB_THREADS, 0, st>>>(blk, lay, s, P.fb_table, P.fb_c, P.fb_Wn, kc,
@@ -692,19 +787,19 @@ static int fb_launch(bpp_ctx *ctx, const uint32_t *blk, const acp_layout &lay, u
 // commitments side by side); part_region: which eighth of the split scratch to use (concurrent split launches must not
 // share it).  With the priority split, the GPU-filling forms go to the low-priority stream.
 static int acp_fb(bpp_acp_batch *b, const fb_shape &sh, uint32_t *dst, uint32_t pitch, cudaStream_t on = nullptr,
-                  uint32_t part_region = 0, uint32_t *deferred_splits = nullptr) {
+                  uint32_t part_region = 0, uint32_t *deferred_splits = nullptr, const fb_sparse &sp = fb_sparse{}) {
     bpp_ctx *ctx = b->ctx;
     const bpp_points &P = *b->gens->pts;
     const fb_plan pl = acp_fb_plan(b, sh);
     uint32_t *part = b->d_part + 32 * (size_t)part_region * b->B * b->fb_splits;
-    if (pl.form == FB_SMALL) return fb_launch(ctx, b->d_blk, b->lay, b->B, P, sh, pl, dst, pitch, ctx->stream, part, deferred_splits);
+    if (pl.form == FB_SMALL) return fb_launch(ctx, b->d_blk, b->lay, b->B, P, sh, pl, dst, pitch, ctx->stream, part, deferred_splits, sp);
     cudaStream_t st = on ? on : ctx->stream;
     if (b->priority_split && !on) {   // the GPU-filling launch goes to the low-priority stream, bracketed by events
         st = b->bulk;
         CK(ctx, cudaEventRecord(b->ev_bfork, ctx->stream));
         CK(ctx, cudaStreamWaitEvent(st, b->ev_bfork, 0));
     }
-    int rc = fb_launch(ctx, b->d_blk, b->lay, b->B, P, sh, pl, dst, pitch, st, part, deferred_splits);
+    int rc = fb_launch(ctx, b->d_blk, b->lay, b->B, P, sh, pl, dst, pitch, st, part, deferred_splits, sp);
     if (rc) return rc;
     if (b->priority_split && !on) {
         CK(ctx, cudaEventRecord(b->ev_bjoin, st));
@@ -744,6 +839,7 @@ extern "C" int bpp_acp_batch_upload_witness(bpp_acp_batch *b, const uint8_t *aL,
         LAUNCH_CHECK(ctx);
     }
     CK(ctx, cudaMemcpyAsync(b->d_seeds, seeds, (size_t)b->B * 32, cudaMemcpyHostToDevice, ctx->stream));
+    b->shuffle_wit = false;
     return BPP_OK;
 }
 
@@ -786,6 +882,7 @@ extern "C" int bpp_acp_batch_gen_shuffle_witness(bpp_acp_batch *b, const uint8_t
     }
     LAUNCH_CHECK(ctx);
     b->have_vwit = true;
+    b->shuffle_wit = true;
     return BPP_OK;
 }
 
@@ -1078,10 +1175,12 @@ extern "C" int bpp_acp_batch_prove(bpp_acp_batch *b) {
             CK(ctx, cudaStreamWaitEvent(b->aux, b->ev_fork, 0));
             CK(ctx, cudaStreamWaitEvent(b->aux3, b->ev_fork, 0));
         }
-        fb_shape sh = acp_shape(1);
+        const bpp_points &P = *b->gens->pts;
+        const bool structured = b->shuffle_wit && b->hsum && b->hsum->fb_c == P.fb_c && acp_ai_structured_ok(b);
+        fb_sparse sp{};
+        fb_shape sh = acp_ai_shape(b, structured, &sp);
+        if ((rc = acp_fb(b, sh, b->d_ext8 + 0, 8, nullptr, 0, nullptr, sp))) return rc;
         const uint32_t gH = 2 + b->gens->n;   // first H generator (gens order g, h, G[..], H[..])
-        acp_seg(sh, L.alpha, 0, 1, 1); acp_seg(sh, L.aL, 0, 2, n); acp_seg(sh, L.aR, 0, gH, n);
-        if ((rc = acp_fb(b, sh, b->d_ext8 + 0, 8))) return rc;
         sh = acp_shape(1);
         acp_seg(sh, L.beta, 0, 1, 1); acp_seg(sh, L.aO, 0, 2, n);
         if ((rc = acp_fb(b, sh, b->d_ext8 + 32, 8, side ? b->aux : nullptr, side ? 1 : 0))) return rc;
@@ -1466,8 +1565,7 @@ extern "C" int bpp_acp_batch_time_commit_msm(bpp_acp_batch *b, int reps, float *
     bpp_ctx *ctx = b->ctx;
     CK(ctx, cudaSetDevice(ctx->device));
     const acp_layout &L = b->lay;
-    fb_shape sh = acp_shape(1);
-    acp_seg(sh, L.alpha, 0, 1, 1); acp_seg(sh, L.aL, 0, 2, L.n); acp_seg(sh, L.aR, 0, 2 + b->gens->n, L.n);
+    const fb_shape sh = acp_ai_shape(b, false);   // the generic A_I shape whatever the witness
     int rc = acp_fb(b, sh, b->d_ext8, 8);  // warm-up
     if (rc) return rc;
     cudaEvent_t e0, e1;
