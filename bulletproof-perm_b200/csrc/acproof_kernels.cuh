@@ -95,7 +95,14 @@ __global__ void __launch_bounds__(128) k_acp_place_witness(const uint32_t *__res
 // dependent multiplications deep instead of 4095.  Products in Montgomery form until the final store.
 // Both forms also write a_R in its structured form: v'[gb + i] = v[vb + i + 1] and -x (sc_sub(0, x)), so that the prover
 // can commit <a_R, H> as <v', H> + (-x) H_sum (bpp_acp_batch_prove).
+// perm is device data: an index >= k asserts in the debug build and is clamped to k - 1 in the product build, so that
+// it reads the deck's last card instead of whatever follows the deck (device data must not fault).
 #define WIT_THREADS 256
+FE_INLINE uint32_t wit_card(const uint32_t *pp, uint32_t j, uint32_t k) {
+    const uint32_t i = pp[j];
+    BPP_ASSERT(i < k);
+    return i < k ? i : k - 1;
+}
 SC_INLINE void acp_store_neg_x(uint32_t *blk, const acp_layout &lay, uint32_t p, const sc &x) {
     sc z, nx;
     sc_set0(z);
@@ -120,8 +127,8 @@ __global__ void __launch_bounds__(WIT_THREADS) k_shuffle_witness(const uint32_t 
     sc_const(r2, SC_R2);
     auto value = [&](uint32_t j) {      // v[vb + j], also written out
         sc v;
-        BPP_ASSERT(j < k && (!c || pp[j] < k));
-        sc_load(v, deck + 8 * (size_t)(c ? pp[j] : j));
+        BPP_ASSERT(j < k);
+        sc_load(v, deck + 8 * (size_t)(c ? wit_card(pp, j, k) : j));
         sc_store(vp + 8 * (size_t)(vb + j), v);
         return v;
     };
@@ -203,15 +210,13 @@ __global__ void __launch_bounds__(64) k_shuffle_witness_serial(const uint32_t *_
     sc x, r2, v, f, fm, P;
     sc_load(x, xs + 8 * (size_t)p);
     sc_const(r2, SC_R2);
-    BPP_ASSERT(!c || pp[0] < k);
-    sc_load(v, deck + 8 * (size_t)(c ? pp[0] : 0));
+    sc_load(v, deck + 8 * (size_t)(c ? wit_card(pp, 0, k) : 0));
     sc_store(vp + 8 * (size_t)vb, v);
     sc_sub(P, v, x);
     sc_store(ACP_PTR(blk, lay, p, lay.aL + gb), P);
 #pragma unroll 1
     for (uint32_t i = 0; i < len; i++) {
-        BPP_ASSERT(!c || pp[i + 1] < k);
-        sc_load(v, deck + 8 * (size_t)(c ? pp[i + 1] : i + 1));
+        sc_load(v, deck + 8 * (size_t)(c ? wit_card(pp, i + 1, k) : i + 1));
         sc_store(vp + 8 * (size_t)(vb + i + 1), v);
         sc_store(ACP_PTR(blk, lay, p, lay.vr + gb + i), v);
         sc_sub(f, v, x);

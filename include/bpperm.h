@@ -299,7 +299,10 @@ int bpp_acp_batch_upload_witness(bpp_acp_batch *b, const uint8_t *aL, const uint
  * of bpp_circuit_create_shuffle): deck = k card values (k x 32, shared by the batch), perm = count x k indices into the
  * deck (proof p's output deck is deck[perm[p][i]]), x = count x 32 challenge values, gamma = count x m x 32 blindings,
  * seeds = count x 32 prover RNG seeds.  Leaves a_L, a_R, a_O, gamma and v = deck | deck[perm] | x resident
- * (bpp_acp_batch_commit with v = NULL commits to that v). */
+ * (bpp_acp_batch_commit with v = NULL commits to that v).  perm is not checked on the host (it may be a device
+ * address) and cannot make the call fault: an index >= k is clamped to k - 1, i.e. read as the deck's last card (the
+ * -DBPP_DEBUG_BOUNDS build asserts instead).  perm is not required to be a permutation; a witness built from one that
+ * is not is not a shuffle, and the verifier rejects its proof. */
 int bpp_acp_batch_gen_shuffle_witness(bpp_acp_batch *b, const uint8_t *deck, const uint32_t *perm, const uint8_t *x,
                                       const uint8_t *gamma, const uint8_t *seeds);
 /* commit_variables (weights.rs:58-61): V_j = v_j*g + gamma_j*h with the uploaded gamma; V_out nullable; v = NULL: the

@@ -431,6 +431,46 @@ def run_flow(core, prover, V, rng, mode="reference-fixed", label=b"test", msm=No
     return proof.proof_bytes(Ts), ok, (y, z, x), proof
 
 
+def verify_proof_bytes(core, V_enc, proof: bytes, mode="reference-fixed", label=b"test", msm=None) -> bool:
+    """The verifier of circuit_lib.rs:478-585 from the proof bytes alone, where ArithmeticCircuitProof.verify reads the
+    prover's own state.  proof: A_I, A_O, S, T_1, T_3..T_6, tau_x, mu, t, l[0..n), r[0..n) as proof_bytes writes them;
+    V_enc: the m commitments' encodings (a list, or their concatenation).  The transcript is replayed from these bytes
+    as create .. random_chall_x append them (mode "reference-fixed"/1: with append_commitments; "reference"/0: without,
+    and "T4" carries T_3's bytes), then checks 1-3 run as in verify(), defects and corrections included.
+    Decoding rules, those of the library's verifier: a scalar >= l is taken mod l; an undecodable point or commitment is
+    a reject (the reference would panic on an undecodable T, circuit_lib.rs:532); the all-zero encoding is the identity."""
+    mode = {0: "reference", 1: "reference-fixed"}.get(mode, mode)
+    n, Q, m = len(core["G_vec"]), len(core["W_L"][0]), len(core["W_V"])
+    if isinstance(V_enc, (bytes, bytearray)):
+        V_enc = [bytes(V_enc[32 * j:32 * j + 32]) for j in range(len(V_enc) // 32)]
+    if len(proof) != 32 * (11 + 2 * n) or len(V_enc) != m:
+        raise ValueError("proof: 32 (11 + 2 n) bytes; V_enc: m encodings")
+    enc = [bytes(proof[32 * i:32 * i + 32]) for i in range(11 + 2 * n)]
+    pts = [R.decompress(e) for e in enc[:8]]
+    V = [R.decompress(bytes(e)) for e in V_enc]
+    if any(p is None for p in pts + V):
+        return False
+    sc = [int.from_bytes(e, "little") % L for e in enc[8:]]
+    self = ArithmeticCircuitProof(mode, msm)
+    self.core, self.n, self.m, self.Q = core, n, m, Q
+    self.A_I, self.A_O, self.S = pts[:3]
+    self.tau_x, self.mu, self.t = sc[:3]
+    self.l, self.r = sc[3:3 + n], sc[3 + n:]
+    trans = Transcript(label)
+    trans.arithmetic_domain_sep(n)
+    if mode != "reference":
+        append_commitments(trans, V_enc, m)
+    for lab, e in zip((b"A_I", b"A_O", b"S"), enc[:3]):
+        trans.append_point(lab, e)
+    y, z = self.challenge_wit_and_const(trans)
+    _, z_q, sigma = self.compute_per_challenges(y, z)
+    Ts = enc[3:8]
+    for lab, e in zip((b"T1", b"T3", b"T4", b"T5", b"T6"), Ts):
+        trans.append_point(lab, Ts[1] if mode == "reference" and lab == b"T4" else e)
+    x = self.random_chall_x(trans)
+    return self.verify(trans, z_q, sigma, x, V, Ts)
+
+
 def make_instance(k, rng, dense_weights=True):
     """Synthetic k-card instance in the reference's shapes: generators as RistrettoPoint::random
     (lib.rs:164-167,179-180), the corrected shuffle circuit, witness, blindings, commitments.

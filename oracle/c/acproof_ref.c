@@ -120,6 +120,7 @@ static void sc_from_wide(sc *r, const u8 in[64]) { /* Scalar::from_bytes_mod_ord
     sc_add(r, &a, &b);
 }
 static void sc_from_u64(sc *r, u64 x) { r->v[0] = x; r->v[1] = r->v[2] = r->v[3] = 0; }
+static void sc_from_bytes_mod_order(sc *r, const u8 *b) { u8 w[64] = {0}; memcpy(w, b, 32); sc_from_wide(r, w); }
 
 /* ------------------------------------------------------------------ util.rs / poly.rs ---------- */
 static void v_inner_product(sc *out, const sc *a, const sc *b, size_t n) { /* util.rs:84-94 */
@@ -345,10 +346,107 @@ static void tr_append_commitments(strobe *tr, const ge_ext *V, const u8 *V_enc, 
     free(digs);
 }
 
+/* verify :478-585 from the proof bytes alone (A_I,A_O,S,T1,T3,T4,T5,T6,tau_x,mu,t,l,r): replays the verifier's
+ * transcript from those bytes (mode 1: with the commitment binding; mode 0: "T4" carries T_3's bytes), then checks
+ * 1 (t == <l, r>), 2 and, in mode 1, 3.  Decoding as the library's verifier: a scalar >= l is taken mod l, an
+ * undecodable point is a reject (the reference unwraps T and panics, circuit_lib.rs:532), the all-zero encoding is the
+ * identity.  V: the commitments as points; V_enc, when given, is what the transcript binds.  Returns 1 for Ok(()). */
+static int acp_verify(int mode, size_t n, size_t Q, size_t m, const sc *W_L, const sc *W_R, const sc *W_O, const sc *W_V,
+                      const sc *cv, const ge_ext *g, const ge_ext *h, const ge_ext *G, const ge_ext *H, const u8 *po,
+                      const ge_ext *V, const u8 *V_enc, const u8 *label, size_t label_len) {
+    static const int DEG[5] = {1, 3, 4, 5, 6};
+    static const char *TL[5] = {"T1", "T3", "T4", "T5", "T6"};
+    ge_ext pts8[8];
+    for (int k = 0; k < 8; k++)
+        if (!ristretto_decompress(&pts8[k], po + 32 * k)) return 0;
+    const ge_ext A_I = pts8[0], A_O = pts8[1], S = pts8[2];
+    size_t big = 2 * n + m + 16;
+    sc *sv = malloc(big * sizeof(sc)); ge_ext *pv = malloc(big * sizeof(ge_ext));
+    sc tau_x, mu, that;
+    sc_from_bytes_mod_order(&tau_x, po + 256); sc_from_bytes_mod_order(&mu, po + 288); sc_from_bytes_mod_order(&that, po + 320);
+    sc *l = malloc(n * sizeof(sc)), *r = malloc(n * sizeof(sc));
+    for (size_t i = 0; i < n; i++) { sc_from_bytes_mod_order(&l[i], po + 352 + 32 * i); sc_from_bytes_mod_order(&r[i], po + 352 + 32 * (n + i)); }
+    /* ---- the transcript, as create .. random_chall_x appended it ---- */
+    strobe tr; tr_new(&tr, label, label_len);
+    { u8 nb[8]; for (int i = 0; i < 8; i++) nb[i] = (u8)((u64)n >> (8 * i)); tr_append(&tr, "dom-sep", (const u8 *)"acp v1", 6); tr_append(&tr, "n", nb, 8); }
+    if (mode != 0) tr_append_commitments(&tr, V, V_enc, m);
+    tr_append(&tr, "A_I", po, 32); tr_append(&tr, "A_O", po + 32, 32); tr_append(&tr, "S", po + 64, 32);
+    sc y, z; tr_challenge_scalar(&tr, "y", &y); tr_challenge_scalar(&tr, "z", &z);
+    for (int k = 0; k < 5; k++) tr_append(&tr, TL[k], (mode == 0 && k == 2) ? po + 96 + 32 : po + 96 + 32 * k, 32);
+    sc x; tr_challenge_scalar(&tr, "x", &x);
+    /* ---- compute_per_challenges :256-302 ---- */
+    sc *y_n = malloc(n * sizeof(sc)), *y_n_inv = malloc(n * sizeof(sc)), *z_q = malloc(Q * sizeof(sc));
+    sc *z_W_R = malloc(n * sizeof(sc)), *z_W_L = malloc(n * sizeof(sc)), *l_in = malloc(n * sizeof(sc));
+    sc *tmp = malloc((Q > n ? Q : n) * sizeof(sc));
+    v_exp_iter(y_n, &y, n);
+    for (size_t i = 0; i < n; i++) sc_invert(&y_n_inv[i], &y_n[i]);
+    v_exp_iter(z_q, &z, Q);
+    v_vm_mult(z_W_R, z_q, W_R, n, Q);
+    v_hadamard(l_in, y_n_inv, z_W_R, n);
+    v_vm_mult(z_W_L, z_q, W_L, n, Q);
+    sc sigma; v_inner_product(&sigma, l_in, z_W_L, n);
+    sc xx, xp3; sc_mul(&xx, &x, &x); v_scalar_exp(&xp3, &x, 3);
+    int result = 1;
+    ge_ext *h_ = malloc(n * sizeof(ge_ext));
+    for (size_t i = 0; i < n; i++) ge_scalarmul_radix16(&h_[i], &y_n_inv[i], &H[i]);           /* :491 */
+    ge_ext wL, wR, wO;
+    msm_sc(&wL, z_W_L, h_, n);                                                                 /* :498 */
+    msm_sc(&wR, l_in, G, n);                                                                   /* :504 */
+    v_vm_mult(tmp, z_q, W_O, n, Q); msm_sc(&wO, tmp, h_, n);                                   /* :509 */
+    sc chk; v_inner_product(&chk, l, r, n);
+    if (memcmp(chk.v, that.v, 32) != 0) result = 0;                                            /* :518 */
+    if (result) {
+        sc g_exp, zc; v_inner_product(&zc, z_q, cv, Q); sc_add(&zc, &zc, &sigma); sc_mul(&g_exp, &xx, &zc);
+        sc *zwv = malloc(m * sizeof(sc)); v_vm_mult(zwv, z_q, W_V, m, Q);
+        sv[0] = g_exp; pv[0] = *g;
+        for (size_t j = 0; j < m; j++) { sc_mul(&sv[1 + j], &xx, &zwv[j]); pv[1 + j] = V[j]; }
+        for (int k = 0; k < 5; k++) { v_scalar_exp(&sv[1 + m + k], &x, DEG[k]); pv[1 + m + k] = pts8[3 + k]; }
+        free(zwv);
+        ge_ext cand, lhs; msm_sc(&cand, sv, pv, 1 + m + 5);                                    /* :525-533 */
+        sv[0] = that; sv[1] = tau_x; pv[0] = *g; pv[1] = *h; msm_sc(&lhs, sv, pv, 2);          /* :535-538 */
+        if (!ge_ristretto_eq(&lhs, &cand)) result = 0;                                         /* :541 */
+    }
+    if (result == 1) {
+        sc one = {{1, 0, 0, 0}};
+        sv[0] = x; sv[1] = xx; pv[0] = A_I; pv[1] = A_O;
+        for (size_t i = 0; i < n; i++) { sc_neg(&sv[2 + i], &y_n[i]); pv[2 + i] = h_[i]; }
+        sv[2 + n] = x; sv[3 + n] = x; sv[4 + n] = one; sv[5 + n] = xp3;
+        pv[2 + n] = wL; pv[3 + n] = wR; pv[4 + n] = wO; pv[5 + n] = S;
+        ge_ext P, candP; msm_sc(&P, sv, pv, n + 6);                                            /* :552-565 */
+        sv[0] = mu; pv[0] = *h; memcpy(sv + 1, l, n * 32); memcpy(sv + 1 + n, r, n * 32);
+        memcpy(pv + 1, G, n * sizeof(ge_ext)); memcpy(pv + 1 + n, mode == 0 ? H : h_, n * sizeof(ge_ext));
+        msm_sc(&candP, sv, pv, 1 + 2 * n);                                                     /* :568-575 */
+        if (mode != 0 && !ge_ristretto_eq(&P, &candP)) result = 0;                             /* :577-582 disabled in mode 0 */
+    }
+    free(h_); free(sv); free(pv); free(l); free(r); free(y_n); free(y_n_inv); free(z_q); free(z_W_R); free(z_W_L);
+    free(l_in); free(tmp);
+    return result;
+}
+
+/* The verifier alone (acp_verify) over caller proof bytes.  V_pts: the commitments as points, or NULL to decode them
+ * from V_enc (an undecodable commitment is a reject); V_enc NULL: the transcript binds the compressed V_pts. */
+int orc_acp_verify(int mode, size_t n, size_t Q, size_t m, const u8 *WLb, const u8 *WRb, const u8 *WOb, const u8 *WVb,
+                   const u8 *cb, const u8 *g_pt, const u8 *h_pt, const u8 *G_pts, const u8 *H_pts, const u8 *proof,
+                   const u8 *V_pts, const u8 *V_enc, const u8 *label, size_t label_len) {
+    orc_init();
+    if (!V_pts && !V_enc) return -1;
+    ge_ext *Vd = NULL;
+    if (!V_pts) {
+        Vd = malloc(m * sizeof(ge_ext));
+        for (size_t j = 0; j < m; j++)
+            if (!ristretto_decompress(&Vd[j], V_enc + 32 * j)) { free(Vd); return 0; }
+    }
+    int rc = acp_verify(mode, n, Q, m, (const sc *)WLb, (const sc *)WRb, (const sc *)WOb, (const sc *)WVb, (const sc *)cb,
+                        (const ge_ext *)g_pt, (const ge_ext *)h_pt, (const ge_ext *)G_pts, (const ge_ext *)H_pts, proof,
+                        V_pts ? (const ge_ext *)V_pts : Vd, V_enc, label, label_len);
+    free(Vd);
+    return rc;
+}
+
 /* lib.rs:219-231 / circuit_lib.rs:133-585.  W_* dense, row-major: W_L,W_R,W_O n x Q, W_V m x Q.
  * mode 0 = reference (defects included), 1 = reference-fixed.  Writes the proof bytes
- * (A_I,A_O,S,T1,T3,T4,T5,T6,tau_x,mu,t,l,r) and returns 1 for Ok(()), 0 for Err(VerificationError),
- * -5 for an undecodable T (the reference panics). */
+ * (A_I,A_O,S,T1,T3,T4,T5,T6,tau_x,mu,t,l,r) and, with do_verify, returns acp_verify's decision over them:
+ * 1 for Ok(()), 0 for Err(VerificationError). */
 int orc_acp_prove_verify(int mode, size_t n, size_t Q, size_t m, const u8 *WLb, const u8 *WRb, const u8 *WOb,
                          const u8 *WVb, const u8 *cb, const u8 *g_pt, const u8 *h_pt, const u8 *G_pts, const u8 *H_pts,
                          const u8 *aLb, const u8 *aRb, const u8 *aOb, const u8 *gammab, const u8 *V_pts, const u8 *V_enc,
@@ -458,50 +556,10 @@ int orc_acp_prove_verify(int mode, size_t n, size_t Q, size_t m, const u8 *WLb, 
     tr_append_vec_scalar(&tr, "l", l, n); tr_append_vec_scalar(&tr, "r", r, n); tr_append_scalar(&tr, "t", &that);
     sc_tobytes(po + 256, &tau_x); sc_tobytes(po + 288, &mu); sc_tobytes(po + 320, &that);
     memcpy(po + 352, l, n * 32); memcpy(po + 352 + 32 * n, r, n * 32);
-    int result = 1;
-    if (do_verify) {
-        /* ---- verify :478-585 ---- */
-        ge_ext *h_ = malloc(n * sizeof(ge_ext));
-        for (size_t i = 0; i < n; i++) ge_scalarmul_radix16(&h_[i], &y_n_inv[i], &H[i]);       /* :491 */
-        ge_ext wL, wR, wO;
-        msm_sc(&wL, z_W_L, h_, n);                                                             /* :498 */
-        msm_sc(&wR, l_in, G, n);                                                               /* :504 */
-        v_vm_mult(tmp, z_q, W_O, n, Q); msm_sc(&wO, tmp, h_, n);                               /* :509 */
-        sc chk; v_inner_product(&chk, l, r, n);
-        if (memcmp(chk.v, that.v, 32) != 0) result = 0;                                        /* :518 */
-        if (result) {
-            sc g_exp, zc; v_inner_product(&zc, z_q, cv, Q); sc_add(&zc, &zc, &sigma); sc_mul(&g_exp, &xx, &zc);
-            sc *zwv = malloc(m * sizeof(sc)); v_vm_mult(zwv, z_q, W_V, m, Q);
-            sv[0] = g_exp; pv[0] = *g;
-            for (size_t j = 0; j < m; j++) { sc_mul(&sv[1 + j], &xx, &zwv[j]); pv[1 + j] = V[j]; }
-            for (int k = 0; k < 5; k++) {
-                v_scalar_exp(&sv[1 + m + k], &x, DEG[k]);
-                if (!ristretto_decompress(&pv[1 + m + k], po + 96 + 32 * k)) { result = -5; break; }
-            }
-            free(zwv);
-            if (result == 1) {
-                ge_ext cand, lhs; msm_sc(&cand, sv, pv, 1 + m + 5);                            /* :525-533 */
-                sv[0] = that; sv[1] = tau_x; pv[0] = *g; pv[1] = *h; msm_sc(&lhs, sv, pv, 2);   /* :535-538 */
-                if (!ge_ristretto_eq(&lhs, &cand)) result = 0;                                 /* :541 */
-            }
-        }
-        if (result == 1) {
-            sc one = {{1, 0, 0, 0}};
-            sv[0] = x; sv[1] = xx; pv[0] = A_I; pv[1] = A_O;
-            for (size_t i = 0; i < n; i++) { sc_neg(&sv[2 + i], &y_n[i]); pv[2 + i] = h_[i]; }
-            sv[2 + n] = x; sv[3 + n] = x; sv[4 + n] = one; sv[5 + n] = xp3;
-            pv[2 + n] = wL; pv[3 + n] = wR; pv[4 + n] = wO; pv[5 + n] = S;
-            ge_ext P, candP; msm_sc(&P, sv, pv, n + 6);                                        /* :552-565 */
-            sv[0] = mu; pv[0] = *h; memcpy(sv + 1, l, n * 32); memcpy(sv + 1 + n, r, n * 32);
-            memcpy(pv + 1, G, n * sizeof(ge_ext)); memcpy(pv + 1 + n, mode == 0 ? H : h_, n * sizeof(ge_ext));
-            msm_sc(&candP, sv, pv, 1 + 2 * n);                                                 /* :568-575 */
-            if (mode != 0 && !ge_ristretto_eq(&P, &candP)) result = 0;                         /* :577-582 disabled in mode 0 */
-        }
-        free(h_);
-    }
     free(sv); free(pv); free(s_l); free(s_r); free(y_n); free(y_n_inv); free(z_q); free(z_W_R); free(z_W_L); free(l_in);
     free(l1); free(r0); free(r1); free(r3); free(tmp); free(tmp2); free(l); free(r); free(zero); free(wvq);
-    return result;
+    if (!do_verify) return 1;
+    return acp_verify(mode, n, Q, m, W_L, W_R, W_O, W_V, cv, g, h, G, H, po, V, V_enc, label, label_len);
 }
 
 /* PedersenGens::commit (weights.rs:58-61): v*B + r*B_blinding for m values */
@@ -540,7 +598,6 @@ static void v_sparse_vm(sc *out, size_t rows, const sc *z_q, const u32 *wire, co
     for (size_t e = 0; e < nnz; e++) { sc t; sc_mul(&t, &coeff[e], &z_q[cons[e]]); sc_add(&out[wire[e]], &out[wire[e]], &t); }
 }
 static int is_zero32(const u8 *b) { u8 o = 0; for (int i = 0; i < 32; i++) o |= b[i]; return o == 0; }
-static void sc_from_bytes_mod_order(sc *r, const u8 *b) { u8 w[64] = {0}; memcpy(w, b, 32); sc_from_wide(r, w); }
 
 size_t orc_acp_fixed_proof_len(size_t n) {
     size_t np = next_pow2_sz(n), lg = 0; while (((size_t)1 << lg) < np) lg++;

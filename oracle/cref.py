@@ -47,6 +47,7 @@ def lib():
         l.orc_msm_vartime_mt.restype = None
         l.orc_acp_prove_verify.argtypes = [c.c_int, c.c_size_t, c.c_size_t, c.c_size_t] + [c.c_char_p] * 17 + [
             c.c_size_t, c.c_char_p, c.c_int]
+        l.orc_acp_verify.argtypes = [c.c_int, c.c_size_t, c.c_size_t, c.c_size_t] + [c.c_char_p] * 13 + [c.c_size_t]
         l.orc_acp_fixed_proof_len.argtypes = [c.c_size_t]
         l.orc_acp_fixed_proof_len.restype = c.c_size_t
         l.orc_acp_fixed_prove_verify.argtypes = [c.c_size_t, c.c_size_t, c.c_size_t, c.c_char_p, c.c_char_p, c.c_char_p] + [
@@ -131,6 +132,20 @@ class AcpInstance:
                                         self.g, self.h, self.G, self.H, aL, aR, aO, gamma, V_pts, V_enc, seed, label,
                                         len(label), out, 1 if do_verify else 0)
         return out.raw, rc
+
+    def verify(self, proof: bytes, V_pts, mode=1, V_enc=None, label=b"test") -> bool:
+        """The verifier of modes 0 and 1 from the proof bytes alone (orc_acp_verify): the transcript is replayed from
+        them, a scalar >= l is taken mod l, an undecodable point is a reject and the all-zero encoding is the identity.
+        V_pts: the commitments as points (orc layout), or None to decode them from V_enc (an undecodable commitment is
+        a reject); V_enc: the encodings the transcript binds (default: V_pts compressed)."""
+        if len(proof) != 32 * (11 + 2 * self.n):
+            raise ValueError("proof: 32 (11 + 2 n) bytes")
+        if V_pts is None and V_enc is None:
+            raise ValueError("verify: V_pts or V_enc")
+        mode = {"reference": 0, "reference-fixed": 1}.get(mode, mode)
+        rc = lib().orc_acp_verify(mode, self.n, self.Q, self.m, self.W[0], self.W[1], self.W[2], self.W[3], self.c,
+                                  self.g, self.h, self.G, self.H, proof, V_pts, V_enc, label, len(label))
+        return rc == 1
 
 
 class AcpFixedInstance:

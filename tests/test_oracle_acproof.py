@@ -93,3 +93,98 @@ def test_transcript_vec_scalar_encoding_is_stable():
     t = A.Transcript(b"test")
     t.append_vec_scalar(b"l", [0, 1, L - 1])
     assert len(t.challenge_bytes(b"c", 8)) == 8
+
+
+# ---- the verifier from proof bytes: oracle.acproof.verify_proof_bytes and cref.AcpInstance.verify -------------------
+def _flow(k, seed, mode):
+    core, prover, V = A.make_instance(k, ChaChaRng(bytes([seed]) * 32))
+    pb, ok, _, _ = A.run_flow(core, prover, V, ChaChaRng(bytes([seed + 1]) * 32), mode)
+    return core, V, pb, ok
+
+
+def _both(core, inst, V_enc, proof, mode):
+    """(Python, C) decisions; the C side decodes the commitments itself."""
+    py = A.verify_proof_bytes(core, V_enc, proof, mode)
+    c = inst.verify(proof, None, mode, V_enc=b"".join(V_enc))
+    return py, c
+
+
+def _sc_field(proof, f, value):
+    return proof[:32 * f] + value.to_bytes(32, "little") + proof[32 * f + 32:]
+
+
+@pytest.mark.parametrize("k", [2, 3, 5])
+@pytest.mark.parametrize("mode", [("reference-fixed", 1), ("reference", 0)])
+def test_from_bytes_verifiers_equal_run_flow_on_honest_proofs(k, mode):
+    core, V, pb, ok = _flow(k, 60 + k, mode[0])
+    assert ok == (mode[1] == 1)
+    inst = _c_instance(core)
+    V_enc = [R.compress(p) for p in V]
+    assert A.verify_proof_bytes(core, V_enc, pb, mode[0]) == ok
+    assert A.verify_proof_bytes(core, b"".join(V_enc), pb, mode[1]) == ok
+    assert inst.verify(pb, None, mode[1], V_enc=b"".join(V_enc)) == ok
+    Vp = cref.decompress(b"".join(V_enc))
+    assert inst.verify(pb, Vp, mode[1]) == ok                      # the transcript binds the compressed points
+    assert inst.verify(pb, Vp, mode[1], V_enc=b"".join(V_enc)) == ok
+    # the same bytes under the other transcript label are a different proof
+    assert not A.verify_proof_bytes(core, V_enc, pb, mode[0], label=b"other")
+    assert not inst.verify(pb, Vp, mode[1], label=b"other")
+
+
+def _corruptions(pb, n):
+    """(name, proof bytes): every 32-byte field with a bit flip, each point field with another valid point, the
+    identity, an invalid encoding and bit 255 set; each scalar field with +1 mod l, s + l and bit 255 set; A_I <-> A_O."""
+    out = []
+    other = R.compress(R.pt_mul(7, R.BASEPOINT))
+    for f in range(11 + 2 * n):
+        b = bytearray(pb)
+        b[32 * f + (f % 31)] ^= 1 << (f % 8)
+        out.append((f"flip{f}", bytes(b)))
+        if f < 8:
+            out.append((f"other{f}", pb[:32 * f] + other + pb[32 * f + 32:]))
+            out.append((f"identity{f}", pb[:32 * f] + bytes(32) + pb[32 * f + 32:]))
+            out.append((f"invalid{f}", pb[:32 * f] + b"\x01" + bytes(31) + pb[32 * f + 32:]))
+            s = int.from_bytes(pb[32 * f:32 * f + 32], "little")
+            out.append((f"bit255_{f}", _sc_field(pb, f, s | 1 << 255)))
+        else:
+            s = int.from_bytes(pb[32 * f:32 * f + 32], "little")
+            out.append((f"plus1_{f}", _sc_field(pb, f, (s + 1) % L)))
+            out.append((f"plusl_{f}", _sc_field(pb, f, s + L)))
+            out.append((f"bit255_{f}", _sc_field(pb, f, s | 1 << 255)))
+    out.append(("swapAIAO", pb[32:64] + pb[:32] + pb[64:]))
+    return out
+
+
+@pytest.mark.parametrize("mode", [("reference-fixed", 1), ("reference", 0)])
+def test_from_bytes_verifiers_agree_on_a_tamper_matrix(mode):
+    k = 2
+    core, V, pb, ok = _flow(k, 70, mode[0])
+    n, m = core["n"], core["m"]
+    inst = _c_instance(core)
+    V_enc = [R.compress(p) for p in V]
+    want_accept = set()
+    for name, bad in _corruptions(pb, n):
+        py, c = _both(core, inst, V_enc, bad, mode[0])
+        assert py == c, name
+        if py:
+            want_accept.add(name)
+    # s + l is s to the verifier: only those stay accepted, and only where the honest proof is
+    assert want_accept == ({f"plusl_{f}" for f in range(8, 11 + 2 * n)} if ok else set())
+    # the commitments: one V_j replaced by another valid point, by an invalid encoding, by the identity
+    for j in (0, m - 1):
+        for name, enc in (("other", R.compress(R.pt_mul(5, R.BASEPOINT))), ("invalid", b"\x01" + bytes(31)),
+                          ("identity", bytes(32))):
+            V2 = list(V_enc)
+            V2[j] = enc
+            assert _both(core, inst, V2, pb, mode[0]) == (False, False), (name, j)
+
+
+def test_scalar_taken_mod_l_pinned():
+    """tau_x + l decodes to tau_x (accepted); tau_x + 1 is another scalar (rejected)."""
+    core, V, pb, ok = _flow(3, 80, "reference-fixed")
+    assert ok
+    inst = _c_instance(core)
+    V_enc = [R.compress(p) for p in V]
+    tau_x = int.from_bytes(pb[256:288], "little")
+    assert _both(core, inst, V_enc, _sc_field(pb, 8, tau_x + L), 1) == (True, True)
+    assert _both(core, inst, V_enc, _sc_field(pb, 8, (tau_x + 1) % L), 1) == (False, False)
