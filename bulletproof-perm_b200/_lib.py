@@ -30,6 +30,7 @@ SYMBOLS = [
     "bpp_acp_batch_time_commit_msm", "bpp_acp_batch_set_host_transcripts", "bpp_transcript_script", "bpp_ipa_fold_generators", "bpp_acp_batch_set_batch_rlc", "bpp_acp_batch_set_priority_split",
     "bpp_transcript_new", "bpp_transcript_append_message", "bpp_transcript_challenge_bytes",
     "bpp_ipa_proof_len", "bpp_ipa_batch_create", "bpp_ipa_batch_free", "bpp_ipa_batch_prove", "bpp_ipa_batch_verify",
+    "bpp_ipa_batch_verify_combined", "bpp_ipa_batch_gather_accept", "bpp_ipa_batch_download_weights",
 ]
 
 _lib = None
@@ -172,5 +173,8 @@ def load() -> ctypes.CDLL:
     lib.bpp_ipa_batch_free.restype = None
     lib.bpp_ipa_batch_prove.argtypes = [vp, u8p, u8p, u8p, u8p, u8p, c.c_char_p, c.c_char_p]
     lib.bpp_ipa_batch_verify.argtypes = [vp, u8p, u8p, u8p, u8p, u8p, c.c_char_p, c.c_char_p]
+    lib.bpp_ipa_batch_verify_combined.argtypes = [vp, u8p, u8p, u8p, u8p, u8p, u8p, c.c_char_p, c.c_char_p]
+    lib.bpp_ipa_batch_gather_accept.argtypes = [vp, sz, c.c_char_p]
+    lib.bpp_ipa_batch_download_weights.argtypes = [vp, c.c_char_p]
     _lib = lib
     return lib

@@ -1387,17 +1387,27 @@ __global__ void __launch_bounds__(128) k_rlc_dyn_scalars(acp_layout lay, uint32_
     sc_mul(v, v, rho);
     sc_store(out + 8 * ((size_t)p * per + k), v);
 }
-// out[i] = sum_p rho_p * vstat_p[i] for the nstat shared generators (g, h, G[], H[]); block per generator
-__global__ void __launch_bounds__(128) k_rlc_stat_scalars(acp_layout lay, uint32_t nstat, uint32_t B, uint32_t rho_off,
+// Where the shared generators' scalars sit in a proof block: generator i of segment k (i < cnt[k]) at off[k] + i, the
+// segments in the order of the generators' points (the shuffle: one segment g, h, G[], H[] at lay.vg; the stand-alone
+// inner-product batch: vG, vH, and the Q coefficient at lay.cl).
+#define RLC_MAX_SEGS 3
+struct rlc_segs {
+    uint32_t off[RLC_MAX_SEGS], cnt[RLC_MAX_SEGS];
+};
+// out[i] = sum_p rho_p * vstat_p[i] for the shared generators of `sg`; block per generator
+__global__ void __launch_bounds__(128) k_rlc_stat_scalars(acp_layout lay, rlc_segs sg, uint32_t B, uint32_t rho_off,
                                                           const uint32_t *__restrict__ blk, uint32_t *__restrict__ out) {
     __shared__ __align__(16) uint32_t red[128][8];
     const uint32_t i = blockIdx.x;
+    uint32_t k = 0, j = i;
+    while (k + 1 < RLC_MAX_SEGS && j >= sg.cnt[k]) j -= sg.cnt[k++];
+    const uint32_t src = sg.off[k] + j;
     sc acc, rho, v, rr;
     sc_set0(acc);
     sc_const(rr, SC_R2);
     for (uint32_t p = threadIdx.x; p < B; p += 128) {
         sc_load(rho, ACP_PTR(blk, lay, p, rho_off));
-        sc_load(v, ACP_PTR(blk, lay, p, lay.vg + i));
+        sc_load(v, ACP_PTR(blk, lay, p, src));
         sc_mont(v, v, rho);      // rho * v / R; the factor R is restored once after the reduction
         sc_add(acc, acc, v);
     }

@@ -968,8 +968,7 @@ static int acp_put_challenges(bpp_acp_batch *b, uint32_t off, uint32_t per, size
 // caller passes NULL.  Soundness of the fused per-proof check and of the batch combination needs weights the prover
 // cannot predict; they are additionally bound to every byte of each proof through its transcript.
 #include <sys/random.h>
-static int acp_set_verifier_seed(bpp_acp_batch *b, const uint8_t *seed, uint8_t host_copy[32]) {
-    bpp_ctx *ctx = b->ctx;
+static int set_verifier_seed(bpp_ctx *ctx, uint32_t *d_vseed, const uint8_t *seed, uint8_t host_copy[32]) {
     if (seed) {
         memcpy(host_copy, seed, 32);
     } else {
@@ -983,8 +982,11 @@ static int acp_set_verifier_seed(bpp_acp_batch *b, const uint8_t *seed, uint8_t 
             got += (size_t)r;
         }
     }
-    CK(ctx, cudaMemcpyAsync(b->d_vseed, host_copy, 32, cudaMemcpyHostToDevice, ctx->stream));   // pageable: staged before return
+    CK(ctx, cudaMemcpyAsync(d_vseed, host_copy, 32, cudaMemcpyHostToDevice, ctx->stream));   // pageable: staged before return
     return BPP_OK;
+}
+static int acp_set_verifier_seed(bpp_acp_batch *b, const uint8_t *seed, uint8_t host_copy[32]) {
+    return set_verifier_seed(b->ctx, b->d_vseed, seed, host_copy);
 }
 // device transcripts: continue every proof's final verifier state into its weights, on the second side stream
 static int acp_fork_weights(bpp_acp_batch *b) {
@@ -1314,7 +1316,7 @@ static int acp_verify_rlc(bpp_acp_batch *b, uint32_t per, int check_t, bool *dec
     LAUNCH_CHECK(ctx);
     k_rlc_dyn_scalars<<<dim3((per + 127) / 128, B), 128, 0, s>>>(L, per, B, L.rho, b->d_blk, b->d_rlc_sc);
     LAUNCH_CHECK(ctx);
-    k_rlc_stat_scalars<<<nstat, 128, 0, s>>>(L, nstat, B, L.rho, b->d_blk, b->d_rlc_sc + 8 * (size_t)B * per);
+    k_rlc_stat_scalars<<<nstat, 128, 0, s>>>(L, rlc_segs{{L.vg, 0, 0}, {nstat, 0, 0}}, B, L.rho, b->d_blk, b->d_rlc_sc + 8 * (size_t)B * per);
     LAUNCH_CHECK(ctx);
     bpp_points view;
     view.niels = b->d_dyn;
@@ -1623,20 +1625,24 @@ extern "C" int bpp_ipa_fold_generators(bpp_ctx *ctx, const bpp_points *points, s
     return BPP_OK;
 }
 
-extern "C" int bpp_acp_batch_gather_accept(bpp_acp_batch *b, size_t per, uint8_t *accept_all) {
-    if (!b || !accept_all || per < b->B) return BPP_ERR_INVALID_ARG;
-    bpp_ctx *ctx = b->ctx;
+// Sharded batch verification: this rank's `count` accept bytes, zero-padded to `per`, all-gathered over the context's
+// communicator into accept_all (nranks x per, host); a single rank gets its own bytes.  Synchronises.
+static int gather_accept(bpp_ctx *ctx, const uint8_t *d_accept, uint32_t count, size_t per, uint8_t *accept_all) {
     CK(ctx, cudaSetDevice(ctx->device));
     const size_t nr = (size_t)ctx->comm_nranks;
     int rc;
     if ((rc = grow(ctx, &ctx->d_small, &ctx->cap_small, per * (nr + 1)))) return rc;
     uint8_t *mine = ctx->d_small, *all = ctx->d_small + per;
     CK(ctx, cudaMemsetAsync(mine, 0, per, ctx->stream));
-    CK(ctx, cudaMemcpyAsync(mine, b->d_accept, b->B, cudaMemcpyDeviceToDevice, ctx->stream));
+    CK(ctx, cudaMemcpyAsync(mine, d_accept, count, cudaMemcpyDeviceToDevice, ctx->stream));
     if ((rc = comm_all_gather(ctx, mine, all, per, ctx->stream))) return rc;
     CK(ctx, cudaMemcpyAsync(accept_all, all, per * nr, cudaMemcpyDeviceToHost, ctx->stream));
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     return BPP_OK;
+}
+extern "C" int bpp_acp_batch_gather_accept(bpp_acp_batch *b, size_t per, uint8_t *accept_all) {
+    if (!b || !accept_all || per < b->B) return BPP_ERR_INVALID_ARG;
+    return gather_accept(b->ctx, b->d_accept, b->B, per, accept_all);
 }
 
 // ---- one-call host forms (what a drop-in for create..blinding_values / verify binds) -------------------
@@ -1737,14 +1743,21 @@ extern "C" int bpp_transcript_challenge_bytes(uint8_t state[BPP_TRANSCRIPT_BYTES
 // ---- stand-alone inner-product argument, batched (bulletproofs 4.0.0 inner_product_proof.rs) -----------------------
 // The prover runs the scalar-fold rounds of the `fixed` mode (ipa_prove_rounds) over a block holding only the
 // inner-product fields (ipa_make_layout); the verifier evaluates dalek's verify as one MSM per proof: the 2 n + 1
-// generator terms through the window table, the 2 lg n + 1 proof points through k_dyn_window_sums.
+// generator terms through the window table, the 2 lg n + 1 proof points through k_dyn_window_sums.  The combined form
+// (bpp_ipa_batch_verify_combined) first runs one random-linear-combination MSM over the whole batch (ipa_verify_rlc).
 struct bpp_ipa_batch {
     bpp_ctx *ctx = nullptr;
     bpp_points *gens = nullptr;
     uint32_t g_off = 0, h_off = 0, q_off = 0, n = 0, lg = 0, B = 0, fb_splits = 1;
     acp_layout lay;
+    // d_dyn: B x (2 lg + 1) decompressed proof points; once the batch has run the combined check (ipa_rlc_alloc), followed
+    // by the Niels forms of G, H and the Q base, so that it holds all of the combined MSM's points
     uint32_t *d_blk = nullptr, *d_lrext = nullptr, *d_part = nullptr, *d_stat = nullptr, *d_wsum = nullptr, *d_bad = nullptr,
              *d_dyn = nullptr;
+    // combined verification: the verifier seed, the MSM's scalars (proof points, then generators), its compressed
+    // result and the fall-back flag
+    uint32_t *d_vseed = nullptr, *d_rlc_sc = nullptr, *d_rlc_flag = nullptr, *h_rlc_flag = nullptr;
+    uint8_t *d_rlc_out = nullptr;
     uint8_t *d_in = nullptr;       // staged inputs: a | b | G factors | H factors (B x n x 32 each) | q (B x 32) | P (B x 32)
     uint8_t *d_lr = nullptr;       // B x (2 lg + 1) x 32: L_j, R_j (prover: the first 2 lg per proof, pitch 2 lg), then P
     uint8_t *d_proofs = nullptr, *d_accept = nullptr;
@@ -1784,6 +1797,7 @@ static acp_layout ipa_make_layout(uint32_t n) {
     L.stab = take(2 * n);
     L.u = take(L.lg); L.uinv = take(L.lg); L.vd = take(2 * L.lg + 1);
     L.wq = take(1); L.cl = take(2); L.pa = take(1); L.pb = take(1);
+    L.rho0 = take(1); L.rho = take(1);
     L.stride = (o + 3) & ~3u;
     return L;
 }
@@ -1800,9 +1814,10 @@ extern "C" void bpp_ipa_batch_free(bpp_ipa_batch *b) {
     cudaSetDevice(b->ctx->device);
     cudaStreamSynchronize(b->ctx->stream);
     void *dev[] = {b->d_blk, b->d_lrext, b->d_part, b->d_stat, b->d_wsum, b->d_bad, b->d_dyn, b->d_in, b->d_lr, b->d_proofs,
-                   b->d_accept, b->d_tr};
+                   b->d_accept, b->d_tr, b->d_vseed, b->d_rlc_sc, b->d_rlc_flag, b->d_rlc_out};
     for (void *p : dev)
         if (p) cudaFree(p);
+    if (b->h_rlc_flag) cudaFreeHost(b->h_rlc_flag);
     for (auto &m : b->marks) cudaEventDestroy(m.second);
     delete b;
 }
@@ -1928,8 +1943,39 @@ extern "C" int bpp_ipa_batch_prove(bpp_ipa_batch *b, const uint8_t *q, const uin
     return BPP_OK;
 }
 
-extern "C" int bpp_ipa_batch_verify(bpp_ipa_batch *b, const uint8_t *q, const uint8_t *G_factors, const uint8_t *H_factors,
-                                    const uint8_t *P, const uint8_t *proofs, uint8_t *transcripts, uint8_t *accept) {
+// The combined check's buffers, on the batch's first combined verification (batches that only prove or only run the
+// per-proof verify never pay for them): d_dyn grows by the Niels forms of G, H and the Q base, copied from the
+// generators; the MSM's scalars, its result, the fall-back flag and the verifier seed.  d_rlc_sc is allocated last and
+// marks the set complete.
+static int ipa_rlc_alloc(bpp_ipa_batch *b) {
+    if (b->d_rlc_sc) return BPP_OK;
+    bpp_ctx *ctx = b->ctx;
+    const size_t npts = (size_t)b->B * (2 * b->lg + 1), n = b->n, nstat = 2 * n + 1;
+    const uint32_t *g = b->gens->niels;
+    uint32_t *dyn = nullptr;
+    CK(ctx, cudaMalloc((void **)&dyn, (npts + nstat) * 96));
+    CK(ctx, cudaFree(b->d_dyn));
+    b->d_dyn = dyn;
+    CK(ctx, cudaMemcpyAsync(dyn + 24 * npts, g + 24 * (size_t)b->g_off, n * 96, cudaMemcpyDeviceToDevice, ctx->stream));
+    CK(ctx, cudaMemcpyAsync(dyn + 24 * (npts + n), g + 24 * (size_t)b->h_off, n * 96, cudaMemcpyDeviceToDevice, ctx->stream));
+    CK(ctx, cudaMemcpyAsync(dyn + 24 * (npts + 2 * n), g + 24 * (size_t)b->q_off, 96, cudaMemcpyDeviceToDevice, ctx->stream));
+    if (!b->d_vseed) CK(ctx, cudaMalloc((void **)&b->d_vseed, 64));
+    if (!b->d_rlc_flag) CK(ctx, cudaMalloc((void **)&b->d_rlc_flag, 64));
+    if (!b->d_rlc_out) CK(ctx, cudaMalloc((void **)&b->d_rlc_out, 256));
+    if (!b->h_rlc_flag) CK(ctx, cudaMallocHost((void **)&b->h_rlc_flag, 64));
+    CK(ctx, cudaMalloc((void **)&b->d_rlc_sc, (npts + nstat) * 32));
+    return BPP_OK;
+}
+
+// Below this many proof points the per-proof path is cheaper than the buckets (the shuffle verifier's rule)
+#define IPA_RLC_MIN_POINTS 1024
+static bool ipa_rlc_pays(const bpp_ipa_batch *b) { return (size_t)b->B * (2 * b->lg + 1) >= IPA_RLC_MIN_POINTS; }
+
+// Verifier up to the per-proof scalars: argument checks, uploads, unpack, decompression, transcript replay, vprep, the
+// s table and k_ipa_vscal.  The proofs stay staged at b->d_in.  rlc: the combined check follows (its buffers are made
+// first, after the argument checks).
+static int ipa_verify_scalars(bpp_ipa_batch *b, const uint8_t *q, const uint8_t *G_factors, const uint8_t *H_factors,
+                              const uint8_t *P, const uint8_t *proofs, uint8_t *transcripts, uint8_t *accept, bool rlc) {
     if (!b || !P || !proofs || !transcripts || !accept) return BPP_ERR_INVALID_ARG;
     bpp_ctx *ctx = b->ctx;
     const size_t B = b->B, n = b->n, lg = b->lg, plen = bpp_ipa_proof_len(n), per = 2 * lg + 1;
@@ -1937,6 +1983,7 @@ extern "C" int bpp_ipa_batch_verify(bpp_ipa_batch *b, const uint8_t *q, const ui
     if ((rc = ipa_check_inputs(b, q, G_factors, H_factors, transcripts))) return rc;
     CK(ctx, cudaSetDevice(ctx->device));
     if (!b->gens->fb_table && (rc = bpp_points_precompute(ctx, b->gens, 8))) return rc;
+    if (rlc && (rc = ipa_rlc_alloc(b))) return rc;
     cudaStream_t s = ctx->stream;
     const acp_layout &L = b->lay;
     ipa_mark(b, "start");
@@ -1960,6 +2007,14 @@ extern "C" int bpp_ipa_batch_verify(bpp_ipa_batch *b, const uint8_t *q, const ui
     LAUNCH_CHECK(ctx);
     k_ipa_vscal<<<dim3((b->n + 1 + 127) / 128, b->B), 128, 0, s>>>(L, b->d_blk);
     LAUNCH_CHECK(ctx);
+    return BPP_OK;
+}
+// Every proof on its own: the generator terms through the window table, the proof points through k_dyn_window_sums.
+static int ipa_verify_per_proof(bpp_ipa_batch *b) {
+    bpp_ctx *ctx = b->ctx;
+    cudaStream_t s = ctx->stream;
+    const acp_layout &L = b->lay;
+    int rc;
     {
         fb_shape sh = acp_shape(1);
         acp_seg(sh, L.vG, 0, b->g_off, b->n);
@@ -1967,15 +2022,98 @@ extern "C" int bpp_ipa_batch_verify(bpp_ipa_batch *b, const uint8_t *q, const ui
         acp_seg(sh, L.cl, 0, b->q_off, 1);
         if ((rc = fb_launch(ctx, b->d_blk, L, b->B, *b->gens, sh, ipa_fb_plan(b, sh), b->d_stat, 1, s, b->d_part, nullptr))) return rc;
     }
-    k_dyn_window_sums<<<b->B, DYN_W, 0, s>>>(b->d_blk, L, b->d_dyn, (uint32_t)per, b->d_wsum);
+    k_dyn_window_sums<<<b->B, DYN_W, 0, s>>>(b->d_blk, L, b->d_dyn, 2 * b->lg + 1, b->d_wsum);
     LAUNCH_CHECK(ctx);
     k_ipa_accept<<<(b->B + 63) / 64, 64, 0, s>>>(b->B, b->d_wsum, b->d_stat, b->d_bad, b->d_accept);
     LAUNCH_CHECK(ctx);
     ipa_mark(b, "check");
-    CK(ctx, cudaMemcpyAsync(accept, b->d_accept, B, cudaMemcpyDeviceToHost, s));
-    CK(ctx, cudaMemcpyAsync(transcripts, b->d_tr, B * BPP_TRANSCRIPT_BYTES, cudaMemcpyDeviceToHost, s));
+    return BPP_OK;
+}
+// accept bytes and the transcripts as the replay left them (never touched by the weights) back to the caller
+static int ipa_verify_download(bpp_ipa_batch *b, uint8_t *transcripts, uint8_t *accept, const char *what) {
+    bpp_ctx *ctx = b->ctx;
+    cudaStream_t s = ctx->stream;
+    CK(ctx, cudaMemcpyAsync(accept, b->d_accept, b->B, cudaMemcpyDeviceToHost, s));
+    CK(ctx, cudaMemcpyAsync(transcripts, b->d_tr, (size_t)b->B * BPP_TRANSCRIPT_BYTES, cudaMemcpyDeviceToHost, s));
     ipa_mark(b, "download");
     CK(ctx, cudaStreamSynchronize(s));
-    ipa_marks_dump(b, "verify");
+    ipa_marks_dump(b, what);
     return BPP_OK;
+}
+
+extern "C" int bpp_ipa_batch_verify(bpp_ipa_batch *b, const uint8_t *q, const uint8_t *G_factors, const uint8_t *H_factors,
+                                    const uint8_t *P, const uint8_t *proofs, uint8_t *transcripts, uint8_t *accept) {
+    int rc;
+    if ((rc = ipa_verify_scalars(b, q, G_factors, H_factors, P, proofs, transcripts, accept, false))) return rc;
+    if ((rc = ipa_verify_per_proof(b))) return rc;
+    return ipa_verify_download(b, transcripts, accept, "verify");
+}
+
+// The batch as one MSM (the shuffle verifier's acp_verify_rlc over this layout): rho_p from a copy of each proof's
+// final transcript rekeyed with the verifier seed (k_ipa_weights; 0 for a proof already refused), then
+// sum_p rho_p (P_p + sum_k u_k^2 L_k + u_k^-2 R_k) + sum_i (sum_p rho_p vG_p,i) G_i + (.. vH ..) H_i + (.. cl ..) Q in one
+// Pippenger MSM over B (2 lg n + 1) proof points and the 2 n + 1 generators, whose scalars add up across proofs.  The
+// identity accepts every proof of nonzero weight; otherwise *decided = false and the caller checks every proof on its own.
+static int ipa_verify_rlc(bpp_ipa_batch *b, const uint8_t *verifier_seed, bool *decided) {
+    bpp_ctx *ctx = b->ctx;
+    const acp_layout &L = b->lay;
+    const uint32_t B = b->B, n = b->n, per = 2 * b->lg + 1, nstat = 2 * n + 1;
+    const size_t N = (size_t)B * per + nstat;
+    cudaStream_t s = ctx->stream;
+    *decided = false;
+    int rc;
+    uint8_t seed[32];
+    if ((rc = set_verifier_seed(ctx, b->d_vseed, verifier_seed, seed))) return rc;
+    TR_LAUNCH(k_ipa_weights, B, s, b->d_tr, b->d_in, b->d_lr, (const uint8_t *)b->d_vseed, L, B, b->d_blk);
+    LAUNCH_CHECK(ctx);
+    k_rlc_weights<<<(B + 127) / 128, 128, 0, s>>>(L, B, 0, b->d_bad, b->d_blk);
+    LAUNCH_CHECK(ctx);
+    k_rlc_dyn_scalars<<<dim3((per + 127) / 128, B), 128, 0, s>>>(L, per, B, L.rho, b->d_blk, b->d_rlc_sc);
+    LAUNCH_CHECK(ctx);
+    k_rlc_stat_scalars<<<nstat, 128, 0, s>>>(L, rlc_segs{{L.vG, L.vH, L.cl}, {n, n, 1}}, B, L.rho, b->d_blk,
+                                             b->d_rlc_sc + 8 * (size_t)B * per);
+    LAUNCH_CHECK(ctx);
+    ipa_mark(b, "rlc-scalars");
+    bpp_points view;
+    view.niels = b->d_dyn;
+    view.n = N;
+    // one window group, as acp_verify_rlc: the SM time of the MSM, not the latency of one call
+    rc = msm_enqueue(ctx, b->d_rlc_sc, &view, 0, N, b->d_rlc_out, 1, true, 1);
+    view.niels = nullptr;
+    if (rc) return rc;
+    ipa_mark(b, "rlc-msm");
+    k_rlc_accept<<<(B + 127) / 128, 128, 0, s>>>(b->d_rlc_out, L, B, L.rho, b->d_blk, b->d_accept, b->d_rlc_flag);
+    LAUNCH_CHECK(ctx);
+    CK(ctx, cudaMemcpyAsync(b->h_rlc_flag, b->d_rlc_flag, 4, cudaMemcpyDeviceToHost, s));
+    CK(ctx, cudaStreamSynchronize(s));
+    *decided = b->h_rlc_flag[0] == 0;
+    return BPP_OK;
+}
+
+extern "C" int bpp_ipa_batch_verify_combined(bpp_ipa_batch *b, const uint8_t *q, const uint8_t *G_factors, const uint8_t *H_factors,
+                                             const uint8_t *P, const uint8_t *proofs, const uint8_t *verifier_seed,
+                                             uint8_t *transcripts, uint8_t *accept) {
+    int rc;
+    const bool rlc = b && ipa_rlc_pays(b);
+    if ((rc = ipa_verify_scalars(b, q, G_factors, H_factors, P, proofs, transcripts, accept, rlc))) return rc;
+    bool decided = false;
+    if (rlc && (rc = ipa_verify_rlc(b, verifier_seed, &decided))) return rc;
+    if (!decided && (rc = ipa_verify_per_proof(b))) return rc;
+    return ipa_verify_download(b, transcripts, accept, "verify_combined");
+}
+
+// The weights rho_p as k_ipa_weights drew them in the batch's last combined check (count x 32, host)
+extern "C" int bpp_ipa_batch_download_weights(bpp_ipa_batch *b, uint8_t *rho) {
+    if (!b || !rho || !b->d_rlc_sc) return BPP_ERR_INVALID_ARG;
+    bpp_ctx *ctx = b->ctx;
+    CK(ctx, cudaSetDevice(ctx->device));
+    CK(ctx, cudaMemcpy2DAsync(rho, 32, b->d_blk + 8 * (size_t)b->lay.rho0, (size_t)b->lay.stride * 32, 32, b->B,
+                              cudaMemcpyDeviceToHost, ctx->stream));
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    return BPP_OK;
+}
+
+extern "C" int bpp_ipa_batch_gather_accept(bpp_ipa_batch *b, size_t per, uint8_t *accept_all) {
+    if (!b || !accept_all || per < b->B) return BPP_ERR_INVALID_ARG;
+    return gather_accept(b->ctx, b->d_accept, b->B, per, accept_all);
 }

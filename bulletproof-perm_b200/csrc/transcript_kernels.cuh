@@ -339,6 +339,33 @@ __global__ void __launch_bounds__(TR_THREADS) k_tr_weights(const uint64_t *__res
     }
 }
 
+// Batch weight of the stand-alone inner-product batch (bpp_ipa_batch_verify_combined), the construction of k_tr_weights:
+// a copy of proof p's final verifier state (k_ipa_vtranscript; `states` is only read, so the caller's transcript never
+// sees these appends) absorbs the proof's a || b and P - which dalek's verify does not absorb: without it two proofs of
+// equal bytes with P + D and P - D would get equal weights under a reused seed and cancel - then the verifier seed and
+// the proof's index, and draws "rho" (at lay.rho0).  lrp: k_ipa_unpack's B x (2 lg + 1) x 32, P last; proofs: the
+// uploaded proofs, a || b in their last 64 bytes.
+template <class T>
+__global__ void __launch_bounds__(TR_THREADS) k_ipa_weights(const uint64_t *__restrict__ states, const uint8_t *__restrict__ proofs,
+                                                            const uint8_t *__restrict__ lrp, const uint8_t *__restrict__ vseed,
+                                                            acp_layout lay, uint32_t B, uint32_t *__restrict__ blk) {
+    const uint32_t p = tr_index<T>();
+    if (p >= B) return;
+    // every address taken before the sponge: this form compiles without spills in both transcript forms
+    const uint32_t words = 2 * lay.lg + 2;
+    const uint8_t *ab = proofs + 32 * ((size_t)p * words + words - 2), *P = lrp + 32 * ((size_t)p * (words - 1) + words - 2);
+    uint32_t *dst = ACP_PTR(blk, lay, p, lay.rho0);
+    T t;
+    t.load(states + MERLIN_STATE_WORDS * (size_t)p);
+    t.append_message(MERLIN_LABEL("proof-tail"), ab, 64);
+    t.append_message(MERLIN_LABEL("P"), P, 32);
+    t.append_message(MERLIN_LABEL("verifier-seed"), vseed, 32);
+    t.append_u64(MERLIN_LABEL("proof-index"), p);
+    sc rho;
+    t.challenge_scalar(MERLIN_LABEL("rho"), rho);
+    if (t.lane == 0) sc_store(dst, rho);
+}
+
 // Scripted transcript for tests (one thread): script = sequence of records
 //   op (1 B: 0 = append_message, 1 = challenge_bytes) | label_len (1 B) | label | n (4 B LE) | msg (op 0 only)
 // starting from Transcript::new(first record's message); challenge outputs are concatenated into out.

@@ -110,6 +110,28 @@ class InnerProductBatch:
         _write_back(transcripts, st, acc.raw)
         return acc.raw
 
+    def verify_combined(self, transcripts: Sequence[Transcript], P: bytes, proofs: bytes, q: bytes = None,
+                        G_factors: bytes = None, H_factors: bytes = None, verifier_seed: bytes = None) -> bytes:
+        """The decisions and transcripts of `verify`, through one random-linear-combination MSM over the batch (every
+        proof on its own only when that combination is not the identity, or for batches of fewer than 1024 proof
+        points).  verifier_seed: 32 bytes of secret, fresh randomness; None = the library draws them from the OS."""
+        if verifier_seed is not None and len(verifier_seed) != 32:
+            raise ValueError("verifier_seed: 32 bytes or None")
+        st = _states(transcripts, self.count)
+        acc = ctypes.create_string_buffer(self.count)
+        self.be._check(self.be._lib.bpp_ipa_batch_verify_combined(self._h, q, G_factors, H_factors, P, proofs, verifier_seed,
+                                                                  st, acc))
+        _write_back(transcripts, st, acc.raw)
+        return acc.raw
+
+    def gather_accept(self, per: int) -> bytes:
+        """Sharded verification: all ranks' accept bytes of their last verify (nranks x per, rank r's at r * per),
+        through the library's NCCL communicator (Backend.comm_init); this rank's own bytes without one."""
+        nr, _ = self.be.comm_info()
+        out = ctypes.create_string_buffer(per * nr)
+        self.be._check(self.be._lib.bpp_ipa_batch_gather_accept(self._h, per, out))
+        return out.raw
+
     def free(self):
         if self._h and self.be._ctx:
             self.be._lib.bpp_ipa_batch_free(self._h)

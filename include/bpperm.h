@@ -402,6 +402,32 @@ int bpp_ipa_batch_prove(bpp_ipa_batch *b, const uint8_t *q, const uint8_t *G_fac
  * leaves them. */
 int bpp_ipa_batch_verify(bpp_ipa_batch *b, const uint8_t *q, const uint8_t *G_factors, const uint8_t *H_factors,
                          const uint8_t *P, const uint8_t *proofs, uint8_t *transcripts, uint8_t *accept);
+/* The same decisions, accept bytes and transcripts as bpp_ipa_batch_verify (and the same errors), reached through ONE
+ * random-linear-combination MSM over the whole batch: sum_p rho_p * (proof p's check) is a Pippenger MSM over the
+ * count x (2 lg n + 1) proof points and the 2n + 1 shared generators, whose scalars add up across proofs.  When it is
+ * the identity every proof is accepted; otherwise, or when count x (2 lg n + 1) < 1024 (too few points for the buckets
+ * to pay), every proof is checked on its own as bpp_ipa_batch_verify checks it.  A proof refused before the MSM (a or
+ * b >= l, an undecodable or all-zero point) has rho_p = 0 and is rejected.
+ * rho_p is the challenge scalar "rho" of a COPY of proof p's transcript as verify leaves it, continued with
+ * append_message("proof-tail", a || b), append_message("P", P_p), append_message("verifier-seed", seed) and
+ * append_u64("proof-index", p) (p counts from 0 within this batch) - the construction of bpp_acp_batch_verify's
+ * weights.  The caller's transcripts never see these appends.  P is bound because verify does not absorb it: two
+ * proofs of equal bytes with P + D and P - D would otherwise cancel under a reused seed.
+ * verifier_seed: 32 bytes of SECRET, FRESH randomness of the verifier, or NULL to have the library draw them from the
+ * operating system (getrandom).  A seed known to the prover before it fixes its proofs would still leave the weights
+ * bound to every proof byte, P and the index, but pass NULL or fresh randomness; a constant is for reproducible tests
+ * only. */
+int bpp_ipa_batch_verify_combined(bpp_ipa_batch *b, const uint8_t *q, const uint8_t *G_factors, const uint8_t *H_factors,
+                                  const uint8_t *P, const uint8_t *proofs, const uint8_t *verifier_seed,
+                                  uint8_t *transcripts, uint8_t *accept);
+/* Sharded verification: every rank verified its own slice of the proofs with this batch (verify or verify_combined);
+ * all ranks' accept bytes are all-gathered (NCCL, bpp_comm_init) into accept_all = nranks x per bytes, rank r's count
+ * bytes at r * per (per >= every rank's count; the rest is zero padding).  Without a communicator: this rank's bytes.
+ * Host buffer; synchronises.  As bpp_acp_batch_gather_accept. */
+int bpp_ipa_batch_gather_accept(bpp_ipa_batch *b, size_t per, uint8_t *accept_all);
+/* Audit and test hook: the weights rho_p (count x 32, as drawn, before refused proofs are zeroed) of the batch's last
+ * bpp_ipa_batch_verify_combined that ran the combined check.  BPP_ERR_INVALID_ARG when none has. */
+int bpp_ipa_batch_download_weights(bpp_ipa_batch *b, uint8_t *rho);
 
 /* ---- measurement helpers --------------------------------------------------------------------- */
 /* IMAD.WIDE.U32 peak microbenchmark: returns wide multiply-adds per second over all SMs. */

@@ -170,6 +170,33 @@ impl InnerProductBatch {
         }
         acc.into_iter().map(|a| if a == 1 { Ok(()) } else { Err(ProofError::VerificationError) }).collect()
     }
+    /// `verify`'s results and transcripts through one random-linear-combination MSM over the batch (every proof on its
+    /// own only when the combination is not the identity).  verifier_seed: 32 bytes of SECRET, FRESH randomness, or
+    /// None to have the library draw them from the OS.
+    pub fn verify_combined(&mut self, transcripts: &mut [GpuTranscript], q: Option<&[Scalar]>, g_factors: Option<&[Scalar]>,
+                           h_factors: Option<&[Scalar]>, p: &[CompressedRistretto], proofs: &[u8],
+                           verifier_seed: Option<&[u8; 32]>) -> Vec<Result<(), ProofError>> {
+        assert!(transcripts.len() == self.count && p.len() == self.count && proofs.len() == self.count * self.proof_len);
+        let mut st = Self::states(transcripts);
+        let mut acc = vec![0u8; self.count];
+        assert_eq!(unsafe { sys::bpp_ipa_batch_verify_combined(self.b, Self::opt(q), Self::opt(g_factors), Self::opt(h_factors),
+                                                               p.as_ptr() as *const u8, proofs.as_ptr(),
+                                                               verifier_seed.map_or(std::ptr::null(), |s| s.as_ptr()),
+                                                               st.as_mut_ptr(), acc.as_mut_ptr()) }, 0);
+        for ((t, s), a) in transcripts.iter_mut().zip(st.chunks_exact(sys::BPP_TRANSCRIPT_BYTES)).zip(&acc) {
+            if *a == 1 { t.state.copy_from_slice(s) }
+        }
+        acc.into_iter().map(|a| if a == 1 { Ok(()) } else { Err(ProofError::VerificationError) }).collect()
+    }
+    /// Sharded verification: every rank's accept bytes of its last verify (nranks x per, rank r's at r * per) through
+    /// the library's communicator; this rank's own bytes without one.
+    pub fn gather_accept(&mut self, per: usize) -> Vec<u8> {
+        let (mut nranks, mut rank) = (0, 0);
+        assert_eq!(with_ctx(|c| unsafe { sys::bpp_comm_info(c, &mut nranks, &mut rank) }), 0);
+        let mut out = vec![0u8; per * nranks as usize];
+        assert_eq!(unsafe { sys::bpp_ipa_batch_gather_accept(self.b, per, out.as_mut_ptr()) }, 0);
+        out
+    }
 }
 impl Drop for InnerProductBatch { fn drop(&mut self) { unsafe { sys::bpp_ipa_batch_free(self.b) } } }
 

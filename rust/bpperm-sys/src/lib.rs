@@ -153,4 +153,12 @@ extern "C" {
                                b_vec: *const u8, transcripts: *mut u8, proofs_out: *mut u8) -> c_int;
     pub fn bpp_ipa_batch_verify(b: *mut bpp_ipa_batch, q: *const u8, g_factors: *const u8, h_factors: *const u8, p: *const u8,
                                 proofs: *const u8, transcripts: *mut u8, accept: *mut u8) -> c_int;
+    /// verify's decisions through one random-linear-combination MSM; verifier_seed nullable (= from the OS)
+    pub fn bpp_ipa_batch_verify_combined(b: *mut bpp_ipa_batch, q: *const u8, g_factors: *const u8, h_factors: *const u8,
+                                         p: *const u8, proofs: *const u8, verifier_seed: *const u8, transcripts: *mut u8,
+                                         accept: *mut u8) -> c_int;
+    /// sharded verification: all ranks' accept bytes (nranks x per) through the library's communicator
+    pub fn bpp_ipa_batch_gather_accept(b: *mut bpp_ipa_batch, per: usize, accept_all: *mut u8) -> c_int;
+    /// audit / test hook: rho_p of the last combined check (count x 32)
+    pub fn bpp_ipa_batch_download_weights(b: *mut bpp_ipa_batch, rho: *mut u8) -> c_int;
 }

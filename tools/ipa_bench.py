@@ -2,7 +2,11 @@
 (1, 8192), beside the inner-product rounds of the `fixed` mode prover on the same padded shape (52, 4 and 4096 cards),
 taken from its BPP_ACP_TRACE=1 stage timeline.  prove / verify: host clock around the C calls, which end in a device
 synchronisation (host input checks, pageable uploads and downloads included), after a warm-up; stage_median_ms: the
-batch's own BPP_ACP_TRACE=1 timeline (device events) in separate runs.  Inputs seeded.  Writes one JSON file (argv[1]) with the card name and power limit beside the numbers."""
+batch's own BPP_ACP_TRACE=1 timeline (device events) in separate runs; verify_vs_combined: verify and verify_combined
+alternating, host clock, on the all-valid batch and on one with ~1 % corrupted proofs.  Inputs seeded.  Writes one JSON
+file (argv[1]) with the card name and power limit beside the numbers.
+--scaling OUT.json: verify_combined of 4096 proofs of n = 128 in total, sharded over the ranks of
+`python -m torch.distributed.run --nproc-per-node N` (strong scaling; see strong_scaling)."""
 import ctypes
 import json
 import os
@@ -95,6 +99,7 @@ def ipa_shape(be, count, n, rs):
 
     tp = timed(prove, REPS)
     tv = timed(verify, REPS)
+    combined = verify_pair(be, bt, count, n, P, proofs.raw, states)
     # stage timeline (device events) in a run of its own: the rounds alone, comparable with the `fixed` prover's stage
     os.environ["BPP_ACP_TRACE"] = "1"
     bt2 = Ipa.InnerProductBatch(be, pts, 0, n, 2 * n, n, count)
@@ -117,10 +122,119 @@ def ipa_shape(be, count, n, rs):
                 stages.setdefault(f"{what}: {name}", []).append(float(us))
     stage_ms = {k: float(np.median(v)) / 1e3 for k, v in stages.items()}
     row = {"count": count, "n": n, "proof_bytes": bt.proof_len, "prove": tp, "verify": tv,
-           "all_accepted": acc.raw == b"\x01" * count, "stage_median_ms": stage_ms}
+           "all_accepted": acc.raw == b"\x01" * count, "stage_median_ms": stage_ms, "verify_vs_combined": combined}
     bt.free()
     pts.free()
     return row
+
+
+def corrupt(proofs: bytes, count: int, plen: int, every: int = 97) -> (bytes, bytes):
+    """about 1 % of the proofs (every 97th, and the only one of a batch of one) with one bit of b flipped; the expected
+    accept bytes"""
+    bad, expect = bytearray(proofs), bytearray(b"\x01" * count)
+    for p in range(min(3, count - 1), count, every):
+        bad[(p + 1) * plen - 29] ^= 0x04
+        expect[p] = 0
+    return bytes(bad), bytes(expect)
+
+
+def verify_pair(be, bt, count, n, P, good, states):
+    """verify and verify_combined side by side, alternating, on the all-valid batch and on the batch with ~1 %
+    corrupted proofs (verifier seed from the OS, as a caller would run it)"""
+    lib = be._lib
+    st = ctypes.create_string_buffer(len(states))
+    acc = ctypes.create_string_buffer(count)
+    bad, expect = corrupt(good, count, bt.proof_len)
+    out = {"corrupted": expect.count(0)}
+    for key, proofs, want in (("all_valid", good, b"\x01" * count), ("corrupted_1pct", bad, expect)):
+        def one(fn):
+            def run():
+                ctypes.memmove(st, states, len(states))
+                if fn == "verify":
+                    be._check(lib.bpp_ipa_batch_verify(bt._h, None, None, None, P, proofs, st, acc))
+                else:
+                    be._check(lib.bpp_ipa_batch_verify_combined(bt._h, None, None, None, P, proofs, None, st, acc))
+                return acc.raw
+            return run
+        ts = {"verify": [], "verify_combined": []}
+        ok = True
+        for fn in ts:
+            ok = ok and one(fn)() == want   # warm-up and decisions
+        for _ in range(REPS):
+            for fn in ts:
+                run = one(fn)
+                t0 = time.perf_counter()
+                run()
+                ts[fn].append(time.perf_counter() - t0)
+        out[key] = {fn: {"median_ms": 1e3 * float(np.median(v)), "min_ms": 1e3 * min(v), "max_ms": 1e3 * max(v)}
+                    for fn, v in ts.items()}
+        out[key]["decisions_match_expected"] = ok
+        out[key]["combined_over_verify"] = out[key]["verify_combined"]["median_ms"] / out[key]["verify"]["median_ms"]
+    return out
+
+
+def strong_scaling(total=4096, n=128, reps=REPS):
+    """4096 proofs of n = 128 IN TOTAL sharded over the ranks (torch.distributed.run, one process per GPU; a plain run
+    is one rank), as bench.py's batch_verify: every rank proves and verifies its slice (verify_combined, seed from the
+    OS), the accept bytes are gathered over the library's NCCL communicator (InnerProductBatch.gather_accept).  Time
+    per step: host clock from a barrier to the gathered bytes on every rank, median over reps; rank 0 returns it."""
+    import torch
+    import torch.distributed as dist
+    world, rank = int(os.environ.get("WORLD_SIZE", "1")), int(os.environ.get("RANK", "0"))
+    Ipa, par = bpperm_b200.ipa, bpperm_b200.parallel
+    if world > 1:
+        torch.cuda.set_device(rank)
+        dist.init_process_group("gloo")
+    be = bpperm_b200.Backend(rank)
+    par.init_comm(be, world, rank, torch.device("cuda", rank))
+    rs = np.random.RandomState(7)
+    pts = be.points_from_uniform(rs.randint(0, 256, size=(2 * n + 1, 64), dtype=np.uint8).tobytes())
+    a, b = scalars(rs, total * n), scalars(rs, total * n)   # the same global set on every rank
+    off, cnt = par.shard_bounds(total, world, rank)
+    per = (total + world - 1) // world
+    A, Bv = a.reshape(total, n, 32)[off:off + cnt], b.reshape(total, n, 32)[off:off + cnt]
+    c = []
+    for p in range(cnt):
+        av = [int.from_bytes(A[p, i].tobytes(), "little") for i in range(n)]
+        bv = [int.from_bytes(Bv[p, i].tobytes(), "little") for i in range(n)]
+        c.append((sum(x * y for x, y in zip(av, bv)) % L).to_bytes(32, "little"))
+    P = be.msm_batch(b"".join(A[p].tobytes() + Bv[p].tobytes() + c[p] for p in range(cnt)), pts, 2 * n + 1, cnt)
+    bt = Ipa.InnerProductBatch(be, pts, 0, n, 2 * n, n, cnt)
+    states = Ipa.Transcript(b"ipa-bench").state * cnt
+    st = ctypes.create_string_buffer(len(states))
+    good = ctypes.create_string_buffer(bt.proof_len * cnt)
+    be._check(be._lib.bpp_ipa_batch_prove(bt._h, None, None, None, A.tobytes(), Bv.tobytes(), st, good))
+    # the corrupted proofs by global index: every 97th from 3
+    bad, expect = bytearray(good.raw), bytearray(b"\x01" * cnt)
+    for g in range(3, total, 97):
+        if off <= g < off + cnt:
+            bad[(g - off + 1) * bt.proof_len - 29] ^= 0x04
+            expect[g - off] = 0
+    acc = ctypes.create_string_buffer(cnt)
+    res = {}
+    for key, proofs in (("all_valid", good.raw), ("corrupted_1pct", bytes(bad))):
+        ts, gathered = [], b""
+        for i in range(reps + 1):
+            if world > 1:
+                dist.barrier()
+            t0 = time.perf_counter()
+            ctypes.memmove(st, states, len(states))
+            be._check(be._lib.bpp_ipa_batch_verify_combined(bt._h, None, None, None, P, proofs, None, st, acc))
+            gathered = bt.gather_accept(per)
+            if i:
+                ts.append(time.perf_counter() - t0)
+        mine = gathered[per * rank:per * rank + cnt]
+        res[key] = {"median_ms": 1e3 * float(np.median(ts)), "min_ms": 1e3 * min(ts), "max_ms": 1e3 * max(ts),
+                    "proofs_per_s": total / float(np.median(ts)),
+                    "decisions_match_expected": mine == (b"\x01" * cnt if key == "all_valid" else bytes(expect))}
+    bt.free()
+    pts.free()
+    be.close()
+    if world > 1:
+        dist.destroy_process_group()
+    if rank != 0:
+        return None
+    return {"n_gpus": world, "total": total, "n": n, "on_rank0": cnt, "reps": reps, "card": card(), **res}
 
 
 def fixed_rounds(be, count, npad, rs):
@@ -157,6 +271,14 @@ def fixed_rounds(be, count, npad, rs):
 
 
 def main():
+    if len(sys.argv) > 2 and sys.argv[1] == "--scaling":
+        # python -m torch.distributed.run --nproc-per-node N tools/ipa_bench.py --scaling OUT.json
+        row = strong_scaling()
+        if row is not None:
+            print(json.dumps(row), flush=True)
+            os.makedirs(os.path.dirname(sys.argv[2]) or ".", exist_ok=True)
+            json.dump(row, open(sys.argv[2], "w"), indent=1)
+        return
     be = bpperm_b200.Backend(0)
     rs = np.random.RandomState(2026)
     res = {"card": card(), "reps": REPS, "rows": []}
