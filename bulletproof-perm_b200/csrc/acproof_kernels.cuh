@@ -799,8 +799,8 @@ __global__ void __launch_bounds__(ACP_POW_THREADS) k_acp_pow(acp_layout lay, uin
     sc_load(nxt, ACP_PTR(blk, lay, p, which == 1 ? lay.z : lay.y));
     if (which == 2) sc_invert(nxt, nxt);
     sc_to_mont(nxt, nxt);
-    // the chain stores Montgomery-form values: one dependent multiplication per step; k_acp_pow_unmont converts
-    // the whole range afterwards with one thread per element
+    // the chain stores Montgomery-form values: one dependent multiplication per step; k_acp_vec1 converts y_n and
+    // y_n_inv afterwards (and uses their Montgomery forms), k_acp_pow_unmont z_q, with one thread per element
 #pragma unroll 1
     for (uint32_t i = 0; i < cnt; i++) {
         ret = nxt;
@@ -809,11 +809,11 @@ __global__ void __launch_bounds__(ACP_POW_THREADS) k_acp_pow(acp_layout lay, uin
         sc_store(dst + 8 * (size_t)i, ret);
     }
 }
-// y_n | y_n_inv | z_q are contiguous in the proof block: Montgomery form -> standard form, in place
+// z_q: Montgomery form -> standard form, in place
 __global__ void __launch_bounds__(128) k_acp_pow_unmont(acp_layout lay, uint32_t *__restrict__ blk) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x, p = blockIdx.y;
-    if (i >= 2 * lay.n + lay.Q) return;
-    uint32_t *ptr = ACP_PTR(blk, lay, p, lay.yn + i);
+    if (i >= lay.Q) return;
+    uint32_t *ptr = ACP_PTR(blk, lay, p, lay.zq + i);
     sc v;
     sc_load(v, ptr);
     sc_from_mont(v, v);
@@ -871,29 +871,45 @@ __global__ void __launch_bounds__(128) k_acp_csr_long(acp_csr W, const uint32_t 
     if (threadIdx.x == 0) sc_store(ACP_PTR(blk, lay, p, lay.zWL + r), tot);
 }
 
-// thread per (proof, i < n): l_in, l1, r0, r1, r3 (circuit_lib.rs:286,313-339)
+// thread per (proof, i < n): l_in (prover and verifier), l1, r0, r1, r3 (prover only; circuit_lib.rs:286,313-339).
+// MONT: y_n[i] and y_n_inv[i] arrive in Montgomery form from k_acp_pow and are written back in standard form here, so
+// that each product y^i v or y^-i v is one Montgomery multiplication; otherwise (k_pow_fill's standard powers) they are
+// taken to Montgomery form first.
+template <bool PROVER, bool MONT>
 __global__ void __launch_bounds__(128) k_acp_vec1(acp_layout lay, uint32_t *__restrict__ blk) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x, p = blockIdx.y;
     if (i >= lay.n) return;
-    sc yn, yi, zwl, zwr, zwo, al, ar, srv, lin, t;
-    sc_load(yn, ACP_PTR(blk, lay, p, lay.yn + i));
-    sc_load(yi, ACP_PTR(blk, lay, p, lay.yninv + i));
-    sc_load(zwl, ACP_PTR(blk, lay, p, lay.zWL + i));
+    sc yn, ynr, yir, zwr, lin, t;
+    sc_load(ynr, ACP_PTR(blk, lay, p, lay.yn + i));
+    sc_load(yir, ACP_PTR(blk, lay, p, lay.yninv + i));
+    if (MONT) {
+        sc_from_mont(yn, ynr);
+        sc_store(ACP_PTR(blk, lay, p, lay.yn + i), yn);
+        sc_from_mont(t, yir);
+        sc_store(ACP_PTR(blk, lay, p, lay.yninv + i), t);
+    } else {
+        yn = ynr;
+        if (PROVER) sc_to_mont(ynr, yn);
+        sc_to_mont(yir, yir);
+    }
     sc_load(zwr, ACP_PTR(blk, lay, p, lay.zWR + i));
+    sc_mont(lin, yir, zwr);
+    sc_store(ACP_PTR(blk, lay, p, lay.lin + i), lin);
+    if (!PROVER) return;
+    sc zwl, zwo, al, ar, srv;
+    sc_load(zwl, ACP_PTR(blk, lay, p, lay.zWL + i));
     sc_load(zwo, ACP_PTR(blk, lay, p, lay.zWO + i));
     sc_load(al, ACP_PTR(blk, lay, p, lay.aL + i));
     sc_load(ar, ACP_PTR(blk, lay, p, lay.aR + i));
     sc_load(srv, ACP_PTR(blk, lay, p, lay.sr + i));
-    sc_mul(lin, yi, zwr);
-    sc_store(ACP_PTR(blk, lay, p, lay.lin + i), lin);
     sc_add(t, al, lin);
     sc_store(ACP_PTR(blk, lay, p, lay.l1 + i), t);
     sc_sub(t, zwo, yn);
     sc_store(ACP_PTR(blk, lay, p, lay.r0 + i), t);
-    sc_mul(t, yn, ar);
+    sc_mont(t, ynr, ar);
     sc_add(t, t, zwl);
     sc_store(ACP_PTR(blk, lay, p, lay.r1 + i), t);
-    sc_mul(t, yn, srv);
+    sc_mont(t, ynr, srv);
     sc_store(ACP_PTR(blk, lay, p, lay.r3 + i), t);
 }
 
@@ -933,7 +949,7 @@ __global__ void __launch_bounds__(128) k_acp_dots(acp_layout lay, uint32_t first
 // block-per-dot form above launches 10 x B blocks of one multiplication per thread - at B = 4096 its time is block
 // dispatch, not arithmetic (261 us for 4.3 M multiplications) - and stays for small batches, where a single proof's
 // n = 8192 needs the blocks.
-__global__ void __launch_bounds__(320) k_acp_dots_warp(acp_layout lay, uint32_t first, uint32_t *__restrict__ blk) {
+__global__ void __launch_bounds__(320, 3) k_acp_dots_warp(acp_layout lay, uint32_t first, uint32_t *__restrict__ blk) {
     const uint32_t k = first + (threadIdx.x >> 5), p = blockIdx.x, lane = threadIdx.x & 31;
     uint32_t ua, vb, len = lay.n;
     switch (k) {
@@ -951,14 +967,27 @@ __global__ void __launch_bounds__(320) k_acp_dots_warp(acp_layout lay, uint32_t 
         default: ua = lay.zWV; vb = lay.gamma; len = lay.m; break;
     }
     const uint32_t *a = ACP_PTR(blk, lay, p, ua), *b = ACP_PTR(blk, lay, p, vb);
+    // a lane's products are summed as 512-bit integers and reduced once (sc_mont_reduce: up to 15 at a time), not one
+    // Montgomery reduction per product: 64 instead of 132 wide multiplies per element
     sc acc, x, y, pr, tot;
     sc_set0(acc);
+    uint32_t t[16], cnt = 0;
+#pragma unroll
+    for (int j = 0; j < 16; j++) t[j] = 0;
     for (uint32_t i = lane; i < len; i += 32) {
         sc_load(x, a + 8 * (size_t)i);
         sc_load(y, b + 8 * (size_t)i);
-        sc_mont(pr, x, y);
-        sc_add(acc, acc, pr);
+        sc_mac(t, x, y);
+        if (++cnt == 15) {
+            sc_mont_reduce(pr, t);
+            sc_add(acc, acc, pr);
+#pragma unroll
+            for (int j = 0; j < 16; j++) t[j] = 0;
+            cnt = 0;
+        }
     }
+    sc_mont_reduce(pr, t);
+    sc_add(acc, acc, pr);
     // the warps leave their integer sums in shared memory; the reductions mod l and out of Montgomery form (three
     // multiplications each) then run side by side in the first lanes of warp 0 instead of once per warp
     __shared__ uint32_t sums[10 * 9];
@@ -1021,17 +1050,23 @@ __global__ void __launch_bounds__(64) k_acp_tcoef(acp_layout lay, uint32_t B, in
 }
 
 // thread per (proof, i): l = l(x), r = r(x)  (poly.rs:67-76 with l0 = 0, r2 = 0)
-// The proof's x is taken to Montgomery form once per block (thread 0, shared memory): a product x * t is then ONE
-// Montgomery multiplication (x R * t / R) instead of the two of sc_mul - 6 instead of 12 per thread.
-__global__ void __launch_bounds__(128) k_acp_final(acp_layout lay, uint32_t *__restrict__ blk) {
-    __shared__ __align__(16) uint32_t sh_x[8];
+// x R, x^2 R, x^3 R are computed once per block (thread 0, shared memory).  Then l = x l1 + x^2 a_O + x^3 s_l and
+// r - r0 = x r1 + x^3 r3 are each a sum of products x^k R * v accumulated as a 512-bit integer and reduced once
+// (sc_mac, sc_mont_reduce): 5 products and 2 reductions per element instead of the 6 Montgomery multiplications of
+// Horner's rule.
+__global__ void __launch_bounds__(128, 10) k_acp_final(acp_layout lay, uint32_t *__restrict__ blk) {
+    __shared__ __align__(16) uint32_t sh_x[3 * 8];   // x R | x^2 R | x^3 R
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x, p = blockIdx.y;
     if (threadIdx.x == 0) {
-        sc x0, r2, xr;
+        sc x0, r2, xr, x2r;
         sc_load(x0, ACP_PTR(blk, lay, p, lay.x));
         sc_const(r2, SC_R2);
         sc_mont(xr, x0, r2);
         sc_store(sh_x, xr);
+        sc_mont(x2r, xr, xr);
+        sc_store(sh_x + 8, x2r);
+        sc_mont(x2r, x2r, xr);
+        sc_store(sh_x + 16, x2r);
     }
     __syncthreads();
     if (i >= lay.np) return;
@@ -1044,23 +1079,29 @@ __global__ void __launch_bounds__(128) k_acp_final(acp_layout lay, uint32_t *__r
         sc_store(ACP_PTR(blk, lay, p, lay.r + i), t);
         return;
     }
-    sc_load(x, sh_x);       // x R
+    sc x2, x3;
+    sc_load(x, sh_x);
+    sc_load(x2, sh_x + 8);
+    sc_load(x3, sh_x + 16);
+    uint32_t w[16];
+#pragma unroll
+    for (int j = 0; j < 16; j++) w[j] = 0;
     sc_load(a, ACP_PTR(blk, lay, p, lay.l1 + i));
     sc_load(b, ACP_PTR(blk, lay, p, lay.aO + i));
     sc_load(c, ACP_PTR(blk, lay, p, lay.sl + i));
-    sc_mont(t, x, c);
-    sc_add(t, t, b);
-    sc_mont(t, x, t);
-    sc_add(t, t, a);
-    sc_mont(t, x, t);
+    sc_mac(w, x, a);
+    sc_mac(w, x2, b);
+    sc_mac(w, x3, c);
+    sc_mont_reduce(t, w);
     sc_store(ACP_PTR(blk, lay, p, lay.l + i), t);
+#pragma unroll
+    for (int j = 0; j < 16; j++) w[j] = 0;
     sc_load(a, ACP_PTR(blk, lay, p, lay.r0 + i));
     sc_load(b, ACP_PTR(blk, lay, p, lay.r1 + i));
     sc_load(c, ACP_PTR(blk, lay, p, lay.r3 + i));
-    sc_mont(t, x, c);       // x*r3
-    sc_mont(t, x, t);       // x^2*r3 (+ r2 = 0)
-    sc_add(t, t, b);
-    sc_mont(t, x, t);
+    sc_mac(w, x, b);
+    sc_mac(w, x3, c);
+    sc_mont_reduce(t, w);
     sc_add(t, t, a);
     sc_store(ACP_PTR(blk, lay, p, lay.r + i), t);
 }
@@ -1376,15 +1417,23 @@ __global__ void k_rlc_weights(acp_layout lay, uint32_t B, int check_t, const uin
     if (!ok) sc_set0(r);
     sc_store(ACP_PTR(blk, lay, p, lay.rho), r);
 }
-// out[p * per + k] = rho_p * vd_p[k]
+// out[p * per + k] = rho_p * vd_p[k]; rho_p R is computed once per block (shared memory), so that each product is one
+// Montgomery multiplication instead of the two of sc_mul
 __global__ void __launch_bounds__(128) k_rlc_dyn_scalars(acp_layout lay, uint32_t per, uint32_t B, uint32_t rho_off,
                                                          const uint32_t *__restrict__ blk, uint32_t *__restrict__ out) {
+    __shared__ __align__(16) uint32_t sh_rho[8];
     const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x, p = blockIdx.y;
-    if (k >= per) return;
     sc rho, v;
-    sc_load(rho, ACP_PTR(blk, lay, p, rho_off));
+    if (threadIdx.x == 0) {
+        sc_load(rho, ACP_PTR(blk, lay, p, rho_off));
+        sc_to_mont(rho, rho);
+        sc_store(sh_rho, rho);
+    }
+    __syncthreads();
+    if (k >= per) return;
+    sc_load(rho, sh_rho);
     sc_load(v, ACP_PTR(blk, lay, p, lay.vd + k));
-    sc_mul(v, v, rho);
+    sc_mont(v, v, rho);
     sc_store(out + 8 * ((size_t)p * per + k), v);
 }
 // Where the shared generators' scalars sit in a proof block: generator i of segment k (i < cnt[k]) at off[k] + i, the

@@ -1010,10 +1010,12 @@ static void acp_host_weights(bpp_host::Transcript &t, const uint8_t *proof, uint
     t.challenge_wide("rho", out128 + 64);
 }
 
-static int acp_challenge_dependent_scalars(bpp_acp_batch *b) {
+// prover: also l1, r0, r1, r3 (k_acp_vec1); the verifier needs l_in only
+static int acp_challenge_dependent_scalars(bpp_acp_batch *b, bool prover) {
     bpp_ctx *ctx = b->ctx;
     const acp_layout &L = b->lay;
-    if (b->mode == 2) {   // standard powers y^i, y^-i (i < n'), z^(q+1)
+    const bool mont = b->mode != 2;   // k_acp_pow leaves y_n, y_n_inv in Montgomery form for k_acp_vec1
+    if (!mont) {   // standard powers y^i, y^-i (i < n'), z^(q+1)
         k_pow_table<<<(b->B + 63) / 64, 64, 0, ctx->stream>>>(L, b->B, b->d_blk);
         LAUNCH_CHECK(ctx);
         k_pow_fill<<<dim3((2 * L.np + L.Q + 127) / 128, b->B), 128, 0, ctx->stream>>>(L, b->d_blk);
@@ -1021,7 +1023,7 @@ static int acp_challenge_dependent_scalars(bpp_acp_batch *b) {
     } else {
         k_acp_pow<<<(b->B + 31) / 32, ACP_POW_THREADS, 0, ctx->stream>>>(L, b->B, b->d_blk);
         LAUNCH_CHECK(ctx);
-        k_acp_pow_unmont<<<dim3((2 * L.n + L.Q + 127) / 128, b->B), 128, 0, ctx->stream>>>(L, b->d_blk);
+        k_acp_pow_unmont<<<dim3((L.Q + 127) / 128, b->B), 128, 0, ctx->stream>>>(L, b->d_blk);
         LAUNCH_CHECK(ctx);
     }
     acp_csr W{b->cir->d_rowptr, b->cir->d_col, b->cir->d_kind, b->cir->d_coeff, b->cir->rows};
@@ -1031,7 +1033,11 @@ static int acp_challenge_dependent_scalars(bpp_acp_batch *b) {
         k_acp_csr_long<<<dim3(b->cir->n_long, b->B), 128, 0, ctx->stream>>>(W, b->cir->d_long, L, b->d_blk);
         LAUNCH_CHECK(ctx);
     }
-    k_acp_vec1<<<dim3((L.n + 127) / 128, b->B), 128, 0, ctx->stream>>>(L, b->d_blk);
+    const dim3 grid((L.n + 127) / 128, b->B);
+    if (prover && mont) k_acp_vec1<true, true><<<grid, 128, 0, ctx->stream>>>(L, b->d_blk);
+    else if (prover) k_acp_vec1<true, false><<<grid, 128, 0, ctx->stream>>>(L, b->d_blk);
+    else if (mont) k_acp_vec1<false, true><<<grid, 128, 0, ctx->stream>>>(L, b->d_blk);
+    else k_acp_vec1<false, false><<<grid, 128, 0, ctx->stream>>>(L, b->d_blk);
     LAUNCH_CHECK(ctx);
     return BPP_OK;
 }
@@ -1227,7 +1233,7 @@ extern "C" int bpp_acp_batch_prove(bpp_acp_batch *b) {
         if ((rc = acp_put_challenges(b, L.y, 2))) return rc;
     }
     acp_mark(b, "y,z");
-    if ((rc = acp_challenge_dependent_scalars(b))) return rc;
+    if ((rc = acp_challenge_dependent_scalars(b, true))) return rc;
     acp_mark(b, "scalars");
     acp_dots_launch(L, 0, 10, B, b->d_blk, s);
     LAUNCH_CHECK(ctx);
@@ -1424,7 +1430,7 @@ static int acp_verify_fixed(bpp_acp_batch *b, const uint8_t *verifier_seed) {
         LAUNCH_CHECK(ctx);
         if ((rc = acp_put_challenges(b, L.w, 2, w_off))) return rc;
     }
-    if ((rc = acp_challenge_dependent_scalars(b))) return rc;
+    if ((rc = acp_challenge_dependent_scalars(b, false))) return rc;
     acp_dots_launch(L, 9, 1, B, b->d_blk, s);   // sigma
     LAUNCH_CHECK(ctx);
     k_ipa_vprep<<<(B + 63) / 64, 64, 0, s>>>(L, B, m + 8, b->d_blk);
@@ -1522,7 +1528,7 @@ extern "C" int bpp_acp_batch_verify(bpp_acp_batch *b, const uint8_t *verifier_se
         if ((rc = acp_put_challenges(b, L.y, 5))) return rc;
     }
     acp_mark(b, "transcript");
-    if ((rc = acp_challenge_dependent_scalars(b))) return rc;
+    if ((rc = acp_challenge_dependent_scalars(b, false))) return rc;
     acp_dots_launch(L, 9, 2, B, b->d_blk, s);  // sigma, <l, r>
     LAUNCH_CHECK(ctx);
     acp_mark(b, "scalars");

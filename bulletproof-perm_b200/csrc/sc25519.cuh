@@ -121,10 +121,12 @@ SC_INLINE void sc_neg(sc &r, const sc &a) {
 // dependency (the classic per-limb m_i = t_i * n' loop is one chain of ~100 dependent steps).
 __device__ __constant__ const uint32_t SC_NP[8] = {0x12547e1bu, 0xd2b51da3u, 0xfdba84ffu, 0xb1a206f2u,
                                                    0xffa36beau, 0x14e75438u, 0x6fe91836u, 0x9db6c6f2u};
+// sc_mont_reduce(r, t) = t / 2^256 mod l for any t < l * 2^256 (the reduction half of sc_mont): (t + q*l) / 2^256 <
+// t / 2^256 + l < 2l, so one conditional subtraction makes it canonical.  A sum of up to 15 products of canonical
+// scalars stays below that bound, so sums of products can be accumulated as 512-bit integers (sc_mac) and reduced once.
 #pragma nv_diag_suppress 550   // `dummy` receives a limb whose carry-out is all that matters
-SC_INLINE void sc_mont(sc &r, const sc &a, const sc &b) {
-    uint32_t t[16], qf[8], u[12], np[8], dl[4];
-    mp_mul8<8>(t, a.v, b.v);
+SC_INLINE void sc_mont_reduce(sc &r, const uint32_t t[16]) {
+    uint32_t qf[8], u[12], np[8], dl[4];
 #pragma unroll
     for (int i = 0; i < 8; i++) np[i] = SC_NP[i];
     mp_mul8_lo(qf, t, np);            // q = t_lo * (-l^-1) mod 2^256: 36 products
@@ -173,6 +175,36 @@ SC_INLINE void sc_mont(sc &r, const sc &a, const sc &b) {
     sc_cond_sub_l(r, s8, 0);          // s < 2l < 2^254
 }
 #pragma nv_diag_default 550
+SC_INLINE void sc_mont(sc &r, const sc &a, const sc &b) {
+    uint32_t t[16];
+    mp_mul8<8>(t, a.v, b.v);
+    sc_mont_reduce(r, t);
+}
+// t += a * b as a 512-bit integer (64 wide multiply-adds and one 16-limb carry chain; no reduction)
+SC_INLINE void sc_mac(uint32_t t[16], const sc &a, const sc &b) {
+    uint32_t p[16];
+    mp_mul8<8>(p, a.v, b.v);
+    asm("add.cc.u32 %0, %0, %16;\n\t"
+        "addc.cc.u32 %1, %1, %17;\n\t"
+        "addc.cc.u32 %2, %2, %18;\n\t"
+        "addc.cc.u32 %3, %3, %19;\n\t"
+        "addc.cc.u32 %4, %4, %20;\n\t"
+        "addc.cc.u32 %5, %5, %21;\n\t"
+        "addc.cc.u32 %6, %6, %22;\n\t"
+        "addc.cc.u32 %7, %7, %23;\n\t"
+        "addc.cc.u32 %8, %8, %24;\n\t"
+        "addc.cc.u32 %9, %9, %25;\n\t"
+        "addc.cc.u32 %10, %10, %26;\n\t"
+        "addc.cc.u32 %11, %11, %27;\n\t"
+        "addc.cc.u32 %12, %12, %28;\n\t"
+        "addc.cc.u32 %13, %13, %29;\n\t"
+        "addc.cc.u32 %14, %14, %30;\n\t"
+        "addc.u32 %15, %15, %31;"
+        : "+&r"(t[0]), "+&r"(t[1]), "+&r"(t[2]), "+&r"(t[3]), "+&r"(t[4]), "+&r"(t[5]), "+&r"(t[6]), "+&r"(t[7]),
+          "+&r"(t[8]), "+&r"(t[9]), "+&r"(t[10]), "+&r"(t[11]), "+&r"(t[12]), "+&r"(t[13]), "+&r"(t[14]), "+&r"(t[15])
+        : "r"(p[0]), "r"(p[1]), "r"(p[2]), "r"(p[3]), "r"(p[4]), "r"(p[5]), "r"(p[6]), "r"(p[7]),
+          "r"(p[8]), "r"(p[9]), "r"(p[10]), "r"(p[11]), "r"(p[12]), "r"(p[13]), "r"(p[14]), "r"(p[15]));
+}
 
 SC_INLINE void sc_to_mont(sc &r, const sc &a) {
     sc k;
