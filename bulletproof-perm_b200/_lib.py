@@ -17,7 +17,7 @@ SYMBOLS = [
     "bpp_init", "bpp_free", "bpp_set_stream", "bpp_synchronize", "bpp_strerror", "bpp_last_error",
     "bpp_launch_count", "bpp_device_info", "bpp_points_upload", "bpp_points_from_uniform", "bpp_points_compress", "bpp_points_free", "bpp_points_len",
     "bpp_comm_unique_id", "bpp_comm_init", "bpp_comm_free", "bpp_comm_info", "bpp_comm_all_gather_dev", "bpp_msm_sharded_dev", "bpp_msm_sharded_submit_dev", "bpp_msm_sharded_wait", "bpp_acp_batch_gather_accept",
-    "bpp_msm_vartime", "bpp_msm_vartime_host", "bpp_points_precompute", "bpp_msm_vartime_batch", "bpp_msm_vartime_batch_dev", "bpp_msm_multi", "bpp_msm_multi_indexed", "bpp_msm_multi_dev", "bpp_msm_multi_indexed_dev", "bpp_msm_vartime_dev", "bpp_msm_partial_dev", "bpp_msm_submit_dev", "bpp_msm_submit_partial_dev", "bpp_msm_wait", "bpp_msm_wait_previous",
+    "bpp_msm_vartime", "bpp_msm_vartime_host", "bpp_points_precompute", "bpp_msm_vartime_batch", "bpp_msm_vartime_batch_dev", "bpp_msm_multi", "bpp_msm_multi_indexed", "bpp_msm_multi_dev", "bpp_msm_multi_indexed_dev", "bpp_msm_mixed", "bpp_msm_mixed_dev", "bpp_msm_vartime_dev", "bpp_msm_partial_dev", "bpp_msm_submit_dev", "bpp_msm_submit_partial_dev", "bpp_msm_wait", "bpp_msm_wait_previous",
     "bpp_points_sum_compress_dev", "bpp_set_window_bits", "bpp_set_msm_groups", "bpp_set_msm_partition", "bpp_set_msm_tile", "bpp_set_msm_trace", "bpp_msm_trace_dump", "bpp_bench_imad_peak", "bpp_device_clock_khz", "bpp_bench_pipe_probe", "bpp_set_profiling",
     "bpp_last_phase_ms", "bpp_last_op_counts", "bpp_test_op",
     "bpp_inner_product", "bpp_hadamard_V", "bpp_vm_mult", "bpp_mv_mult", "bpp_exp_iter", "bpp_scalar_powers",
@@ -91,6 +91,8 @@ def load() -> ctypes.CDLL:
     lib.bpp_msm_multi_indexed.argtypes = [vp, sz, u32p, u8p, vp, u32p, c.c_char_p]
     lib.bpp_msm_multi_dev.argtypes = [vp, sz, u32p, vp, vp, vp, vp]
     lib.bpp_msm_multi_indexed_dev.argtypes = [vp, sz, u32p, vp, vp, vp, vp]
+    lib.bpp_msm_mixed.argtypes = [vp, sz, vp, sz, sz, u8p, u32p, u8p, u8p, c.c_char_p, c.c_char_p]
+    lib.bpp_msm_mixed_dev.argtypes = [vp, sz, vp, sz, sz, vp, u32p, vp, vp, vp, vp]
     lib.bpp_msm_vartime_dev.argtypes = [vp, vp, vp, sz, sz, vp]
     lib.bpp_msm_partial_dev.argtypes = [vp, vp, vp, sz, sz, vp]
     lib.bpp_msm_submit_dev.argtypes = [vp, vp, vp, sz, sz, vp]

@@ -262,6 +262,29 @@ class Backend:
         self._check(self._lib.bpp_msm_multi_indexed_dev(self._ctx, count, arr, ctypes.c_void_p(d_scalars), points._h,
                                                         ctypes.c_void_p(d_index), ctypes.c_void_p(d_out32)))
 
+    # -- mixed MSMs (bpp_msm_mixed*): a static part over points[off:off+n_static] plus the next sizes[j] caller terms ----
+    def msm_mixed(self, static_scalars: bytes, points: Points, n_static: int, dyn_scalars: bytes, dyn_points_enc: bytes, sizes,
+                  off: int = 0):
+        """`len(sizes)` MSMs, MSM j = sum_i static_scalars[j][i] points[off + i] + its sizes[j] dynamic terms (T x 32
+        scalars, T x 32 encodings) -> (encodings, ok flags).  An undecodable dynamic point fails only its own MSM (ok False,
+        32 zero bytes)."""
+        arr, count, T = self._sizes(sizes)
+        if len(static_scalars) != 32 * n_static * count:
+            raise ValueError("static scalars: len(sizes) x n_static x 32 bytes")
+        if len(dyn_scalars) != 32 * T or len(dyn_points_enc) != 32 * T:
+            raise ValueError("dynamic scalars and points: sum(sizes) x 32 bytes each")
+        out, ok = ctypes.create_string_buffer(32 * count), ctypes.create_string_buffer(count)
+        self._check(self._lib.bpp_msm_mixed(self._ctx, count, points._h, off, n_static, bytes(static_scalars), arr,
+                                            bytes(dyn_scalars), bytes(dyn_points_enc), out, ok))
+        return [out.raw[32 * j:32 * j + 32] for j in range(count)], [b != 0 for b in ok.raw]
+
+    def msm_mixed_dev(self, points: Points, n_static: int, d_static_scalars: int, sizes, d_dyn_scalars: int, d_dyn_points_enc: int,
+                      d_out32: int, d_ok: int, off: int = 0):
+        arr, count, _ = self._sizes(sizes)
+        self._check(self._lib.bpp_msm_mixed_dev(self._ctx, count, points._h, off, n_static, ctypes.c_void_p(d_static_scalars), arr,
+                                                ctypes.c_void_p(d_dyn_scalars), ctypes.c_void_p(d_dyn_points_enc),
+                                                ctypes.c_void_p(d_out32), ctypes.c_void_p(d_ok)))
+
     # device-pointer forms (pointers are ints, e.g. torch.Tensor.data_ptr())
     def msm_dev(self, d_scalars: int, points: Points, off: int, n: int, d_out: int):
         self._check(self._lib.bpp_msm_vartime_dev(self._ctx, ctypes.c_void_p(d_scalars), points._h, off, n,

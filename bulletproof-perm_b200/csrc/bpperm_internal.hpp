@@ -136,4 +136,10 @@ int msm_wait_pending(bpp_ctx *ctx, bool keep_latest = false);
 // call; bpp_set_msm_groups / bpp_set_msm_partition override it)
 int msm_enqueue(bpp_ctx *ctx, const uint32_t *d_scalars, const bpp_points *pts, size_t off, size_t n, uint8_t *d_out,
                 int do_compress, bool join = true, int groups = 0);
+// defined in capi_acproof.cu: bpp_msm_vartime_batch's table-gather MSM (`count` MSMs over pts[off, off + n), count x n
+// scalars at d_sc) up to the extended sums, count x 128 B at d_ext.  d_part: msm_table_part_bytes of split partials.
+// madd / add: its operation counts.  The window table must exist.  Stream-ordered on ctx->stream.
+size_t msm_table_part_bytes(const bpp_ctx *ctx, const bpp_points *P, size_t n, size_t count);
+int msm_table_ext(bpp_ctx *ctx, const uint32_t *d_sc, const bpp_points *P, size_t off, size_t n, size_t count, uint32_t *d_ext,
+                  uint32_t *d_part, uint64_t *madd, uint64_t *add);
 

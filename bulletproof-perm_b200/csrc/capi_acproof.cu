@@ -367,9 +367,9 @@ static fb_plan fb_choose(const bpp_ctx *ctx, uint64_t outputs, uint32_t terms, i
 static fb_plan msm_table_plan(const bpp_ctx *ctx, const bpp_points *P, size_t n, size_t count) {
     return fb_choose(ctx, count, (uint32_t)n, P->fb_Wn, false, 256);
 }
-// d_sc: count x n scalars; d_out32: count x 32.  Stream-ordered, no synchronisation.
-static int msm_table_run(bpp_ctx *ctx, const uint32_t *d_sc, const bpp_points *P, size_t off, size_t n, size_t count, uint8_t *d_out32,
-                         uint32_t *d_ext, uint32_t *d_part, const fb_plan &pl) {
+// d_sc: count x n scalars; d_ext: count x 128 B extended sums.  Stream-ordered, no synchronisation.
+static int msm_table_sums(bpp_ctx *ctx, const uint32_t *d_sc, const bpp_points *P, size_t off, size_t n, size_t count,
+                          uint32_t *d_ext, uint32_t *d_part, const fb_plan &pl) {
     acp_layout lay;
     memset(&lay, 0, sizeof(lay));
     lay.stride = (uint32_t)n;          // one "proof block" per MSM: its n scalars
@@ -391,9 +391,30 @@ static int msm_table_run(bpp_ctx *ctx, const uint32_t *d_sc, const bpp_points *P
             LAUNCH_CHECK(ctx);
         }
     }
-    k_compress_strided<<<(unsigned)((count + 127) / 128), 128, 0, st>>>(d_ext, 1, 0, 1, (uint32_t)count, d_out32);
+    return BPP_OK;
+}
+// the same, then d_out32: count x 32 compressed results
+static int msm_table_run(bpp_ctx *ctx, const uint32_t *d_sc, const bpp_points *P, size_t off, size_t n, size_t count, uint8_t *d_out32,
+                         uint32_t *d_ext, uint32_t *d_part, const fb_plan &pl) {
+    int rc = msm_table_sums(ctx, d_sc, P, off, n, count, d_ext, d_part, pl);
+    if (rc) return rc;
+    k_compress_strided<<<(unsigned)((count + 127) / 128), 128, 0, ctx->stream>>>(d_ext, 1, 0, 1, (uint32_t)count, d_out32);
     LAUNCH_CHECK(ctx);
     return BPP_OK;
+}
+// bpp_msm_mixed*: bpp_msm_vartime_batch's launches up to the extended sums.  The table must exist.
+size_t msm_table_part_bytes(const bpp_ctx *ctx, const bpp_points *P, size_t n, size_t count) {
+    const fb_plan pl = msm_table_plan(ctx, P, n, count);
+    return pl.splits > 1 ? count * pl.splits * 128 : 0;
+}
+int msm_table_ext(bpp_ctx *ctx, const uint32_t *d_sc, const bpp_points *P, size_t off, size_t n, size_t count, uint32_t *d_ext,
+                  uint32_t *d_part, uint64_t *madd, uint64_t *add) {
+    const fb_plan pl = msm_table_plan(ctx, P, n, count);
+    // every digit taken as non-zero, as mm_make_plan counts; the adds are the warp's five shuffle steps (31 adds) or the
+    // block tree (127) per split, and k_fb_sum_splits
+    *madd = (uint64_t)count * n * P->fb_Wn;
+    *add = (uint64_t)count * (pl.form == FB_WARP ? 31 : 127ull * pl.splits + (pl.splits > 1 ? pl.splits + 31 : 0));
+    return msm_table_sums(ctx, d_sc, P, off, n, count, d_ext, d_part, pl);
 }
 extern "C" int bpp_msm_vartime_batch_dev(bpp_ctx *ctx, const void *d_scalars, size_t count, bpp_points *points, size_t off, size_t n,
                                          void *d_out32) {

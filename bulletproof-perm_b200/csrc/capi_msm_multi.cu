@@ -1,5 +1,6 @@
 // capi_msm_multi.cu - C ABI of the batched variable-base MSM (bpp_msm_multi*, include/bpperm.h): `count` independent
-// vartime_multiscalar_mul calls with ragged sizes, each over its own points, in a few launches on the context's stream.
+// vartime_multiscalar_mul calls with ragged sizes, each over its own points, in a few launches on the context's stream;
+// and its mixed form (bpp_msm_mixed*), which adds a static part over a tabled point set to every MSM.
 #include "bpperm_internal.hpp"
 #include "msm_multi_kernels.cuh"
 
@@ -88,9 +89,11 @@ size_t mm_bytes(const mm_plan &pl, size_t count, bool enc) {
 }
 
 // Enqueues a call whose plan mm_make_plan made; the arena holds mm_bytes() from byte `base` on.  enc: the T x 32
-// encodings (device) or NULL; then index (T, device) selects from `points`.
+// encodings (device) or NULL; then index (T, device) selects from `points`.  st_ext (bpp_msm_mixed*): count x 128 B
+// extended points, MSM j's static part, added by the finish kernel (k_mm_finish_mixed instead of k_mm_finish).
 int mm_run(bpp_ctx *ctx, const mm_plan &pl, size_t count, const uint32_t *d_scalars, const uint8_t *d_enc,
-           const bpp_points *points, const uint32_t *d_index, uint8_t *d_out32, uint8_t *d_ok, size_t base) {
+           const bpp_points *points, const uint32_t *d_index, uint8_t *d_out32, uint8_t *d_ok, size_t base,
+           const uint32_t *d_st_ext = nullptr) {
     const size_t niels_b = d_enc ? al256(pl.T * 96) : 0;
     uint8_t *d = ctx->d_multi + base;
     uint32_t *d_niels = reinterpret_cast<uint32_t *>(d);
@@ -123,8 +126,12 @@ int mm_run(bpp_ctx *ctx, const mm_plan &pl, size_t count, const uint32_t *d_scal
                                                                 d_wsum);
         LAUNCH_CHECK(ctx);
     }
-    k_mm_finish<<<(unsigned)((count + MM_THREADS_FINISH - 1) / MM_THREADS_FINISH), MM_THREADS_FINISH, 0, s>>>(
-        d_msms, (uint32_t)count, d_wsum, d_enc ? d_bad : nullptr, d_out32, d_ok);
+    const unsigned fin = (unsigned)((count + MM_THREADS_FINISH - 1) / MM_THREADS_FINISH);
+    if (d_st_ext)
+        k_mm_finish_mixed<<<fin, MM_THREADS_FINISH, 0, s>>>(d_msms, (uint32_t)count, d_wsum, d_st_ext, d_enc ? d_bad : nullptr,
+                                                            d_out32, d_ok);
+    else
+        k_mm_finish<<<fin, MM_THREADS_FINISH, 0, s>>>(d_msms, (uint32_t)count, d_wsum, d_enc ? d_bad : nullptr, d_out32, d_ok);
     LAUNCH_CHECK(ctx);
     ctx->n_madd = pl.madd;
     ctx->n_add = pl.add;
@@ -143,6 +150,49 @@ int mm_check_common(bpp_ctx *ctx, size_t count, const uint32_t *sizes, uint64_t 
 int mm_check_scalars(const uint8_t *scalars, uint64_t T) {
     for (uint64_t i = 0; i < T; i++)
         if (scalars[32 * i + 31] & 0x80) return BPP_ERR_SCALAR_RANGE;
+    return BPP_OK;
+}
+
+// ---- bpp_msm_mixed*: a static part over a tabled sub-range plus a ragged dynamic part, per MSM ----------------
+// The static part is bpp_msm_vartime_batch's table-gather launches, stopped at the extended sums (count x 128 B); the
+// dynamic part is mm_run's decode and window-sum kernels; k_mm_finish_mixed adds the two per MSM and compresses.
+
+// what the host sees, both forms
+int mx_check(bpp_ctx *ctx, size_t count, const bpp_points *points, size_t off, size_t n_static, const uint32_t *sizes, uint64_t &T) {
+    int rc = mm_check_common(ctx, count, sizes, T);
+    if (rc) return rc;
+    if (!points || n_static == 0 || n_static >= (1ull << 31) || (uint64_t)count * n_static >= (1ull << 31)) return BPP_ERR_INVALID_ARG;
+    if (off > points->n || n_static > points->n - off) return BPP_ERR_LENGTH_MISMATCH;
+    return BPP_OK;
+}
+
+// The arena from byte `own` on: the static extended points | their split partials | mm_run's regions.
+struct mx_layout {
+    size_t ext_b = 0, part_b = 0, mm_b = 0;
+    size_t total(size_t own) const { return own + ext_b + part_b + mm_b; }
+};
+int mx_prepare(bpp_ctx *ctx, size_t count, bpp_points *points, size_t n_static, const uint32_t *sizes, mm_plan &pl, mx_layout &ly) {
+    int rc;
+    CK(ctx, cudaSetDevice(ctx->device));
+    if (!points->fb_table && (rc = bpp_points_precompute(ctx, points, 8))) return rc;
+    if ((rc = mm_make_plan(ctx, count, sizes, pl))) return rc;
+    ly.ext_b = al256(count * 128);
+    ly.part_b = al256(msm_table_part_bytes(ctx, points, n_static, count));
+    ly.mm_b = mm_bytes(pl, count, true);
+    return BPP_OK;
+}
+// Enqueues the call; the arena holds ly.total(own) bytes.  d_st_sc: count x n_static scalars with bit 255 clear.
+int mx_run(bpp_ctx *ctx, size_t count, const bpp_points *points, size_t off, size_t n_static, const uint32_t *d_st_sc,
+           const mm_plan &pl, const mx_layout &ly, const uint32_t *d_dyn_sc, const uint8_t *d_enc, uint8_t *d_out32, uint8_t *d_ok,
+           size_t own) {
+    uint32_t *d_ext = reinterpret_cast<uint32_t *>(ctx->d_multi + own);
+    uint32_t *d_part = reinterpret_cast<uint32_t *>(ctx->d_multi + own + ly.ext_b);
+    uint64_t t_madd = 0, t_add = 0;
+    int rc = msm_table_ext(ctx, d_st_sc, points, off, n_static, count, d_ext, d_part, &t_madd, &t_add);
+    if (rc) return rc;
+    if ((rc = mm_run(ctx, pl, count, d_dyn_sc, d_enc, nullptr, nullptr, d_out32, d_ok, own + ly.ext_b + ly.part_b, d_ext))) return rc;
+    ctx->n_madd += t_madd;
+    ctx->n_add += t_add + count;   // and the finish kernel's static + dynamic add
     return BPP_OK;
 }
 
@@ -223,6 +273,58 @@ extern "C" int bpp_msm_multi_indexed(bpp_ctx *ctx, size_t count, const uint32_t 
     }
     if ((rc = mm_run(ctx, pl, count, (const uint32_t *)d_sc, nullptr, points, (const uint32_t *)d_ix, d_out, nullptr, own))) return rc;
     CK(ctx, cudaMemcpyAsync(out32, d_out, count * 32, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    return BPP_OK;
+}
+
+extern "C" int bpp_msm_mixed_dev(bpp_ctx *ctx, size_t count, bpp_points *points, size_t off, size_t n_static,
+                                 const void *d_static_scalars, const uint32_t *sizes, const void *d_dyn_scalars,
+                                 const void *d_dyn_points_enc, void *d_out32, void *d_ok) {
+    uint64_t T = 0;
+    if (!d_static_scalars || !d_dyn_scalars || !d_dyn_points_enc || !d_out32 || !d_ok) return BPP_ERR_INVALID_ARG;
+    int rc = mx_check(ctx, count, points, off, n_static, sizes, T);
+    if (rc) return rc;
+    mm_plan pl;
+    mx_layout ly;
+    if ((rc = mx_prepare(ctx, count, points, n_static, sizes, pl, ly))) return rc;
+    // arena: the static scalars with bit 255 cleared, then mx_run's regions
+    const uint64_t n_sc = (uint64_t)count * n_static;
+    const size_t own = al256(n_sc * 32);
+    if ((rc = grow(ctx, &ctx->d_multi, &ctx->cap_multi, ly.total(own)))) return rc;
+    k_mm_scalars_low255<<<(unsigned)((2 * n_sc + 127) / 128), 128, 0, ctx->stream>>>((const uint4 *)d_static_scalars, n_sc,
+                                                                                    (uint4 *)ctx->d_multi);
+    LAUNCH_CHECK(ctx);
+    return mx_run(ctx, count, points, off, n_static, (const uint32_t *)ctx->d_multi, pl, ly, (const uint32_t *)d_dyn_scalars,
+                  (const uint8_t *)d_dyn_points_enc, (uint8_t *)d_out32, (uint8_t *)d_ok, own);
+}
+
+extern "C" int bpp_msm_mixed(bpp_ctx *ctx, size_t count, bpp_points *points, size_t off, size_t n_static,
+                             const uint8_t *static_scalars, const uint32_t *sizes, const uint8_t *dyn_scalars,
+                             const uint8_t *dyn_points_enc, uint8_t *out32, uint8_t *ok) {
+    uint64_t T = 0;
+    if (!static_scalars || !dyn_scalars || !dyn_points_enc || !out32 || !ok) return BPP_ERR_INVALID_ARG;
+    int rc = mx_check(ctx, count, points, off, n_static, sizes, T);
+    if (rc) return rc;
+    const uint64_t n_sc = (uint64_t)count * n_static;
+    if ((rc = mm_check_scalars(static_scalars, n_sc)) || (rc = mm_check_scalars(dyn_scalars, T))) return rc;
+    mm_plan pl;
+    mx_layout ly;
+    if ((rc = mx_prepare(ctx, count, points, n_static, sizes, pl, ly))) return rc;
+    // arena: static scalars | dynamic scalars | encodings | results | ok bytes, then mx_run's regions
+    const size_t st_b = al256(n_sc * 32), sc_b = al256(T * 32), out_b = al256(count * 32), ok_b = al256(count),
+                 own = st_b + 2 * sc_b + out_b + ok_b;
+    if ((rc = grow(ctx, &ctx->d_multi, &ctx->cap_multi, ly.total(own)))) return rc;
+    uint8_t *d_st = ctx->d_multi, *d_sc = d_st + st_b, *d_enc = d_sc + sc_b, *d_out = d_enc + sc_b, *d_ok = d_out + out_b;
+    CK(ctx, cudaMemcpyAsync(d_st, static_scalars, n_sc * 32, cudaMemcpyHostToDevice, ctx->stream));
+    if (T) {
+        CK(ctx, cudaMemcpyAsync(d_sc, dyn_scalars, T * 32, cudaMemcpyHostToDevice, ctx->stream));
+        CK(ctx, cudaMemcpyAsync(d_enc, dyn_points_enc, T * 32, cudaMemcpyHostToDevice, ctx->stream));
+    }
+    if ((rc = mx_run(ctx, count, points, off, n_static, (const uint32_t *)d_st, pl, ly, (const uint32_t *)d_sc, d_enc, d_out, d_ok,
+                     own)))
+        return rc;
+    CK(ctx, cudaMemcpyAsync(out32, d_out, count * 32, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(ctx, cudaMemcpyAsync(ok, d_ok, count, cudaMemcpyDeviceToHost, ctx->stream));
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     return BPP_OK;
 }

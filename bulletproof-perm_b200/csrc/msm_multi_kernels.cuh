@@ -8,6 +8,7 @@
 //   k_mm_pippenger   larger MSMs (c = MM_PIPPENGER_C): block per chunk of at most MM_CHUNK terms, thread per window,
 //                    the 2^(c-1) buckets of the thread's window in local memory (as k_dyn_window_sums); running-sum fold
 //   k_mm_finish      thread per MSM: adds the window sums of its chunks, Horner (c doublings per window), compress
+//                    (k_mm_finish_mixed, bpp_msm_mixed*: the same, plus the MSM's static part from the table kernels)
 // Digits: s' = s + K with K = sum_{w < W-1} 2^(c-1) 2^(cw); d_w = field w of s' minus 2^(c-1), the top window unsigned.
 // With s < 2^255 and cW >= 256, s' < 2^256 and every |d_w| <= 2^(c-1).
 #pragma once
@@ -208,10 +209,12 @@ __global__ void __launch_bounds__(64) k_mm_pippenger(const mm_item *__restrict__
 }
 
 // Thread per MSM: window sums of all its chunks, Horner, then the encoding (32 zero bytes and ok = 0 when one of its
-// points failed to decode; the identity also encodes as 32 zero bytes).
-__global__ void __launch_bounds__(MM_THREADS_FINISH) k_mm_finish(const mm_msm *__restrict__ msms, uint32_t count,
-                                                                 const uint32_t *__restrict__ wsum, const uint32_t *__restrict__ bad,
-                                                                 uint8_t *__restrict__ out32, uint8_t *__restrict__ ok) {
+// points failed to decode; the identity also encodes as 32 zero bytes).  MIXED (k_mm_finish_mixed, bpp_msm_mixed*): the
+// MSM's static part, an extended point at st_ext[j] from the table-gather kernels, is added after the Horner step.
+template <bool MIXED>
+__device__ __forceinline__ void mm_finish(const mm_msm *__restrict__ msms, uint32_t count, const uint32_t *__restrict__ wsum,
+                                          const uint32_t *__restrict__ st_ext, const uint32_t *__restrict__ bad,
+                                          uint8_t *__restrict__ out32, uint8_t *__restrict__ ok) {
     const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= count) return;
     const mm_msm m = msms[j];
@@ -233,6 +236,10 @@ __global__ void __launch_bounds__(MM_THREADS_FINISH) k_mm_finish(const mm_msm *_
             }
         }
     }
+    if (MIXED) {
+        ge_load(t, st_ext + 32 * (size_t)j);
+        ge_add(acc, acc, t);
+    }
     const bool good = !bad || bad[j] == 0;
     if (good) {
         ge_compress(out32 + 32 * (size_t)j, acc);
@@ -241,4 +248,26 @@ __global__ void __launch_bounds__(MM_THREADS_FINISH) k_mm_finish(const mm_msm *_
         for (int i = 0; i < 32; i += 4) *reinterpret_cast<uint32_t *>(out32 + 32 * (size_t)j + i) = 0u;
     }
     if (ok) ok[j] = good ? 1 : 0;
+}
+__global__ void __launch_bounds__(MM_THREADS_FINISH) k_mm_finish(const mm_msm *__restrict__ msms, uint32_t count,
+                                                                 const uint32_t *__restrict__ wsum, const uint32_t *__restrict__ bad,
+                                                                 uint8_t *__restrict__ out32, uint8_t *__restrict__ ok) {
+    mm_finish<false>(msms, count, wsum, nullptr, bad, out32, ok);
+}
+__global__ void __launch_bounds__(MM_THREADS_FINISH) k_mm_finish_mixed(const mm_msm *__restrict__ msms, uint32_t count,
+                                                                       const uint32_t *__restrict__ wsum,
+                                                                       const uint32_t *__restrict__ st_ext,
+                                                                       const uint32_t *__restrict__ bad, uint8_t *__restrict__ out32,
+                                                                       uint8_t *__restrict__ ok) {
+    mm_finish<true>(msms, count, wsum, st_ext, bad, out32, ok);
+}
+
+// bpp_msm_mixed_dev: a copy of the static part's n scalars with bit 255 cleared, so that device data cannot drive a table
+// digit past the window's 2^(c-1) entries (the host form rejects such scalars before any device work).
+__global__ void __launch_bounds__(128) k_mm_scalars_low255(const uint4 *__restrict__ src, uint64_t n, uint4 *__restrict__ dst) {
+    const uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+    if (i >= 2 * n) return;
+    uint4 v = src[i];
+    if (i & 1) v.w &= 0x7fffffffu;
+    dst[i] = v;
 }

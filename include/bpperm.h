@@ -225,6 +225,33 @@ int bpp_msm_multi_dev(bpp_ctx *ctx, size_t count, const uint32_t *sizes, const v
 int bpp_msm_multi_indexed_dev(bpp_ctx *ctx, size_t count, const uint32_t *sizes, const void *d_scalars,
                               const bpp_points *points, const void *d_index, void *d_out32);
 
+/* ---- mixed MSMs: a tabled generator set plus caller points in each MSM (dalek VartimePrecomputedMultiscalarMul) ----
+ * A verifier's MSM is mostly long-lived generators (g, h, G_vec, H_vec) and a few points from the proof (V, A_I, A_O, S,
+ * T_i, L_j, R_j: circuit_lib.rs:525-533, :552-565).  MSM j =
+ *   sum_{i < n_static} S[j][i] * points[off + i]  +  sum_{t = start_j}^{start_j + sizes[j] - 1} s_t * P_t
+ * The static part always uses the sub-range [off, off + n_static) of a resident set, with count x n_static scalars
+ * (row-major, one row per MSM: the layout of bpp_msm_vartime_batch); it runs through the set's window table at whatever
+ * width bpp_points_precompute gave it (built on first use at c = 8 if the set has none).  A caller with fewer static terms
+ * passes zero scalars: a zero digit costs no table add.  The dynamic part is ragged as in bpp_msm_multi: MSM j takes the
+ * next sizes[j] terms (T = sum sizes; sizes is host memory), its points as 32-byte RFC 9496 encodings.
+ * out32[j] is the canonical encoding of MSM j and ok[j] = 1; an undecodable dynamic encoding fails only its own MSM,
+ * whatever its static part: ok[j] = 0 and out32[j] = 32 zero bytes (dalek: optional_mixed_multiscalar_mul -> None).
+ * sizes[j] == 0 gives the static MSM alone, with bpp_msm_vartime_batch's bytes.  Scalars of both parts: 32-byte
+ * little-endian below 2^255; non-canonical values are accepted, as dalek accepts them.  A fixed handful of launches per
+ * call whatever count is, all on the context's stream; no device allocation after the first call of a size.
+ * Errors, host form, before any device work (outputs untouched): NULL pointers, count == 0, n_static == 0 (use
+ * bpp_msm_multi), T >= 2^31 or count x n_static >= 2^31: BPP_ERR_INVALID_ARG; off + n_static > bpp_points_len(points):
+ * BPP_ERR_LENGTH_MISMATCH; a scalar with bit 255 set, in either part: BPP_ERR_SCALAR_RANGE.  The _dev form checks what the
+ * host sees (pointers, count, n_static, sizes, the sub-range); its scalars, encodings, out32 and ok are device pointers,
+ * stream-ordered, no synchronisation, and device data cannot make it fault: bit 255 of a scalar is read as zero. */
+int bpp_msm_mixed(bpp_ctx *ctx, size_t count, bpp_points *points, size_t off, size_t n_static,
+                  const uint8_t *static_scalars /* count x n_static x 32 */, const uint32_t *sizes /* count, host */,
+                  const uint8_t *dyn_scalars /* T x 32 */, const uint8_t *dyn_points_enc /* T x 32 */,
+                  uint8_t *out32 /* count x 32 */, uint8_t *ok /* count */);
+int bpp_msm_mixed_dev(bpp_ctx *ctx, size_t count, bpp_points *points, size_t off, size_t n_static,
+                      const void *d_static_scalars, const uint32_t *sizes, const void *d_dyn_scalars,
+                      const void *d_dyn_points_enc, void *d_out32, void *d_ok);
+
 /* ---- the arithmetic-circuit (shuffle) proof, batched ------------------------------------------------
  * Replaces the group/scalar arithmetic of ACProof::ArithmeticCircuitProof (circuit_lib.rs:133-585) for
  * `count` independent proofs that share one circuit and one generator set, driven in the reference's

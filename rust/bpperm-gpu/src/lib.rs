@@ -4,7 +4,7 @@ use bpperm_sys as sys;
 use bulletproofs::ProofError;
 use curve25519_dalek_ng::ristretto::{CompressedRistretto, RistrettoPoint};
 use curve25519_dalek_ng::scalar::Scalar;
-use curve25519_dalek_ng::traits::VartimeMultiscalarMul;
+use curve25519_dalek_ng::traits::{VartimeMultiscalarMul, VartimePrecomputedMultiscalarMul};
 use once_cell::sync::Lazy;
 use std::borrow::Borrow;
 use std::sync::Mutex;
@@ -108,8 +108,60 @@ impl GeneratorSet {
         assert_eq!(rc, 0);
         out.chunks_exact(32).map(|c| CompressedRistretto(<[u8; 32]>::try_from(c).unwrap())).collect()
     }
+    /// Mixed MSMs in one `bpp_msm_mixed`: call j = sum_i static_scalars[j n + i] * points[off + i] + sum of the call's own
+    /// (scalars, points).  `static_scalars` holds calls.len() rows of n scalars (zeros where a call has fewer static
+    /// terms).  A call whose points do not all decode gives `None`; the other calls are unaffected.
+    pub fn mixed_msm_many(&self, static_scalars: &[Scalar], off: usize, n: usize, calls: &[(Vec<Scalar>, Vec<CompressedRistretto>)])
+                          -> Vec<Option<RistrettoPoint>> {
+        if calls.is_empty() { return Vec::new(); }
+        assert!(n > 0 && off + n <= self.n && static_scalars.len() == calls.len() * n);
+        let sizes: Vec<u32> = calls.iter().map(|(s, p)| { assert_eq!(s.len(), p.len()); s.len() as u32 }).collect();
+        let s: Vec<u8> = calls.iter().flat_map(|(s, _)| s.iter().flat_map(|x| x.to_bytes().to_vec())).collect();
+        let enc: Vec<u8> = calls.iter().flat_map(|(_, p)| p.iter().flat_map(|q| q.to_bytes().to_vec())).collect();
+        let mut out = vec![0u8; 32 * calls.len()];
+        let mut ok = vec![0u8; calls.len()];
+        let rc = with_ctx(|c| unsafe {
+            sys::bpp_msm_mixed(c, calls.len(), self.pts, off, n, bytes_of(static_scalars).as_ptr(), sizes.as_ptr(), s.as_ptr(),
+                               enc.as_ptr(), out.as_mut_ptr(), ok.as_mut_ptr())
+        });
+        assert_eq!(rc, 0);
+        out.chunks_exact(32).zip(ok.iter())
+            .map(|(o, &k)| if k == 1 { CompressedRistretto(<[u8; 32]>::try_from(o).unwrap()).decompress() } else { None })
+            .collect()
+    }
 }
 impl Drop for GeneratorSet { fn drop(&mut self) { with_ctx(|c| unsafe { sys::bpp_points_free(c, self.pts) }) } }
+
+/// `ristretto::VartimeRistrettoPrecomputation` -> `GpuRistrettoPrecomputation`: dalek's `VartimePrecomputedMultiscalarMul`
+/// (the verifier's MSM: static generators plus points from the proof).  `new` uploads the static points and builds their
+/// window table (c = 8) once; each call is a one-MSM `bpp_msm_mixed`.  For many such MSMs at once use
+/// `GeneratorSet::mixed_msm_many`.
+pub struct GpuRistrettoPrecomputation { set: Option<GeneratorSet> }   // None: no static points
+impl VartimePrecomputedMultiscalarMul for GpuRistrettoPrecomputation {
+    type Point = RistrettoPoint;
+    fn new<I>(static_points: I) -> Self where I: IntoIterator, I::Item: Borrow<RistrettoPoint> {
+        let pts: Vec<RistrettoPoint> = static_points.into_iter().map(|p| *p.borrow()).collect();
+        GpuRistrettoPrecomputation { set: if pts.is_empty() { None } else { Some(GeneratorSet::new(&pts, 8)) } }
+    }
+    fn optional_mixed_multiscalar_mul<I, J, K>(&self, static_scalars: I, dynamic_scalars: J, dynamic_points: K) -> Option<RistrettoPoint>
+    where I: IntoIterator, I::Item: Borrow<Scalar>, J: IntoIterator, J::Item: Borrow<Scalar>, K: IntoIterator<Item = Option<RistrettoPoint>> {
+        let st: Vec<Scalar> = static_scalars.into_iter().map(|s| *s.borrow()).collect();
+        let ds: Vec<Scalar> = dynamic_scalars.into_iter().map(|s| *s.borrow()).collect();
+        let dp: Vec<RistrettoPoint> = dynamic_points.into_iter().collect::<Option<Vec<_>>>()?;
+        assert_eq!(ds.len(), dp.len());
+        let enc: Vec<CompressedRistretto> = dp.iter().map(|p| p.compress()).collect();
+        match &self.set {
+            Some(set) => {
+                assert_eq!(st.len(), set.n, "one static scalar per static point");
+                set.mixed_msm_many(&st, 0, set.n, &[(ds, enc)]).pop().unwrap()
+            }
+            None => {
+                assert!(st.is_empty(), "one static scalar per static point");
+                GpuRistretto::optional_multiscalar_mul_many(&[(ds, enc)]).pop().unwrap()
+            }
+        }
+    }
+}
 
 /// A merlin `Transcript` held as the library's state (bpperm.h: bpp_transcript_*).  merlin::Transcript cannot be
 /// exported, so a caller that hands its protocol's inner-product argument to `InnerProductBatch` runs the transcript

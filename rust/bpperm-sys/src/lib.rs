@@ -66,6 +66,15 @@ extern "C" {
     pub fn bpp_msm_multi_indexed_dev(ctx: *mut bpp_ctx, count: usize, sizes: *const u32, d_scalars: *const core::ffi::c_void,
                                      points: *const bpp_points, d_index: *const core::ffi::c_void,
                                      d_out32: *mut core::ffi::c_void) -> c_int;
+    // mixed MSMs: count x n_static scalars over points[off..off + n_static) (window table) plus MSM j's next sizes[j]
+    // caller terms (encodings); a bad encoding fails only its own MSM (ok[j] = 0)
+    pub fn bpp_msm_mixed(ctx: *mut bpp_ctx, count: usize, points: *mut bpp_points, off: usize, n_static: usize,
+                         static_scalars: *const u8, sizes: *const u32, dyn_scalars: *const u8, dyn_points_enc: *const u8,
+                         out32: *mut u8, ok: *mut u8) -> c_int;
+    pub fn bpp_msm_mixed_dev(ctx: *mut bpp_ctx, count: usize, points: *mut bpp_points, off: usize, n_static: usize,
+                             d_static_scalars: *const core::ffi::c_void, sizes: *const u32, d_dyn_scalars: *const core::ffi::c_void,
+                             d_dyn_points_enc: *const core::ffi::c_void, d_out32: *mut core::ffi::c_void,
+                             d_ok: *mut core::ffi::c_void) -> c_int;
     // multi-GPU: one process per GPU, NCCL inside the library
     pub fn bpp_comm_unique_id(id: *mut u8) -> c_int;                      // 128 bytes, made on rank 0
     pub fn bpp_comm_init(ctx: *mut bpp_ctx, nranks: c_int, rank: c_int, id: *const u8) -> c_int;
