@@ -70,7 +70,8 @@ __global__ void k_acp_rng(const uint32_t *__restrict__ seeds /* B x 8 */, acp_la
     sc_store(ACP_PTR(blk, lay, p, lay.alpha + j), r);
 }
 
-// staged witness [a_L (B x n) | a_R (B x n) | a_O (B x n) | gamma (B x m)] -> the proofs' scalar blocks
+// staged witness [a_L (B x n) | a_R (B x n) | a_O (B x n) | gamma (B x m)] -> the proofs' scalar blocks, each value reduced
+// mod l (Scalar::from_bytes_mod_order): every kernel after this one takes canonical scalars
 __global__ void __launch_bounds__(128) k_acp_place_witness(const uint32_t *__restrict__ st, acp_layout lay, uint32_t B,
                                                            uint32_t *__restrict__ blk) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x, p = blockIdx.y;
@@ -79,10 +80,22 @@ __global__ void __launch_bounds__(128) k_acp_place_witness(const uint32_t *__res
     const uint32_t which = i < 3 * n ? i / n : 3, k = i - which * n;
     const uint32_t *src = which < 3 ? st + 8 * (((size_t)which * B + p) * n + k) : st + 8 * ((size_t)3 * B * n + (size_t)p * m + k);
     const uint32_t off = which == 0 ? lay.aL : which == 1 ? lay.aR : which == 2 ? lay.aO : lay.gamma;
-    uint4 lo = *reinterpret_cast<const uint4 *>(src), hi = *reinterpret_cast<const uint4 *>(src + 4);
-    uint32_t *dst = ACP_PTR(blk, lay, p, off + k);
-    *reinterpret_cast<uint4 *>(dst) = lo;
-    *reinterpret_cast<uint4 *>(dst + 4) = hi;
+    sc s;
+    sc_load(s, src);
+    sc_reduce256(s, s);
+    sc_store(ACP_PTR(blk, lay, p, off + k), s);
+}
+
+// caller scalars in place, mod l: rows x cnt values, row r at p + r * pitch (u32).  The shuffle witness' deck, x and
+// gamma and the caller's v of bpp_acp_batch_commit, which may be any 256-bit values.
+__global__ void __launch_bounds__(128) k_sc_reduce_rows(uint32_t *__restrict__ p, size_t pitch, uint32_t cnt) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= cnt) return;
+    uint32_t *q = p + pitch * blockIdx.y + 8 * (size_t)i;
+    sc s;
+    sc_load(s, q);
+    sc_reduce256(s, s);
+    sc_store(q, s);
 }
 
 // ---- shuffle witness on the device (replaces weights.rs:38-113 create_variables / create_a for the corrected k-card
@@ -967,7 +980,7 @@ __global__ void __launch_bounds__(320, 3) k_acp_dots_warp(acp_layout lay, uint32
         default: ua = lay.zWV; vb = lay.gamma; len = lay.m; break;
     }
     const uint32_t *a = ACP_PTR(blk, lay, p, ua), *b = ACP_PTR(blk, lay, p, vb);
-    // a lane's products are summed as 512-bit integers and reduced once (sc_mont_reduce: up to 15 at a time), not one
+    // a lane's products are summed as 512-bit integers and reduced once (sc_mont_reduce: up to SC_MAC_MAX at a time), not one
     // Montgomery reduction per product: 64 instead of 132 wide multiplies per element
     sc acc, x, y, pr, tot;
     sc_set0(acc);
@@ -978,7 +991,7 @@ __global__ void __launch_bounds__(320, 3) k_acp_dots_warp(acp_layout lay, uint32
         sc_load(x, a + 8 * (size_t)i);
         sc_load(y, b + 8 * (size_t)i);
         sc_mac(t, x, y);
-        if (++cnt == 15) {
+        if (++cnt == SC_MAC_MAX) {
             sc_mont_reduce(pr, t);
             sc_add(acc, acc, pr);
 #pragma unroll

@@ -142,4 +142,7 @@ int msm_enqueue(bpp_ctx *ctx, const uint32_t *d_scalars, const bpp_points *pts, 
 size_t msm_table_part_bytes(const bpp_ctx *ctx, const bpp_points *P, size_t n, size_t count);
 int msm_table_ext(bpp_ctx *ctx, const uint32_t *d_sc, const bpp_points *P, size_t off, size_t n, size_t count, uint32_t *d_ext,
                   uint32_t *d_part, uint64_t *madd, uint64_t *add);
+// defined in capi_msm_multi.cu: dst = n scalars of src with bit 255 cleared (the _dev table MSMs: device data cannot drive
+// a table digit past the window's 2^(c-1) entries).  Stream-ordered on ctx->stream.
+int msm_scalars_low255(bpp_ctx *ctx, const void *src, uint64_t n, void *dst);
 

@@ -424,10 +424,13 @@ extern "C" int bpp_msm_vartime_batch_dev(bpp_ctx *ctx, const void *d_scalars, si
     int rc;
     if (!points->fb_table && (rc = bpp_points_precompute(ctx, points, 8))) return rc;
     const fb_plan pl = msm_table_plan(ctx, points, n, count);
-    const size_t ext_b = count * 128, part_b = pl.splits > 1 ? count * pl.splits * 128 : 0;
-    if ((rc = grow(ctx, &ctx->d_small, &ctx->cap_small, ext_b + part_b))) return rc;
-    return msm_table_run(ctx, (const uint32_t *)d_scalars, points, off, n, count, (uint8_t *)d_out32, (uint32_t *)ctx->d_small,
-                         (uint32_t *)(ctx->d_small + ext_b), pl);
+    // the scalars with bit 255 cleared, as bpp_msm_mixed_dev takes them (the host form rejects such scalars instead)
+    const size_t sc_b = count * n * 32, ext_b = count * 128, part_b = pl.splits > 1 ? count * pl.splits * 128 : 0;
+    if ((rc = grow(ctx, &ctx->d_small, &ctx->cap_small, sc_b + ext_b + part_b))) return rc;
+    uint8_t *d = ctx->d_small;
+    if ((rc = msm_scalars_low255(ctx, d_scalars, (uint64_t)count * n, d))) return rc;
+    return msm_table_run(ctx, (const uint32_t *)d, points, off, n, count, (uint8_t *)d_out32, (uint32_t *)(d + sc_b),
+                         (uint32_t *)(d + sc_b + ext_b), pl);
 }
 extern "C" int bpp_msm_vartime_batch(bpp_ctx *ctx, const uint8_t *scalars, size_t count, bpp_points *points, size_t off, size_t n,
                                      uint8_t *out32) {
@@ -889,6 +892,11 @@ extern "C" int bpp_acp_batch_gen_shuffle_witness(bpp_acp_batch *b, const uint8_t
     CK(ctx, cudaMemcpyAsync(st + m32 + dk, x, xb, cudaMemcpyHostToDevice, ctx->stream));
     CK(ctx, cudaMemcpyAsync(st + m32 + dk + xb, perm, pk, cudaMemcpyHostToDevice, ctx->stream));
     CK(ctx, cudaMemcpyAsync(b->d_seeds, seeds, (size_t)B * 32, cudaMemcpyHostToDevice, ctx->stream));
+    {   // gamma | deck | x mod l, where they land: the inputs may be device data, which no host check can see
+        const uint32_t cnt = (uint32_t)((m32 + dk + xb) / 32);
+        k_sc_reduce_rows<<<dim3((cnt + 127) / 128, 1), 128, 0, ctx->stream>>>((uint32_t *)st, 0, cnt);
+        LAUNCH_CHECK(ctx);
+    }
     k_acp_place_gamma<<<dim3((L.m + 127) / 128, B), 128, 0, ctx->stream>>>((const uint32_t *)st, L, b->d_blk);
     LAUNCH_CHECK(ctx);
     if (k <= 64 || (k <= 1024 && 2ull * B >= 2048)) {
@@ -920,6 +928,10 @@ extern "C" int bpp_acp_batch_commit(bpp_acp_batch *b, const uint8_t *v, uint8_t 
     const size_t pitch = (size_t)L.stride * 32, m32 = (size_t)L.m * 32;
     CK(ctx, cudaMemcpy2DAsync((uint8_t *)b->d_blk + 32 * (size_t)L.l, pitch, v ? (const void *)v : (const void *)b->d_vwit, m32, m32, b->B,
                               v ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, ctx->stream));
+    if (v) {   // the caller's values mod l (those of bpp_acp_batch_gen_shuffle_witness already are)
+        k_sc_reduce_rows<<<dim3((L.m + 127) / 128, b->B), 128, 0, ctx->stream>>>(b->d_blk + 8 * (size_t)L.l, 8 * (size_t)L.stride, L.m);
+        LAUNCH_CHECK(ctx);
+    }
     fb_shape sh = acp_shape(L.m);
     acp_seg(sh, L.l, 1, 0, 1);
     acp_seg(sh, L.gamma, 1, 1, 1);

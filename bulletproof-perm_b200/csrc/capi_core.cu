@@ -978,6 +978,7 @@ extern "C" int bpp_bench_pipe_probe(bpp_ctx *ctx, int mode, int iters, double *o
 
 extern "C" int bpp_test_op(bpp_ctx *ctx, int op, const uint8_t *a, const uint8_t *b, uint8_t *out, size_t n) {
     if (!ctx || !a || !b || !out || n == 0 || n >= (1ull << 31)) return BPP_ERR_INVALID_ARG;
+    if (op < 0 || op >= BPP_TEST_SC_MAC + SC_MAC_MAX || (op == BPP_TEST_SC_WARP_SUM && n % 32)) return BPP_ERR_INVALID_ARG;
     CK(ctx, cudaSetDevice(ctx->device));
     uint8_t *d = nullptr;
     CK(ctx, cudaMalloc((void **)&d, n * 96));

@@ -277,6 +277,11 @@ extern "C" int bpp_msm_multi_indexed(bpp_ctx *ctx, size_t count, const uint32_t 
     return BPP_OK;
 }
 
+int msm_scalars_low255(bpp_ctx *ctx, const void *src, uint64_t n, void *dst) {
+    k_mm_scalars_low255<<<(unsigned)((2 * n + 127) / 128), 128, 0, ctx->stream>>>((const uint4 *)src, n, (uint4 *)dst);
+    LAUNCH_CHECK(ctx);
+    return BPP_OK;
+}
 extern "C" int bpp_msm_mixed_dev(bpp_ctx *ctx, size_t count, bpp_points *points, size_t off, size_t n_static,
                                  const void *d_static_scalars, const uint32_t *sizes, const void *d_dyn_scalars,
                                  const void *d_dyn_points_enc, void *d_out32, void *d_ok) {
@@ -291,9 +296,7 @@ extern "C" int bpp_msm_mixed_dev(bpp_ctx *ctx, size_t count, bpp_points *points,
     const uint64_t n_sc = (uint64_t)count * n_static;
     const size_t own = al256(n_sc * 32);
     if ((rc = grow(ctx, &ctx->d_multi, &ctx->cap_multi, ly.total(own)))) return rc;
-    k_mm_scalars_low255<<<(unsigned)((2 * n_sc + 127) / 128), 128, 0, ctx->stream>>>((const uint4 *)d_static_scalars, n_sc,
-                                                                                    (uint4 *)ctx->d_multi);
-    LAUNCH_CHECK(ctx);
+    if ((rc = msm_scalars_low255(ctx, d_static_scalars, n_sc, ctx->d_multi))) return rc;
     return mx_run(ctx, count, points, off, n_static, (const uint32_t *)ctx->d_multi, pl, ly, (const uint32_t *)d_dyn_scalars,
                   (const uint8_t *)d_dyn_points_enc, (uint8_t *)d_out32, (uint8_t *)d_ok, own);
 }

@@ -17,6 +17,7 @@
 //   k_msm_finish      last merge per window, Horner over windows (c doublings each), compress
 #pragma once
 #include "ge25519.cuh"
+#include "vec_kernels.cuh"
 
 #define BPP_ACC_THREADS 128
 
@@ -879,6 +880,53 @@ __global__ void k_test_op(int op, const uint8_t *__restrict__ a, const uint8_t *
     if (i >= n) return;
     const uint8_t *pa = a + 32 * (size_t)i, *pb = b + 32 * (size_t)i;
     uint8_t *po = out + 32 * (size_t)i;
+    if (op >= BPP_TEST_SC_ADD) {   // scalars mod l (bpp_test_op checks the op code and, for SC_WARP_SUM, n % 32)
+        sc x, y, r;
+        uint32_t t[16];
+#pragma unroll
+        for (int k = 0; k < 8; k++) {
+            x.v[k] = t[k] = pa[4 * k] | (uint32_t)pa[4 * k + 1] << 8 | (uint32_t)pa[4 * k + 2] << 16 | (uint32_t)pa[4 * k + 3] << 24;
+            y.v[k] = t[8 + k] = pb[4 * k] | (uint32_t)pb[4 * k + 1] << 8 | (uint32_t)pb[4 * k + 2] << 16 | (uint32_t)pb[4 * k + 3] << 24;
+        }
+        switch (op) {
+            case BPP_TEST_SC_ADD: sc_add(r, x, y); break;
+            case BPP_TEST_SC_SUB: sc_sub(r, x, y); break;
+            case BPP_TEST_SC_NEG: sc_neg(r, x); break;
+            case BPP_TEST_SC_MONT: sc_mont(r, x, y); break;
+            case BPP_TEST_SC_MUL: sc_mul(r, x, y); break;
+            case BPP_TEST_SC_INVERT: sc_invert(r, x); break;
+            case BPP_TEST_SC_REDUCE256: sc_reduce256(r, x); break;
+            case BPP_TEST_SC_FROM_WIDE: sc_from_wide(r, t); break;
+            case BPP_TEST_SC_MONT_REDUCE: sc_mont_reduce(r, t); break;
+            case BPP_TEST_SC_WARP_SUM: {   // n % 32 == 0: whole warps, each over 32 consecutive values
+                uint32_t s9[9];
+                warp_sum9(s9, x);
+#pragma unroll
+                for (int k = 0; k < 9; k++) s9[k] = __shfl_sync(0xffffffffu, s9[k], 0);
+                sc_from9(r, s9);
+                break;
+            }
+            default: {   // SC_MAC + K - 1: K products accumulated by sc_mac, one sc_mont_reduce
+                const uint32_t K = (uint32_t)(op - BPP_TEST_SC_MAC) + 1;
+#pragma unroll
+                for (int k = 0; k < 16; k++) t[k] = 0;
+                for (uint32_t j = 0; j < K; j++) {
+                    const uint32_t e = (uint32_t)(((uint64_t)i + j) % n);
+                    const uint8_t *qa = a + 32 * (size_t)e, *qb = b + 32 * (size_t)e;
+#pragma unroll
+                    for (int k = 0; k < 8; k++) {
+                        x.v[k] = qa[4 * k] | (uint32_t)qa[4 * k + 1] << 8 | (uint32_t)qa[4 * k + 2] << 16 | (uint32_t)qa[4 * k + 3] << 24;
+                        y.v[k] = qb[4 * k] | (uint32_t)qb[4 * k + 1] << 8 | (uint32_t)qb[4 * k + 2] << 16 | (uint32_t)qb[4 * k + 3] << 24;
+                    }
+                    sc_mac(t, x, y);
+                }
+                sc_mont_reduce(r, t);
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < 32; k++) po[k] = (uint8_t)(r.v[k >> 2] >> (8 * (k & 3)));
+        return;
+    }
     if (op <= 4 || op == 9) {
         fe x, y, r;
         fe_frombytes(x, pa);

@@ -262,7 +262,7 @@ __global__ void __launch_bounds__(MM_THREADS_FINISH) k_mm_finish_mixed(const mm_
     mm_finish<true>(msms, count, wsum, st_ext, bad, out32, ok);
 }
 
-// bpp_msm_mixed_dev: a copy of the static part's n scalars with bit 255 cleared, so that device data cannot drive a table
+// bpp_msm_mixed_dev, bpp_msm_vartime_batch_dev: a copy of the table MSM's n scalars with bit 255 cleared, so that device data cannot drive a table
 // digit past the window's 2^(c-1) entries (the host form rejects such scalars before any device work).
 __global__ void __launch_bounds__(128) k_mm_scalars_low255(const uint4 *__restrict__ src, uint64_t n, uint4 *__restrict__ dst) {
     const uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;

@@ -124,6 +124,8 @@ __device__ __constant__ const uint32_t SC_NP[8] = {0x12547e1bu, 0xd2b51da3u, 0xf
 // sc_mont_reduce(r, t) = t / 2^256 mod l for any t < l * 2^256 (the reduction half of sc_mont): (t + q*l) / 2^256 <
 // t / 2^256 + l < 2l, so one conditional subtraction makes it canonical.  A sum of up to 15 products of canonical
 // scalars stays below that bound, so sums of products can be accumulated as 512-bit integers (sc_mac) and reduced once.
+// SC_MAC_MAX is that count: 15 (l-1)^2 < l * 2^256 <= 16 (l-1)^2, so a 16th product of large operands can exceed it.
+#define SC_MAC_MAX 15
 #pragma nv_diag_suppress 550   // `dummy` receives a limb whose carry-out is all that matters
 SC_INLINE void sc_mont_reduce(sc &r, const uint32_t t[16]) {
     uint32_t qf[8], u[12], np[8], dl[4];

@@ -194,7 +194,9 @@ int bpp_msm_sharded_wait(bpp_ctx *ctx);
  * buckets, no doublings: three short launches), and bpp_msm_vartime_batch evaluates `count` MSMs over the same
  * points[off..off+n) with count x n scalars in one launch (out32: count x 32 compressed results).  The table is built
  * on first use (c = 8) if bpp_points_precompute was not called.  _dev: scalars and results in device memory,
- * stream-ordered, no synchronisation. */
+ * stream-ordered, no synchronisation.  Scalars are taken below 2^255 (their digits index the table's 2^(c-1) rows): the
+ * host form rejects a scalar with bit 255 set (BPP_ERR_SCALAR_RANGE); the _dev form, which cannot see device data
+ * before it runs, clears bit 255 of every scalar, as bpp_msm_mixed_dev does. */
 int bpp_points_precompute(bpp_ctx *ctx, bpp_points *points, int window_bits);
 int bpp_msm_vartime_batch(bpp_ctx *ctx, const uint8_t *scalars, size_t count, bpp_points *points, size_t off, size_t n,
                           uint8_t *out32);
@@ -320,6 +322,9 @@ int bpp_acproof_verify_batch(bpp_ctx *ctx, const bpp_circuit *cir, const bpp_gen
 int bpp_acp_batch_create(bpp_ctx *ctx, const bpp_circuit *cir, const bpp_gens *gens, int mode, size_t count,
                          const uint8_t *label, size_t label_len, bpp_acp_batch **out);
 void bpp_acp_batch_free(bpp_acp_batch *b);
+/* Caller scalars of the prover (a_L, a_R, a_O and gamma here; deck, x and gamma of bpp_acp_batch_gen_shuffle_witness; v
+ * of bpp_acp_batch_commit) may be any 32-byte values: each is reduced mod l on the device where it lands
+ * (Scalar::from_bytes_mod_order), so a value and its representatives >= l give the same commitments and proofs. */
 int bpp_acp_batch_upload_witness(bpp_acp_batch *b, const uint8_t *aL, const uint8_t *aR, const uint8_t *aO,
                                  const uint8_t *gamma, const uint8_t *seeds);
 /* The shuffle witness generated on the device (replaces weights.rs:38-113 create_variables + create_a for the circuit
@@ -480,7 +485,15 @@ int bpp_last_op_counts(bpp_ctx *ctx, uint64_t *mixed_adds, uint64_t *full_adds, 
 /* ---- element-wise self-test hooks (used by tests/ to compare single operations with the oracle) */
 enum { BPP_TEST_FE_MUL = 0, BPP_TEST_FE_ADD, BPP_TEST_FE_SUB, BPP_TEST_FE_INVERT, BPP_TEST_FE_CANON,
        BPP_TEST_GE_ADD, BPP_TEST_GE_DOUBLE, BPP_TEST_GE_COMPRESS_ROUNDTRIP, BPP_TEST_GE_SCALARMULT,
-       BPP_TEST_FE_SQR, BPP_TEST_GE_DOUBLE_Z1 /* doubling with a compile-time Z = 1 */ };
+       BPP_TEST_FE_SQR, BPP_TEST_GE_DOUBLE_Z1 /* doubling with a compile-time Z = 1 */,
+       /* scalars mod l, 32-byte little-endian; R = 2^256.  SC_ADD, SC_SUB, SC_NEG, SC_MUL, SC_INVERT (0 -> 0) take canonical
+        * operands; SC_MONT: a * b / R mod l for a * b < l * R; SC_REDUCE256: a mod l for any 256-bit a; SC_FROM_WIDE: the
+        * 512-bit a || b (a low) mod l; SC_MONT_REDUCE: t / R mod l for t = a || b < l * R; SC_WARP_SUM: the sum of each
+        * group of 32 consecutive a mod l, in every slot of the group (n a multiple of 32); SC_MAC + K - 1, K = 1..15: the
+        * 512-bit sum of a[j] * b[j], j = i .. i + K - 1 (mod n), then t / R mod l - the dot kernels' accumulation of at
+        * most 15 products of canonical scalars between reductions.  Other op codes: BPP_ERR_INVALID_ARG. */
+       BPP_TEST_SC_ADD, BPP_TEST_SC_SUB, BPP_TEST_SC_NEG, BPP_TEST_SC_MONT, BPP_TEST_SC_MUL, BPP_TEST_SC_INVERT,
+       BPP_TEST_SC_REDUCE256, BPP_TEST_SC_FROM_WIDE, BPP_TEST_SC_MONT_REDUCE, BPP_TEST_SC_WARP_SUM, BPP_TEST_SC_MAC };
 /* a, b: n x 32-byte operands (points as compressed encodings); out: n x 32 bytes. */
 int bpp_test_op(bpp_ctx *ctx, int op, const uint8_t *a, const uint8_t *b, uint8_t *out, size_t n);
 
